@@ -149,6 +149,61 @@ def oracle_config(spec):
                           exclude=c.get("exclude"), want_dosage=bool(c.get("dosage")))
 
 
+DUMP_SEED = 20130502
+DUMP_ROW_WINDOWS, DUMP_WINDOW_BYTES = 128, 64 << 10  # 8 MiB of row text -> 32 MiB as float32
+DUMP_DOSAGE_BYTES = 20 << 20  # whole dosage rows as float32 (2,093 rows of 2,504 samples)
+DUMP_DIAGS = 1 << 16  # x 4 float64
+
+
+def dump_outputs(tr, stats, out_dir):
+    """What the last timed resident run returned to its caller, as .npy files in out_dir (under 60 MB in all): the
+    run's counts, the TSV rows, the dosage matrix and loci of dosage configs, the diagnostics.  Outputs larger than
+    that are sampled at positions drawn from DUMP_SEED, the same for every run of the same arguments."""
+    import random
+
+    import numpy as np
+
+    from bystro_vcf_b200 import _lib
+
+    os.makedirs(out_dir, exist_ok=True)
+    rng = random.Random(DUMP_SEED)
+
+    def save(name, a, dtype):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=dtype))
+
+    keys = ("n_lines", "n_records", "n_rows", "in_bytes", "out_bytes")
+    save("stats", [stats[k] for k in keys], np.float64)
+    n = stats["out_bytes"]
+    if n <= DUMP_ROW_WINDOWS * DUMP_WINDOW_BYTES:
+        offsets, width = [0], n
+    else:  # one window in each of DUMP_ROW_WINDOWS equal strata of the output
+        stratum = n // DUMP_ROW_WINDOWS
+        offsets = [i * stratum + rng.randrange(stratum - DUMP_WINDOW_BYTES + 1) for i in range(DUMP_ROW_WINDOWS)]
+        width = DUMP_WINDOW_BYTES
+    rows = [np.frombuffer(tr.resident_download(o, width), dtype=np.uint8) for o in offsets]
+    save("rows", np.stack(rows), np.float32)  # [windows, bytes]: byte values of the row text
+    save("rows_offsets", offsets, np.float64)
+
+    dos = _lib.CDosageBatch()
+    dg = C.POINTER(_lib.CDiag)()
+    nd = C.c_size_t()
+    _lib.check(_lib.lib().bvcf_resident_results(tr._ctx, C.byref(dos), C.byref(dg), C.byref(nd)), tr._ctx,
+               "bvcf_resident_results")
+    if dos.n_rows:
+        nr, ns = dos.n_rows, dos.n_samples
+        pick = sorted(rng.sample(range(nr), min(nr, max(1, DUMP_DOSAGE_BYTES // (4 * ns)))))
+        mat = np.ctypeslib.as_array(dos.dosage, shape=(nr, ns))
+        save("dosage", mat[pick], np.float32)  # [sampled rows, samples]
+        save("dosage_rows", pick, np.float64)
+        offs = np.ctypeslib.as_array(dos.loci_off, shape=(nr + 1,))
+        base = C.cast(dos.loci, C.c_void_p).value
+        loci = b"\n".join(C.string_at(base + int(offs[i]), int(offs[i + 1] - offs[i])) for i in pick) + b"\n"
+        save("loci", np.frombuffer(loci, dtype=np.uint8), np.float32)  # the sampled rows' loci, newline-separated
+    picked = sorted(rng.sample(range(nd.value), min(nd.value, DUMP_DIAGS)))
+    diags = [(dg[i].line_no, dg[i].alt_no, dg[i].code, dg[i].line_start) for i in picked]
+    save("diagnostics", np.asarray(diags, dtype=np.float64).reshape(-1, 4), np.float64)  # line, alt, code, line start
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -213,6 +268,8 @@ def run_ours(args):
     stats, acc, wall_ms, gpu_launches, clk = resident_steps(need, n_lines)
     dev_ms = acc["total_ms"]  # CUDA events on the launching stream, first to last launch of every step
     out_bytes, n_rows = stats["out_bytes"], stats["n_rows"]
+    if args.dump_outputs and rank == 0:  # before anything else runs on the resident regions
+        dump_outputs(tr, stats, args.dump_outputs)
 
     # ---- parity of what was just timed: the rows of the first lines against the CPU oracle (outside the timed region) ----
     parity = None
@@ -578,7 +635,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-bgzf", action="store_true", help="skip the bgzf-compressed end-to-end line")
     ap.add_argument("--bgzf-mb", type=int, default=1024, help="text bytes of the bgzf end-to-end sample")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rows, counts, dosage) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the timed CUDA path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3 if args.impl == "ours" else args.warmup
     if args.impl == "reference":

@@ -185,6 +185,9 @@ DOSAGE_CASE = (
 BASE_HEADER = ["chrom", "pos", "type", "ref", "alt", "trTv", "heterozygotes", "heterozygosity", "homozygotes",
                "homozygosity", "missingGenos", "missingness", "ac", "an", "sampleMaf"]
 
-GOLDEN_MD5_INPUT_ORDER = "1fc986559394c755f4fce080a3366dc4"  # default flags, body only, 20,370,676 B
-GOLDEN_MD5_SORTED = "ce2e87ef3a6c7634598b4f8c0df889a7"  # LC_ALL=C sort -k1,1 -k2,2n -k5,5 (reference procedure)
-GOLDEN_MD5_KEEPID_KEEPINFO = "9a837060579f4e079fcb9f27cbc6d3ef"  # oracle-derived (no reference golden exists)
+# chr1 goldens (tests/conftest.py): the 400-line sample and the sample CHR1_REPEATS times over (chr1_fixture)
+CHR1_REPEATS = 49
+GOLDEN_SAMPLE_LINES, GOLDEN_SAMPLE_ROWS = 400, 410
+GOLDEN_MD5_SORTED = "9d2c0824f4f6d584d711e65519b8acae"  # sample, LC_ALL=C sort -k1,1 -k2,2n -k5,5 (reference procedure)
+GOLDEN_MD5_INPUT_ORDER = "548d4a7464de83108ca88130c7a5e065"  # chr1_fixture, default flags, body only, 32,496,849 B
+GOLDEN_MD5_KEEPID_KEEPINFO = "39f2056b35704d34a6aad24630eb2b2a"  # chr1_fixture, oracle-derived (no reference golden exists)

@@ -84,7 +84,7 @@ def test_allele_vectors(inp, exp):
 
 def test_golden_chr1(chr1_fixture):
     got = gpu_rows(chr1_fixture)
-    assert len(got) == 20370676
+    assert len(got) == 32496849
     assert hashlib.md5(got).hexdigest() == V.GOLDEN_MD5_INPUT_ORDER
 
 
@@ -95,7 +95,7 @@ def test_golden_chr1_keepid_keepinfo_small_chunks(chr1_fixture):
     cfg.chunkBytes = 7 << 20  # many chunks, lines straddle every read boundary
     out = io.BytesIO()
     st = read_vcf(cfg, io.BytesIO(chr1_fixture), out)
-    assert st["n_lines"] == 19747 and st["n_rows"] == 19821
+    assert st["n_lines"] == 19600 and st["n_rows"] == 20090
     assert hashlib.md5(out.getvalue()).hexdigest() == V.GOLDEN_MD5_KEEPID_KEEPINFO
 
 

@@ -70,12 +70,15 @@ def test_unterminated_last_line_dropped():
     assert [x[1] for x in rows_of(r.tsv)] == ["5"]
 
 
-def test_golden_chr1(chr1_fixture, tmp_path):
-    """previous_out_check/README.md:3-10: sort both, compare.  Plus the input-order md5."""
-    r = O.read_vcf(O.OracleConfig(), chr1_fixture)
-    assert r.n_lines == 19747 and r.n_rows == 19821
-    assert hashlib.md5(r.tsv).hexdigest() == V.GOLDEN_MD5_INPUT_ORDER
-    with gzip.open(os.path.join(ROOT, "tests", "golden", "chr1_20klines.golden_out_10_3_18.tsv.gz")) as f:
+def test_golden_chr1(chr1_sample, chr1_fixture, tmp_path):
+    """previous_out_check/README.md:3-10 on the sampled lines: sort both, compare.  Plus the input-order md5 of the
+    sample repeated (chr1_fixture), which is the sample's rows as often."""
+    r = O.read_vcf(O.OracleConfig(), chr1_sample)
+    assert r.n_lines == V.GOLDEN_SAMPLE_LINES and r.n_rows == V.GOLDEN_SAMPLE_ROWS
+    big = O.read_vcf(O.OracleConfig(), chr1_fixture)
+    assert big.tsv == r.tsv * V.CHR1_REPEATS
+    assert hashlib.md5(big.tsv).hexdigest() == V.GOLDEN_MD5_INPUT_ORDER
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "chr1_400lines.golden_out_10_3_18.tsv.gz")) as f:
         gold = f.read()
     head, _, body = gold.partition(b"\n")
     assert head.decode() == O.header(O.OracleConfig())
@@ -88,7 +91,7 @@ def test_golden_chr1(chr1_fixture, tmp_path):
     assert sa == sb
     assert hashlib.md5(sa).hexdigest() == V.GOLDEN_MD5_SORTED
     # threads: same bytes in the same order
-    assert O.read_vcf(O.OracleConfig(), chr1_fixture, threads=4).tsv == r.tsv
+    assert O.read_vcf(O.OracleConfig(), chr1_fixture, threads=4).tsv == big.tsv
 
 
 def test_query_fixture_counts(query_fixture):
