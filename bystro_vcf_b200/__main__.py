@@ -2,7 +2,8 @@
 
 Same flags, same stdin/stdout behaviour: header line first (main.go:199), then rows in input order; the
 reference's log.Printf lines ("chrom:pos ALT #k message", main.go:730-986) on stderr, or appended to --err.
-`--gpus N` (extension) shards the input over N GPUs of the box (shard.read_vcf_multi); `--bgzfOut` (extension) writes
+`--gpus N` (extension) shards the input -- plain or bgzf (.vcf.gz) -- over N GPUs of the box (shard.read_vcf_multi);
+`--bgzfOut` (extension) writes
 the rows as bgzf blocks deflated on the GPU -- with a .vcf.gz input the command stands for the whole
 `pigz -d -c in.vcf.gz | bystro-vcf ... | pigz -c > out.gz` of README.md:10."""
 from __future__ import annotations
@@ -10,6 +11,7 @@ from __future__ import annotations
 import os
 import sys
 
+from ._lib import BvcfError
 from .host import NotAVcfError, read_vcf, setup, string_header
 
 
@@ -82,6 +84,9 @@ def main(argv=None) -> int:
             out.write(bgzf.EOF_BLOCK)
     except NotAVcfError as e:
         print(str(e), file=err)  # log.Fatal main.go:263,293
+        return 1
+    except BvcfError as e:  # a corrupt .vcf.gz member, a line longer than a chunk ...
+        print(str(e), file=sys.stderr)
         return 1
     finally:
         if out is not None:

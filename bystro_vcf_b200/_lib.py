@@ -81,6 +81,7 @@ SYMBOLS = [
     "bvcf_resident_run", "bvcf_resident_download", "bvcf_resident_peek", "bvcf_resident_line_index", "bvcf_strerror",
     "bvcf_last_error", "bvcf_abi_version", "bvcf_launch_count", "bvcf_resident_run_at", "bvcf_resident_inflate_bgzf",
     "bvcf_bgzf_text_bytes", "bvcf_resident_download_bgzf", "bvcf_resident_write_output", "bvcf_resident_results",
+    "bvcf_submit_bgzf", "bvcf_diag_fields",
 ]
 
 _lib = None
@@ -115,6 +116,10 @@ def lib():
     L.bvcf_collect.argtypes = [vp, u64, C.POINTER(vp), C.POINTER(sz), C.POINTER(CDosageBatch),
                                C.POINTER(C.POINTER(CDiag)), C.POINTER(sz), C.POINTER(CChunkStats)]
     L.bvcf_release.restype = C.c_int
+    L.bvcf_submit_bgzf.restype = C.c_int
+    L.bvcf_submit_bgzf.argtypes = [vp, u64, vp, sz, sz, vp, sz]
+    L.bvcf_diag_fields.restype = C.c_int
+    L.bvcf_diag_fields.argtypes = [vp, u64, C.POINTER(vp), C.POINTER(C.POINTER(u64))]
     L.bvcf_release.argtypes = [vp, u64]
     L.bvcf_resident_alloc.restype = C.c_int
     L.bvcf_resident_alloc.argtypes = [vp, sz, sz, C.POINTER(vp), C.POINTER(vp)]
@@ -157,6 +162,8 @@ def check(rc: int, ctx=None, what: str = "") -> None:
         return
     L = lib()
     msg = L.bvcf_strerror(rc).decode()
-    if ctx is not None and rc == -2:
-        msg += ": " + L.bvcf_last_error(ctx).decode()
+    if ctx is not None and rc in (-1, -2):
+        detail = L.bvcf_last_error(ctx).decode()
+        if detail or rc == -2:
+            msg += ": " + detail
     raise BvcfError(f"{what or 'libbvcf'} failed ({rc}): {msg}")

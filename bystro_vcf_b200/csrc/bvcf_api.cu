@@ -11,6 +11,8 @@
 //   bvcf_copyout_kernel            rows to the output with aligned stores, loci, RowDesc work lists
 //   bvcf_slow_rows_kernel          the few records that do not fit a tile's arena
 //   bvcf_names_{vec,long,big}_     long sample-name lists, their dosage rows  (north-star kernel 4b)
+// A bgzf chunk (bvcf_submit_bgzf) is inflated on the same stream first (bvcf_inflate_kernel, into the slot's input
+// buffer); bvcf_diag_fields_kernel gathers the CHROM and POS fields of its diagnosed lines for the host's log lines.
 #include "../../include/bvcf.h"
 
 #include <algorithm>
@@ -55,6 +57,7 @@ struct Slot {
   cudaStream_t stream = nullptr;
   cudaEvent_t done = nullptr;
   DevBuf d_in, d_out, d_dosage, d_loci, d_loci_off, d_diags;
+  DevBuf d_comp, d_blocks, d_fields, d_field_off, d_diag_starts;  // bgzf chunks; diagnostic fields
   Scratch sc;
   RunCounters *d_ctr = nullptr;
   RunCounters *h_ctr = nullptr;  // pinned
@@ -73,6 +76,17 @@ struct Slot {
   const uint8_t *h_src = nullptr;
   size_t len = 0;
   uint32_t retries = 0;
+  uint32_t diag_cap = 0;         // entries of d_diags the chunk was enqueued with
+  // bgzf chunk: the text is inflate(comp) [0, text_len) then the tail; data lines start at `skip`
+  bool bgzf = false;
+  size_t skip = 0, text_len = 0, tail_len = 0;
+  uint8_t *h_stage = nullptr;    // pinned: compressed bytes, block table, tail
+  size_t h_stage_cap = 0;
+  uint32_t *d_bad = nullptr;     // blocks that failed to inflate
+  uint32_t *h_bad = nullptr;     // pinned copy
+  std::vector<InflateBlock> blocks;
+  std::vector<uint8_t> h_fields;
+  std::vector<uint64_t> h_field_off, h_diag_starts;
 };
 
 constexpr uint32_t LOCI_GUESS = 32;          // first guess of locus bytes per row; the buffer grows to what a chunk reports
@@ -223,7 +237,7 @@ struct StageEvents {  // optional per-stage timing of one sub-chunk
 int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t *d_in, uint64_t begin, uint64_t len, uint64_t buf_len,
                      uint8_t *d_out, uint64_t out_cap, RunCounters *d_ctr, int8_t *d_dosage, uint64_t dosage_cap_rows,
                      uint8_t *d_loci, uint64_t loci_cap, unsigned long long *d_loci_off, uint32_t *d_diags,
-                     std::vector<StageEvents> *timing) {
+                     uint32_t diag_cap, std::vector<StageEvents> *timing) {
   const DevCfg &dc = ctx->dcfg;
   // data lines live in [begin, len); ranges tile the region from begin rounded down to 512 bytes
   const uint64_t a0 = begin & ~511ull;
@@ -318,7 +332,7 @@ int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t 
     }
     tp.dosage = d_dosage; tp.dosage_cap_rows = dosage_cap_rows;
     tp.loci = d_loci; tp.loci_cap = loci_cap; tp.loci_off = d_loci_off;
-    tp.diag.diags = d_diags; tp.diag.cap = ctx->diag_cap; tp.diag.ctr = d_ctr;
+    tp.diag.diags = d_diags; tp.diag.cap = diag_cap; tp.diag.ctr = d_ctr;
     {
       auto launch = [&](auto kern, uint32_t arena, uint32_t rows, int minb) {
         const uint32_t smem = TILE_WARPS * tile_smem_warp(arena, rows);
@@ -478,12 +492,43 @@ void decode_diags(const uint32_t *raw, uint32_t nd, std::vector<bvcf_diag> &out)
   }
 }
 
-int slot_enqueue(bvcf_ctx *ctx, Slot &s, bool upload) {
+// A bgzf chunk's compressed bytes, block table and tail are in the slot's pinned staging buffer: upload them, inflate the
+// blocks into d_in, put the tail after the text.  Only the first attempt does this -- a retry finds the text on the device.
+int slot_inflate(bvcf_ctx *ctx, Slot &s, size_t comp_len) {
+  const size_t nb = s.blocks.size(), tab_off = round_up(comp_len, 16), tail_off = tab_off + nb * sizeof(InflateBlock);
+  int rc;
+  if ((rc = dev_reserve(ctx, s.d_comp, comp_len + 16))) return rc;  // the bit reader may look 11 bytes past the payload
+  if ((rc = dev_reserve(ctx, s.d_blocks, nb * sizeof(InflateBlock)))) return rc;
+  if (!s.d_bad) CK(cudaMalloc(&s.d_bad, 4));
+  if (!s.h_bad) CK(cudaMallocHost(&s.h_bad, 8));  // [0] bad blocks, [1] last text byte
+  s.h_bad[0] = s.h_bad[1] = 0;
+  CK(cudaMemsetAsync(s.d_bad, 0, 4, s.stream));
+  if (nb) {
+    CK(cudaMemcpyAsync(s.d_comp.p, s.h_stage, comp_len, cudaMemcpyHostToDevice, s.stream));
+    CK(cudaMemcpyAsync(s.d_blocks.p, s.h_stage + tab_off, nb * sizeof(InflateBlock), cudaMemcpyHostToDevice, s.stream));
+    InflateParams ip{};
+    ip.comp = (const uint8_t *)s.d_comp.p; ip.out = (uint8_t *)s.d_in.p; ip.blocks = (const InflateBlock *)s.d_blocks.p;
+    ip.n_blocks = (uint32_t)nb; ip.n_bad = s.d_bad;
+    cudaFuncSetAttribute(bvcf_inflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)INF_SMEM);
+    bvcf_inflate_kernel<<<ip.n_blocks, 32, INF_SMEM, s.stream>>>(ip);
+    ctx->launches++;
+  }
+  if (s.tail_len)
+    CK(cudaMemcpyAsync((uint8_t *)s.d_in.p + s.text_len, s.h_stage + tail_off, s.tail_len, cudaMemcpyHostToDevice, s.stream));
+  CK(cudaMemcpyAsync(s.h_bad, s.d_bad, 4, cudaMemcpyDeviceToHost, s.stream));
+  if (s.len > s.skip && !s.tail_len)  // the text must end with a newline: its last byte, for bvcf_collect
+    CK(cudaMemcpyAsync(s.h_bad + 1, (const uint8_t *)s.d_in.p + s.len - 1, 1, cudaMemcpyDeviceToHost, s.stream));
+  else
+    s.h_bad[1] = '\n';
+  return 0;
+}
+
+int slot_enqueue(bvcf_ctx *ctx, Slot &s, bool upload, size_t comp_len = 0) {
   const uint64_t len = s.len;
   const uint64_t buf_len = round_up(len, 1024) + 2048;
   int rc;
   if ((rc = dev_reserve(ctx, s.d_in, buf_len + IN_SLACK))) return rc;
-  if ((rc = scratch_reserve(ctx, s.sc, len, ctx->cfg.resident_subchunk_bytes))) return rc;
+  if ((rc = scratch_reserve(ctx, s.sc, len - (s.skip & ~511ull), ctx->cfg.resident_subchunk_bytes))) return rc;
   if (s.d_out.cap == 0) {
     if ((rc = dev_reserve(ctx, s.d_out, std::max<size_t>(len / 2, 1 << 20)))) return rc;
   }
@@ -499,13 +544,18 @@ int slot_enqueue(bvcf_ctx *ctx, Slot &s, bool upload) {
       dos_rows = est;
     }
   }
-  if ((rc = dev_reserve(ctx, s.d_diags, (size_t)ctx->diag_cap * DIAG_WORDS * 4))) return rc;
-  if (upload) CK(cudaMemcpyAsync(s.d_in.p, s.h_src, len, cudaMemcpyHostToDevice, s.stream));
+  s.diag_cap = ctx->diag_cap;
+  if ((rc = dev_reserve(ctx, s.d_diags, (size_t)s.diag_cap * DIAG_WORDS * 4))) return rc;
+  if (upload && s.bgzf) {
+    if ((rc = slot_inflate(ctx, s, comp_len))) return rc;
+  } else if (upload) {
+    CK(cudaMemcpyAsync(s.d_in.p, s.h_src, len, cudaMemcpyHostToDevice, s.stream));
+  }
   CK(cudaMemsetAsync((uint8_t *)s.d_in.p + len, '\n', buf_len - len, s.stream));
   CK(cudaMemsetAsync(s.d_ctr, 0, sizeof(RunCounters), s.stream));
-  rc = enqueue_pipeline(ctx, s.sc, s.stream, (const uint8_t *)s.d_in.p, 0, len, buf_len, (uint8_t *)s.d_out.p, s.d_out.cap,
+  rc = enqueue_pipeline(ctx, s.sc, s.stream, (const uint8_t *)s.d_in.p, s.skip, len, buf_len, (uint8_t *)s.d_out.p, s.d_out.cap,
                         s.d_ctr, (int8_t *)s.d_dosage.p, dos_rows, (uint8_t *)s.d_loci.p, s.d_loci.cap,
-                        (unsigned long long *)s.d_loci_off.p, (uint32_t *)s.d_diags.p, nullptr);
+                        (unsigned long long *)s.d_loci_off.p, (uint32_t *)s.d_diags.p, s.diag_cap, nullptr);
   if (rc) return rc;
   CK(cudaMemcpyAsync(s.h_ctr, s.d_ctr, sizeof(RunCounters), cudaMemcpyDeviceToHost, s.stream));
   CK(cudaEventRecord(s.done, s.stream));
@@ -618,7 +668,12 @@ void bvcf_destroy(bvcf_ctx *ctx) {
   for (auto &s : ctx->slots) {
     if (s.stream) cudaStreamDestroy(s.stream);
     if (s.done) cudaEventDestroy(s.done);
-    for (DevBuf *b : {&s.d_in, &s.d_out, &s.d_dosage, &s.d_loci, &s.d_loci_off, &s.d_diags}) dev_free(*b);
+    for (DevBuf *b : {&s.d_in, &s.d_out, &s.d_dosage, &s.d_loci, &s.d_loci_off, &s.d_diags, &s.d_comp, &s.d_blocks, &s.d_fields,
+                      &s.d_field_off, &s.d_diag_starts})
+      dev_free(*b);
+    if (s.d_bad) cudaFree(s.d_bad);
+    if (s.h_bad) cudaFreeHost(s.h_bad);
+    if (s.h_stage) cudaFreeHost(s.h_stage);
     scratch_free(s.sc);
     if (s.d_ctr) cudaFree(s.d_ctr);
     if (s.h_ctr) cudaFreeHost(s.h_ctr);
@@ -728,6 +783,7 @@ int bvcf_submit(bvcf_ctx *ctx, uint64_t seq, const uint8_t *chunk, size_t len) {
   if (!s) return BVCF_E_STATE;
   cudaSetDevice(ctx->device);
   s->busy = true; s->seq = seq; s->h_src = chunk; s->len = len; s->retries = 0;
+  s->bgzf = false; s->skip = 0; s->text_len = len; s->tail_len = 0;
   const int rc = slot_enqueue(ctx, *s, true);
   if (rc) s->busy = false;
   return rc;
@@ -739,11 +795,17 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
   Slot *s = find_slot(ctx, seq);
   if (!s) return BVCF_E_STATE;
   cudaSetDevice(ctx->device);
+  ctx->last_error.clear();
   const DevCfg &dc = ctx->dcfg;
   static const bool trace = getenv("BVCF_TRACE") != nullptr;  // experiments: where a collect spends its time
   const auto t_begin = std::chrono::steady_clock::now();
   for (;;) {
     CK(cudaEventSynchronize(s->done));
+    if (s->bgzf && s->h_bad[0]) {  // a corrupt member: whatever the pipeline made of its text is not looked at
+      ctx->last_error = std::to_string(s->h_bad[0]) + " bgzf block(s) failed to inflate or failed their CRC-32 / ISIZE check";
+      return BVCF_E_ARG;
+    }
+    if (s->bgzf && s->len > s->skip && (s->h_bad[1] & 0xFFu) != '\n') return BVCF_E_NOT_ALIGNED;
     const RunCounters &c = *s->h_ctr;
     bool again = false;
     if (c.slot_overflow) {                                              // lines shorter than assumed: more line slots
@@ -782,7 +844,9 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
         again = true;
       }
     }
-    if (c.n_diags > ctx->diag_cap) { ctx->diag_cap = c.n_diags + c.n_diags / 4; again = true; }  // every log line or none
+    // every log line or none.  Compared with the capacity this chunk ran with: another slot may have raised ctx->diag_cap
+    // since, and this slot's buffer is still the old size
+    if (c.n_diags > s->diag_cap) { ctx->diag_cap = std::max(ctx->diag_cap, c.n_diags + c.n_diags / 4); again = true; }
     if (c.scratch_overflow) { s->sc.scratch_cap = c.scratch_cursor + c.scratch_cursor / 4 + (1ull << 20); again = true; }
     if (c.slow_overflow) { s->sc.slow_cap = c.n_slow + c.n_slow / 4 + 1024; again = true; }
     if (!again) break;
@@ -832,7 +896,7 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
   // <= diag_cap: larger counts re-ran the chunk above.  A caller that takes no diagnostics does not pay for them: on
   // sites-only input with 9 % rejected alleles their copy, decode and sort was 3.6 ms of every 128 MiB chunk, more than
   // its PCIe time
-  const uint32_t nd = (diags || n_diags) ? c.n_diags : 0u;
+  const uint32_t nd = (diags || n_diags) ? std::min(c.n_diags, s->diag_cap) : 0u;
   if (nd) {
     s->h_diag_raw.resize((size_t)nd * DIAG_WORDS);
     CK(cudaMemcpyAsync(s->h_diag_raw.data(), s->d_diags.p, (size_t)nd * DIAG_WORDS * 4, cudaMemcpyDeviceToHost, s->stream));
@@ -865,7 +929,7 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
   if (n_diags) *n_diags = s->h_diags.size();
   if (stats) {
     stats->n_lines = c.n_lines; stats->n_records = c.n_records; stats->n_rows = c.row_cursor;
-    stats->in_bytes = s->len; stats->out_bytes = c.out_cursor; stats->retries = s->retries;
+    stats->in_bytes = s->len - s->skip; stats->out_bytes = c.out_cursor; stats->retries = s->retries;
   }
   return BVCF_OK;
 }
@@ -933,7 +997,7 @@ int bvcf_resident_run_at(bvcf_ctx *ctx, size_t begin, size_t len, bvcf_chunk_sta
     rc = enqueue_pipeline(ctx, ctx->r_sc, ctx->r_stream, (const uint8_t *)ctx->r_in.p, begin, len, buf_len,
                           (uint8_t *)ctx->r_out.p, ctx->r_out.cap, ctx->r_d_ctr, (int8_t *)ctx->r_dosage.p, dos_rows,
                           (uint8_t *)ctx->r_loci.p, ctx->r_loci.cap, (unsigned long long *)ctx->r_loci_off.p,
-                          (uint32_t *)ctx->r_diags.p, times ? &timing : nullptr);
+                          (uint32_t *)ctx->r_diags.p, ctx->diag_cap, times ? &timing : nullptr);
     if (rc) return rc;
     CK(cudaMemcpyAsync(ctx->r_h_ctr, ctx->r_d_ctr, sizeof(RunCounters), cudaMemcpyDeviceToHost, ctx->r_stream));
     CK(cudaStreamSynchronize(ctx->r_stream));
@@ -1020,6 +1084,9 @@ static int bgzf_walk(const uint8_t *c, size_t n, std::vector<InflateBlock> *bloc
     if (isize && blocks) {
       InflateBlock b;
       b.in_off = p + 12 + xlen; b.in_len = (uint32_t)(bsize - 12 - xlen - 8); b.out_off = out; b.out_len = isize;
+      b.crc = (uint32_t)c[p + bsize - 8] | ((uint32_t)c[p + bsize - 7] << 8) | ((uint32_t)c[p + bsize - 6] << 16) |
+              ((uint32_t)c[p + bsize - 5] << 24);
+      b.pad = 0;
       blocks->push_back(b);
     }
     out += isize;
@@ -1040,6 +1107,7 @@ int bvcf_bgzf_text_bytes(const void *comp, size_t comp_len, uint64_t *text_bytes
 int bvcf_resident_inflate_bgzf(bvcf_ctx *ctx, const void *comp, size_t comp_len, size_t dst_offset, size_t *text_bytes) {
   if (!ctx || !comp) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
+  ctx->last_error.clear();
   std::vector<InflateBlock> blocks;
   uint64_t total = 0;
   int rc = bgzf_walk((const uint8_t *)comp, comp_len, &blocks, &total);
@@ -1064,7 +1132,84 @@ int bvcf_resident_inflate_bgzf(bvcf_ctx *ctx, const void *comp, size_t comp_len,
   uint32_t bad = 0;
   CK(cudaMemcpyAsync(&bad, ctx->r_d_bad, 4, cudaMemcpyDeviceToHost, ctx->r_stream));
   CK(cudaStreamSynchronize(ctx->r_stream));
-  if (bad) { ctx->last_error = std::to_string(bad) + " bgzf block(s) did not inflate to their ISIZE"; return BVCF_E_ARG; }
+  if (bad) { ctx->last_error = std::to_string(bad) + " bgzf block(s) failed to inflate or failed their CRC-32 / ISIZE check"; return BVCF_E_ARG; }
+  return BVCF_OK;
+}
+
+int bvcf_submit_bgzf(bvcf_ctx *ctx, uint64_t seq, const uint8_t *comp, size_t comp_len, size_t skip, const uint8_t *tail,
+                     size_t tail_len) {
+  if (!ctx || (!comp && comp_len) || (!tail && tail_len)) return BVCF_E_ARG;
+  if (!ctx->header_set) return BVCF_E_STATE;
+  if (find_slot(ctx, seq)) return BVCF_E_STATE;
+  Slot *s = nullptr;
+  for (auto &x : ctx->slots)
+    if (!x.busy) { s = &x; break; }
+  if (!s) return BVCF_E_STATE;
+  ctx->last_error.clear();
+  s->blocks.clear();
+  uint64_t text = 0;
+  int rc = comp_len ? bgzf_walk(comp, comp_len, &s->blocks, &text) : 0;
+  if (rc) { ctx->last_error = "not whole bgzf blocks"; return rc; }
+  if (skip > text) return BVCF_E_ARG;
+  const uint64_t len = text + tail_len;
+  if (len > ctx->cfg.max_chunk_bytes || len >= (1ull << 31) || s->blocks.size() >= (1ull << 31)) return BVCF_E_TOO_LARGE;
+  if (tail_len && tail[tail_len - 1] != '\n') return BVCF_E_NOT_ALIGNED;  // (an empty tail: checked on the device)
+  cudaSetDevice(ctx->device);
+  // pinned staging: compressed bytes | block table | tail, so that the copies below are asynchronous
+  const size_t tab_off = round_up(comp_len, 16), tail_off = tab_off + s->blocks.size() * sizeof(InflateBlock);
+  const size_t need = tail_off + tail_len;
+  if (need > s->h_stage_cap || !s->h_stage) {
+    if (s->h_stage) cudaFreeHost(s->h_stage);
+    s->h_stage = nullptr;
+    s->h_stage_cap = 0;
+    CK(cudaMallocHost(&s->h_stage, need + need / 4 + 4096));
+    s->h_stage_cap = need + need / 4 + 4096;
+  }
+  if (comp_len) memcpy(s->h_stage, comp, comp_len);
+  if (!s->blocks.empty()) memcpy(s->h_stage + tab_off, s->blocks.data(), s->blocks.size() * sizeof(InflateBlock));
+  if (tail_len) memcpy(s->h_stage + tail_off, tail, tail_len);
+  s->busy = true; s->seq = seq; s->h_src = nullptr; s->len = len; s->retries = 0;
+  s->bgzf = true; s->skip = skip; s->text_len = text; s->tail_len = tail_len;
+  rc = slot_enqueue(ctx, *s, true, comp_len);
+  if (rc) s->busy = false;
+  return rc;
+}
+
+int bvcf_diag_fields(bvcf_ctx *ctx, uint64_t seq, const uint8_t **text, const uint64_t **off) {
+  if (!ctx || !text || !off) return BVCF_E_ARG;
+  Slot *s = find_slot(ctx, seq);
+  if (!s) return BVCF_E_STATE;
+  cudaSetDevice(ctx->device);
+  const size_t n = s->h_diags.size();
+  s->h_field_off.assign(n + 1, 0);
+  if (n) {
+    if (n >= (1ull << 32)) return BVCF_E_TOO_LARGE;
+    s->h_diag_starts.resize(n);
+    for (size_t i = 0; i < n; i++) s->h_diag_starts[i] = s->h_diags[i].line_start;
+    int rc;
+    if ((rc = dev_reserve(ctx, s->d_diag_starts, n * 8))) return rc;
+    if ((rc = dev_reserve(ctx, s->d_field_off, (n + 1) * 8))) return rc;
+    CK(cudaMemcpyAsync(s->d_diag_starts.p, s->h_diag_starts.data(), n * 8, cudaMemcpyHostToDevice, s->stream));
+    const unsigned long long *st = (const unsigned long long *)s->d_diag_starts.p;
+    unsigned long long *fo = (unsigned long long *)s->d_field_off.p;
+    bvcf_diag_fields_len_kernel<<<1, 1024, 0, s->stream>>>((const uint8_t *)s->d_in.p, s->len, st, (uint32_t)n, fo);
+    ctx->launches++;
+    CK(cudaMemcpyAsync(s->h_field_off.data(), fo, (n + 1) * 8, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    const size_t total = (size_t)s->h_field_off[n];
+    s->h_fields.resize(total);
+    if (total) {
+      if ((rc = dev_reserve(ctx, s->d_fields, total))) return rc;
+      bvcf_diag_fields_copy_kernel<<<(unsigned)std::min<size_t>((n + 7) / 8, 1184), 256, 0, s->stream>>>(
+          (const uint8_t *)s->d_in.p, st, fo, (uint32_t)n, (uint8_t *)s->d_fields.p);
+      ctx->launches++;
+      CK(cudaMemcpyAsync(s->h_fields.data(), s->d_fields.p, total, cudaMemcpyDeviceToHost, s->stream));
+      CK(cudaStreamSynchronize(s->stream));
+    }
+    CK(cudaGetLastError());
+  }
+  *text = s->h_fields.data();
+  *off = s->h_field_off.data();
   return BVCF_OK;
 }
 

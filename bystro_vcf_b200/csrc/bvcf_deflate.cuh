@@ -9,13 +9,13 @@
 //   * Encoding: DEFLATE fixed Huffman codes (RFC 1951 3.2.6) -- no tree to build or ship; every lane knows its token's
 //     bits, a warp prefix sum places them, and they are OR-ed into the (zeroed) output words with reductions
 //     (RED.OR: fire and forget).
-//   * CRC-32 of the slice (gzip's trailer): each lane takes a 1.5 KiB run with the byte table, and the runs are joined
-//     with x^(8n) mod P multiplications (the combine identity zlib's crc32_combine uses).
+//   * CRC-32 of the slice (gzip's trailer): crc_warp (bvcf_crc.cuh), each lane a 1.5 KiB run.
 // bvcf_deflate_pack_kernel then moves the blocks, now of known size, back to back.
 // This is a throughput-first compressor (single candidate per hash, no lazy matching, fixed codes): sample-name lists
 // deflate about 2.3x with it where `gzip -6` reaches 3-4x.
 #pragma once
 #include "bvcf_common.cuh"
+#include "bvcf_crc.cuh"
 
 namespace bvcf {
 
@@ -31,19 +31,6 @@ struct DeflateParams {
   uint32_t *sizes;              // bytes of each finished block
   uint32_t n_blocks;
 };
-
-__device__ __forceinline__ uint32_t crc_multmodp(uint32_t a, uint32_t b) {  // a * b mod P, reflected CRC-32 polynomial
-  uint32_t m = 1u << 31, p = 0;
-  for (;;) {
-    if (a & m) {
-      p ^= b;
-      if ((a & (m - 1)) == 0) break;
-    }
-    m >>= 1;
-    b = (b & 1u) ? (b >> 1) ^ 0xEDB88320u : b >> 1;
-  }
-  return p;
-}
 
 // the bits of one DEFLATE token, LSB first, and their count (at most 31)
 __device__ __forceinline__ uint32_t def_rev(uint32_t code, int bits) { return __brev(code) >> (32 - bits); }
@@ -102,32 +89,10 @@ __global__ void __launch_bounds__(32) bvcf_deflate_kernel(const DeflateParams p)
   // the DEFLATE bits start at byte 18: stream bit b lives in bit (b + 16) % 32 of word (b + 16) / 32 of this view
   uint32_t *sw = reinterpret_cast<uint32_t *>(slot + 16);
   for (int i = lane; i < (1 << DEF_HASH_BITS); i += 32) s_hash[i] = 0;
-  for (int i = lane; i < 256; i += 32) {  // CRC-32 byte table
-    uint32_t c = (uint32_t)i;
-    for (int k = 0; k < 8; k++) c = (c & 1u) ? (c >> 1) ^ 0xEDB88320u : c >> 1;
-    s_crc[i] = c;
-  }
+  crc_table_init(s_crc, lane);
   __syncwarp();
 
-  // ---- CRC-32: lane l takes bytes [l * run, (l + 1) * run), then crc(A || B) = crc(A) * x^(8 |B|) + crc(B) ----
-  uint32_t crc;
-  {
-    const uint32_t run = (len + 31u) / 32u;
-    const uint32_t lo = (uint32_t)lane * run < len ? (uint32_t)lane * run : len, hi = lo + run < len ? lo + run : len;
-    uint32_t c = 0xFFFFFFFFu;
-    for (uint32_t i = lo; i < hi; i++) c = s_crc[(c ^ in[i]) & 0xFFu] ^ (c >> 8);
-    c ^= 0xFFFFFFFFu;                                   // the finished CRC of this lane's run (0 for an empty run)
-    const uint32_t after = len - hi;                    // bytes that follow it: multiply by x^(8 * after) mod P
-    uint32_t x = 0x00800000u, f = 0x80000000u;          // x^8 and 1 in the reflected representation
-    for (uint32_t n = after; n; n >>= 1) {
-      if (n & 1u) f = crc_multmodp(x, f);
-      x = crc_multmodp(x, x);
-    }
-    c = hi > lo ? crc_multmodp(f, c) : 0u;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) c ^= __shfl_xor_sync(FULL, c, d);
-    crc = c;
-  }
+  const uint32_t crc = crc_warp([&](uint32_t i) { return (uint32_t)in[i]; }, len, lane, s_crc);
 
   // ---- LZ77 + fixed Huffman ----
   uint32_t bitpos = 3;   // BFINAL = 1, BTYPE = 01 (fixed codes): bits 1, 1, 0 -> value 3, written with the header below

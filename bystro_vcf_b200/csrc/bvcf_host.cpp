@@ -4,7 +4,8 @@
 // The per-line work happens on the GPU(s).  Threads mirror the reference's producer + worker pool
 // (main.go:345-380) with GPUs as the workers:
 //   reader     finds newline-aligned chunk boundaries; stdin is read straight into pinned buffers, a regular
-//              --in file is memory-mapped and only the boundaries are computed here;
+//              --in file is memory-mapped and only the boundaries are computed here.  A .vcf.gz (bgzf) input is cut
+//              into groups of whole blocks instead (BgzfIn / plan rule below): the compressed bytes go to the GPUs;
 //   GPU worker one per GPU (chunk k goes to GPU k mod N): stages its chunks into its own pinned ring (parallel
 //              memcpy out of the mapping), keeps n_slots chunks in flight on its context, and -- when it is chunk
 //              k's turn -- writes the rows, appends the dosage batch to the Arrow file and logs the diagnostics,
@@ -162,14 +163,8 @@ const char *diag_text(int code) {  // main.go:41-51
   return "?";
 }
 
-// one of the reference's log.Printf lines (main.go:730-986); `line` points at the diagnosed line (CHROM \t POS \t ...)
-void log_one_diag(const char *line, size_t avail, const bvcf_diag &d) {
-  const char *end = line + avail;
-  const char *t0 = (const char *)memchr(line, '\t', avail);
-  if (!t0) return;
-  const char *t1 = (const char *)memchr(t0 + 1, '\t', end - t0 - 1);
-  if (!t1) return;
-  const std::string chrom(line, t0), pos(t0 + 1, t1);
+// one of the reference's log.Printf lines (main.go:730-986)
+void print_diag(const std::string &chrom, const std::string &pos, const bvcf_diag &d) {
   const char *msg = diag_text(d.code);
   switch (d.code) {
     case BVCF_DIAG_SAME: fprintf(stderr, "%s:%s : %s\n", chrom.c_str(), pos.c_str(), msg); break;
@@ -177,6 +172,24 @@ void log_one_diag(const char *line, size_t avail, const bvcf_diag &d) {
       fprintf(stderr, "%s:%s ALT#%d %s\n", chrom.c_str(), pos.c_str(), d.alt_no, msg); break;
     case BVCF_DIAG_POS_LIST: fprintf(stderr, "%s:%s %s\n", chrom.c_str(), pos.c_str(), msg); break;
     default: fprintf(stderr, "%s:%s ALT #%d %s\n", chrom.c_str(), pos.c_str(), d.alt_no, msg);
+  }
+}
+// `line` points at the diagnosed line (CHROM \t POS \t ...)
+void log_one_diag(const char *line, size_t avail, const bvcf_diag &d) {
+  const char *end = line + avail;
+  const char *t0 = (const char *)memchr(line, '\t', avail);
+  if (!t0) return;
+  const char *t1 = (const char *)memchr(t0 + 1, '\t', end - t0 - 1);
+  if (!t1) return;
+  print_diag(std::string(line, t0), std::string(t0 + 1, t1), d);
+}
+// the diagnostics of a bgzf chunk, whose text is on the device only: CHROM \t POS of each (bvcf_diag_fields)
+void log_diag_fields(const uint8_t *text, const uint64_t *off, const bvcf_diag *d, size_t n) {
+  for (size_t k = 0; k < n; k++) {
+    const char *f = (const char *)text + off[k];
+    const size_t m = (size_t)(off[k + 1] - off[k]);
+    const char *t0 = (const char *)memchr(f, '\t', m);
+    if (t0) print_diag(std::string(f, t0), std::string(t0 + 1, f + m), d[k]);
   }
 }
 // the diagnostics of a chunk that is still pinned: every entry carries its line's offset
@@ -190,16 +203,20 @@ struct Chunk {
   uint8_t *buf = nullptr;        // pinned buffer holding the chunk (filled by the reader, or by the worker from `src`)
   const uint8_t *src = nullptr;  // memory-mapped input: where the chunk's bytes are
   size_t len = 0;
+  // bgzf input: buf holds whole blocks, the chunk's text is inflate(buf)[skip:] + tail (bvcf_submit_bgzf)
+  bool gz = false;
+  size_t skip = 0;
+  std::string tail;
 };
 
 // bounded FIFO between the reader and one GPU worker
 class ChunkQueue {
  public:
   explicit ChunkQueue(size_t cap) : cap_(cap) {}
-  void push(const Chunk &c) {
+  void push(Chunk c) {
     std::unique_lock<std::mutex> l(m_);
     cv_.wait(l, [&] { return q_.size() < cap_; });
-    q_.push_back(c);
+    q_.push_back(std::move(c));
     cv_.notify_all();
   }
   void close() {
@@ -212,7 +229,7 @@ class ChunkQueue {
     std::unique_lock<std::mutex> l(m_);
     if (block) cv_.wait(l, [&] { return !q_.empty() || closed_; });
     if (q_.empty()) return closed_ ? -1 : 0;
-    c = q_.front();
+    c = std::move(q_.front());
     q_.pop_front();
     cv_.notify_all();
     return 1;
@@ -264,11 +281,16 @@ bool looks_bgzf(const uint8_t *p, size_t n) {
 }
 size_t bgzf_block_size(const uint8_t *p, size_t n) {  // 0: header incomplete
   if (n < 18) return 0;
+  if (p[0] != 0x1f || p[1] != 0x8b || p[2] != 8 || !(p[3] & 4)) fatal("bgzf input: bytes that are not a bgzf block");
   const size_t xlen = (size_t)p[10] | ((size_t)p[11] << 8);
   if (n < 12 + xlen) return 0;
   for (size_t q = 12; q + 4 <= 12 + xlen;) {
     const size_t slen = (size_t)p[q + 2] | ((size_t)p[q + 3] << 8);
-    if (p[q] == 'B' && p[q + 1] == 'C' && slen == 2) return ((size_t)p[q + 4] | ((size_t)p[q + 5] << 8)) + 1;
+    if (p[q] == 'B' && p[q + 1] == 'C' && slen == 2) {
+      const size_t bsize = ((size_t)p[q + 4] | ((size_t)p[q + 5] << 8)) + 1;
+      if (bsize < 12 + xlen + 8) fatal("bgzf input: a block smaller than its header and trailer");
+      return bsize;
+    }
     q += 4 + slen;
   }
   fatal("gzip input without the bgzf BC subfield: decompress it first (gzip -dc | ...)");
@@ -317,6 +339,193 @@ std::vector<uint8_t> bgzf_block_host(const uint8_t *text, size_t n) {
 }
 const uint8_t BGZF_EOF[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 
+// main.go:250-294 on the first bytes of the text: EOL width, the ##fileformat check, the #CHROM line.  true when found;
+// false when more text is needed (fatal at eof)
+bool find_preamble(const uint8_t *p, size_t n, bool eof, std::string &chrom_line, size_t &data_off, int &eol_width) {
+  if (n == 0 && eof) fatal("Not a VCF file");
+  const uint8_t *nl = (const uint8_t *)memchr(p, '\n', n);
+  if (!nl) { if (eof) fatal("Not a VCF file"); return false; }
+  size_t first_end = nl - p;
+  eol_width = 1;
+  if (first_end > 0 && p[first_end - 1] == '\r') { eol_width = 2; first_end--; }
+  if (!memmem(p, first_end, "##fileformat=VCFv4", 18)) fatal("Not a VCF file");  // main.go:256-264
+  for (size_t q = (nl - p) + 1; q < n;) {
+    const uint8_t *e = (const uint8_t *)memchr(p + q, '\n', n - q);
+    if (!e) break;
+    size_t cl = (e - p) - q;
+    cl = cl + 1 >= (size_t)eol_width ? cl + 1 - eol_width : 0;
+    if (cl >= 6 && memcmp(p + q, "#CHROM", 6) == 0 && (cl == 6 || p[q + 6] == '\t')) {
+      chrom_line.assign((const char *)p + q, cl);
+      data_off = (e - p) + 1;
+      return true;
+    }
+    q = (e - p) + 1;
+  }
+  if (eof) fatal("No header found");  // main.go:293
+  return false;
+}
+
+// The blocks of a bgzf input, memory-mapped or read from a pipe as they are needed.  Blocks without text (the EOF
+// block among them) are left out of the list; offsets are absolute in the compressed stream.
+class BgzfIn {
+ public:
+  struct Blk { size_t off, size; uint64_t start; uint32_t isize; };
+  BgzfIn(int fd, const uint8_t *map, size_t map_len, std::vector<uint8_t> &head) : fd_(fd), map_(map), map_len_(map_len) {
+    if (!map_) buf_.swap(head);
+    eof_ = map_ != nullptr;
+  }
+  // block i exists (reads and walks headers until it does or the input ends; a truncated block is fatal)
+  bool has(size_t i) {
+    while (blk_.size() <= i && !walked_) {
+      fill(walk_ + (1u << 16) + 18);
+      if (walk_ == end()) { walked_ = true; break; }
+      size_t bs = bgzf_block_size(at(walk_), end() - walk_);
+      if (bs && walk_ + bs > end()) { fill(walk_ + bs); }
+      bs = bgzf_block_size(at(walk_), end() - walk_);
+      if (!bs || walk_ + bs > end()) fatal("bgzf input: truncated block at the end");
+      const uint8_t *e = at(walk_ + bs - 4);
+      const uint32_t isize = (uint32_t)e[0] | ((uint32_t)e[1] << 8) | ((uint32_t)e[2] << 16) | ((uint32_t)e[3] << 24);
+      if (isize) blk_.push_back({walk_, bs, text_, isize});
+      text_ += isize;
+      walk_ += bs;
+    }
+    return i < blk_.size();
+  }
+  const Blk &operator[](size_t i) const { return blk_[i]; }
+  size_t off(size_t i) { return has(i) ? blk_[i].off : walk_; }  // where block i starts (the end past the last)
+  const uint8_t *at(size_t abs) const { return map_ ? map_ + abs : buf_.data() + (abs - base_); }
+  // block i inflated on the host, its CRC-32 and ISIZE checked
+  std::string inflate_block(size_t i) {
+    const Blk &b = blk_[i];
+    const uint8_t *p = at(b.off);
+    const size_t xlen = (size_t)p[10] | ((size_t)p[11] << 8);
+    std::string text(b.isize, '\0');
+    z_stream z{};
+    if (inflateInit2(&z, -15) != Z_OK) fatal("zlib: inflateInit2 failed");
+    z.next_in = const_cast<Bytef *>(p + 12 + xlen); z.avail_in = (uInt)(b.size - 12 - xlen - 8);
+    z.next_out = (Bytef *)text.data(); z.avail_out = b.isize;
+    const int zr = inflate(&z, Z_FINISH);
+    const size_t got = z.total_out;
+    inflateEnd(&z);
+    const uint8_t *t = p + b.size - 8;
+    const uint32_t crc = (uint32_t)t[0] | ((uint32_t)t[1] << 8) | ((uint32_t)t[2] << 16) | ((uint32_t)t[3] << 24);
+    if (zr != Z_STREAM_END || got != b.isize || crc32(crc32(0L, Z_NULL, 0), (const Bytef *)text.data(), (uInt)got) != crc)
+      fatal("bgzf input: a corrupt block (inflate, CRC-32 or ISIZE check failed)");
+    return text;
+  }
+  // the first `want` text bytes (fewer at the end of the input): the preamble
+  std::string prefix(size_t want) {
+    std::string out;
+    for (size_t i = 0; out.size() < want && has(i); i++) out += inflate_block(i);
+    return out;
+  }
+  // pipe input: bytes before `abs` are no longer needed
+  void release_before(size_t abs) {
+    if (map_ || abs - base_ < (64u << 20)) return;
+    buf_.erase(buf_.begin(), buf_.begin() + (abs - base_));
+    base_ = abs;
+  }
+
+ private:
+  size_t end() const { return map_ ? map_len_ : base_ + buf_.size(); }
+  void fill(size_t want) {  // bytes up to absolute offset `want` (or the end of the input)
+    while (!eof_ && end() < want) {
+      const size_t old = buf_.size();
+      buf_.resize(old + (8u << 20));
+      const ssize_t r = read(fd_, buf_.data() + old, 8u << 20);
+      if (r < 0) { buf_.resize(old); if (errno == EINTR) continue; fatal(std::string("read: ") + strerror(errno)); }
+      buf_.resize(old + (size_t)r);
+      if (r == 0) eof_ = true;
+    }
+  }
+  int fd_;
+  const uint8_t *map_;
+  size_t map_len_;
+  std::vector<uint8_t> buf_;
+  size_t base_ = 0, walk_ = 0;
+  uint64_t text_ = 0;
+  bool eof_ = false, walked_ = false;
+  std::vector<Blk> blk_;
+};
+
+// The groups of a bgzf input (the rule of bystro_vcf_b200/bgzf.py plan_groups): blocks are taken while a group's text
+// is below chunk_bytes; the first group starts at the block holding text byte data_off.  The line that crosses into the
+// next group belongs to this one: the next group's text up to and including its first newline, inflated here, is this
+// group's tail and the next group's skip; a next group with no newline is merged into this one.  The last group ends at
+// the last newline of the input (an unterminated last line is dropped, main.go:354-357): the blocks from the one
+// holding it on are inflated here and left out, their text up to it is the tail.  emit(lo_block, hi_block, skip, tail)
+// receives each group in order (hi_block: one past its last block).
+template <class Emit>
+void plan_bgzf_groups(BgzfIn &in, uint64_t data_off, size_t chunk_bytes, size_t cap, Emit emit_out) {
+  size_t b = 0;
+  while (in.has(b) && in[b].start + in[b].isize <= data_off) b++;
+  if (!in.has(b)) return;
+  size_t skip = (size_t)(data_off - in[b].start);
+  auto take = [&](size_t i) {
+    size_t e = i;
+    while (in.has(e) && in[e].start - in[i].start < chunk_bytes) e++;
+    return e;
+  };
+  auto text_of = [&](size_t lo, size_t hi) { return (uint64_t)((in.has(hi) ? in[hi].start : in[hi - 1].start + in[hi - 1].isize) - in[lo].start); };
+  // one group is held back: the last group may still hand its text to it
+  struct G { size_t lo, hi, skip; std::string tail; bool set = false; } prev;
+  auto emit = [&](size_t lo, size_t hi, size_t skip_, std::string tail) {
+    const uint64_t text = hi > lo ? text_of(lo, hi) : 0;
+    if (text + tail.size() > cap) fatal("a single line exceeds the chunk capacity; raise --chunkBytes");
+    if (text - skip_ + tail.size() == 0) return;
+    if (prev.set) emit_out(prev.lo, prev.hi, prev.skip, prev.tail);
+    prev.lo = lo; prev.hi = hi; prev.skip = skip_; prev.tail = std::move(tail); prev.set = true;
+  };
+  for (;;) {
+    size_t e = take(b);
+    bool found = false;
+    std::string tail;
+    while (in.has(e) && !found) {
+      const size_t e2 = take(e);
+      tail.clear();
+      for (size_t j = e; j < e2 && !found; j++) {  // the continuation: inflated until its newline
+        const std::string t = in.inflate_block(j);
+        const size_t k = t.find('\n');
+        if (k != std::string::npos) { tail.append(t, 0, k + 1); found = true; }
+        else tail += t;
+      }
+      if (!found) e = e2;  // no newline in the next group: it joins this one
+    }
+    if (found) {
+      const size_t n = tail.size();
+      emit(b, e, skip, std::move(tail));
+      b = e; skip = n;
+      continue;
+    }
+    // the last group [b, n): it ends at the input's last newline
+    size_t f = e;
+    std::string last;
+    bool nl = false;
+    while (f > b && !nl) {
+      f--;
+      const std::string t = in.inflate_block(f);
+      const size_t k = t.rfind('\n');
+      if (k != std::string::npos) { last.assign(t, 0, k + 1); nl = true; }
+    }
+    if (nl) {
+      const uint64_t data_start = in[b].start + skip;
+      if (data_start < in[f].start) {
+        emit(b, f, skip, std::move(last));
+      } else if (data_start - in[f].start < last.size()) {  // the rest is inside the block of the last newline
+        std::string rest = last.substr((size_t)(data_start - in[f].start));
+        if (prev.set) {
+          prev.tail += rest;  // the previous group's tail takes it
+          if (text_of(prev.lo, prev.hi) + prev.tail.size() > cap) fatal("a single line exceeds the chunk capacity; raise --chunkBytes");
+        } else {
+          emit(f, f, 0, std::move(rest));
+        }
+      }
+    }
+    if (prev.set) emit_out(prev.lo, prev.hi, prev.skip, prev.tail);
+    return;
+  }
+}
+
 // readVcf over the resident regions, for compressed streams on either side: bgzf input is inflated on the GPU
 // (compressed_in), --bgzfOut rows are deflated there
 int run_resident(const Config &config, int in_fd, const uint8_t *map, size_t map_len, std::vector<uint8_t> &head, int out_fd,
@@ -344,27 +553,7 @@ int run_resident(const Config &config, int in_fd, const uint8_t *map, size_t map
   for (size_t want = 1u << 20;; want *= 4) {
     fill(want);
     const std::string t = compressed_in ? bgzf_inflate_host(at(0), avail(), want * 4) : std::string((const char *)at(0), std::min(avail(), want * 4));
-    const char *nl = (const char *)memchr(t.data(), '\n', t.size());
-    if (!nl) { if (eof) fatal("Not a VCF file"); continue; }
-    size_t first_end = nl - t.data();
-    if (first_end > 0 && t[first_end - 1] == '\r') { eol_width = 2; first_end--; }
-    if (!memmem(t.data(), first_end, "##fileformat=VCFv4", 18)) fatal("Not a VCF file");
-    bool found = false;
-    for (size_t q = (nl - t.data()) + 1; q < t.size();) {
-      const char *e = (const char *)memchr(t.data() + q, '\n', t.size() - q);
-      if (!e) break;
-      size_t cl = (e - t.data()) - q;
-      cl = cl + 1 >= (size_t)eol_width ? cl + 1 - eol_width : 0;
-      if (cl >= 6 && memcmp(t.data() + q, "#CHROM", 6) == 0 && (cl == 6 || t[q + 6] == '\t')) {
-        chrom_line.assign(t.data() + q, cl);
-        data_off = (e - t.data()) + 1;
-        found = true;
-        break;
-      }
-      q = (e - t.data()) + 1;
-    }
-    if (found) break;
-    if (eof) fatal("No header found");
+    if (find_preamble((const uint8_t *)t.data(), t.size(), eof, chrom_line, data_off, eol_width)) break;
   }
   if (!config.sampleListPath.empty() && !config.noOut) {
     FILE *f = fopen(config.sampleListPath.c_str(), "w");
@@ -578,8 +767,8 @@ int main(int argc, char **argv) {
   }
 
   std::vector<uint8_t> head;  // pipe input: what has been read so far
-  {  // .vcf.gz (bgzf): another path altogether
-    bool bz = false;
+  bool bz = false;            // .vcf.gz (bgzf) input
+  {
     if (map) bz = looks_bgzf(map, map_len);
     else {
       head.resize(1 << 16);
@@ -593,20 +782,28 @@ int main(int argc, char **argv) {
       head.resize(got);
       bz = looks_bgzf(head.data(), head.size());
     }
-    if (bz || config.bgzfOut) {
-      if (config.bgzfOut && config.gpus > 1) fatal("--bgzfOut runs on one GPU");
+    if (config.bgzfOut) {  // the rows are deflated where they are, on one GPU's resident regions
+      if (config.gpus > 1) fatal("--bgzfOut runs on one GPU");
       const int rc = run_resident(config, in_fd, map, map_len, head, out_fd, bz);
       if (map) munmap((void *)map, map_len);
       if (out_fd != 1) close(out_fd);
       return rc;
     }
   }
-  // ---- preamble (main.go:250-294): EOL, ##fileformat check, #CHROM line ----
+  // ---- preamble (main.go:250-294): EOL, ##fileformat check, #CHROM line; a bgzf input's is inflated on the host ----
   size_t data_off = 0;
   int eol_width = 1;
   std::string chrom_line;
   bool eof = false;
-  for (bool found = false; !found;) {
+  std::unique_ptr<BgzfIn> gz;
+  if (bz) {
+    gz.reset(new BgzfIn(in_fd, map, map_len, head));
+    for (size_t want = 1u << 20;; want *= 4) {
+      const std::string t = gz->prefix(want);
+      if (find_preamble((const uint8_t *)t.data(), t.size(), t.size() < want, chrom_line, data_off, eol_width)) break;
+    }
+  }
+  while (!gz) {
     const uint8_t *p;
     size_t n;
     if (map) {
@@ -620,27 +817,7 @@ int main(int argc, char **argv) {
       if (r == 0) eof = true;
       p = head.data(); n = head.size();
     }
-    if (n == 0 && eof) fatal("Not a VCF file");
-    const uint8_t *nl = (const uint8_t *)memchr(p, '\n', n);
-    if (!nl) { if (eof) fatal("Not a VCF file"); continue; }
-    size_t first_end = nl - p;
-    if (first_end > 0 && p[first_end - 1] == '\r') { eol_width = 2; first_end--; }
-    if (!memmem(p, first_end, "##fileformat=VCFv4", 18)) fatal("Not a VCF file");  // main.go:256-264
-    size_t q = (nl - p) + 1;
-    while (q < n) {
-      const uint8_t *e = (const uint8_t *)memchr(p + q, '\n', n - q);
-      if (!e) break;
-      size_t cl = (e - p) - q;
-      cl = cl + 1 >= (size_t)eol_width ? cl + 1 - eol_width : 0;
-      if (cl >= 6 && memcmp(p + q, "#CHROM", 6) == 0 && (cl == 6 || p[q + 6] == '\t')) {
-        chrom_line.assign((const char *)p + q, cl);
-        data_off = (e - p) + 1;
-        found = true;
-        break;
-      }
-      q = (e - p) + 1;
-    }
-    if (!found && eof) fatal("No header found");  // main.go:293
+    if (find_preamble(p, n, eof, chrom_line, data_off, eol_width)) break;
   }
   std::vector<std::string> sample_names;
   {
@@ -732,27 +909,36 @@ int main(int argc, char **argv) {
           c.buf = pools[g].take();
           memcpy(c.buf, c.src, c.len);
         }
-        const int rc = bvcf_submit(ctx, c.seq, c.buf, c.len);
+        const int rc = c.gz ? bvcf_submit_bgzf(ctx, c.seq, c.buf, c.len, c.skip, (const uint8_t *)c.tail.data(), c.tail.size())
+                            : bvcf_submit(ctx, c.seq, c.buf, c.len);
         if (rc) { std::lock_guard<std::mutex> l(fatal_m); fatal(std::string("bvcf_submit: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx)); }
-        inflight.push_back(c);
+        inflight.push_back(std::move(c));
       }
       if (inflight.empty()) {
         if (closed) break;
         continue;
       }
-      const Chunk c = inflight.front();
+      const Chunk c = std::move(inflight.front());
       inflight.pop_front();
       const uint8_t *tsv; size_t n; const bvcf_diag *dg; size_t nd;
       bvcf_dosage_batch dos;
       const int rc = bvcf_collect(ctx, c.seq, &tsv, &n, &dos, &dg, &nd, nullptr);
+      int rc2 = 0;
       if (rc) { std::lock_guard<std::mutex> l(fatal_m); fatal(std::string("bvcf_collect: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx)); }
+      const uint8_t *ftext = nullptr;
+      const uint64_t *foff = nullptr;
+      if (c.gz && nd && (rc2 = bvcf_diag_fields(ctx, c.seq, &ftext, &foff))) {
+        std::lock_guard<std::mutex> l(fatal_m);
+        fatal(std::string("bvcf_diag_fields: ") + bvcf_strerror(rc2) + " " + bvcf_last_error(ctx));
+      }
       turn.wait_for(c.seq);  // input order
       if (!config.noOut) write_all(out_fd, tsv, n);
 #ifndef BVCF_NO_ARROW
       if (arrow && dos.n_rows && bvcf_arrow_write(arrow, dos.n_rows, dos.dosage, dos.loci, dos.loci_off))
         fatal(std::string("dosage output: ") + bvcf_arrow_error(arrow));
 #endif
-      log_diags(c.buf, c.len, dg, nd);
+      if (c.gz) log_diag_fields(ftext, foff, dg, nd);
+      else log_diags(c.buf, c.len, dg, nd);
       turn.done();
       bvcf_release(ctx, c.seq);
       pools[g].give(c.buf);
@@ -763,7 +949,23 @@ int main(int argc, char **argv) {
 
   // ---- reader: newline-aligned chunks, chunk k to GPU k mod N ----
   uint64_t seq = 0;
-  if (map) {
+  if (gz) {  // groups of whole bgzf blocks: a mapped input is staged by the workers, a pipe's by the reader
+    plan_bgzf_groups(*gz, data_off, config.chunkBytes, cap, [&](size_t lo_b, size_t hi_b, size_t skip, const std::string &tail) {
+      const size_t lo = gz->off(lo_b), hi = gz->off(hi_b);
+      if (hi - lo > cap) fatal("a bgzf group exceeds the chunk capacity; raise --chunkBytes");
+      Chunk c;
+      c.seq = seq; c.len = hi - lo; c.gz = true; c.skip = skip; c.tail = tail;
+      if (map) {
+        c.src = map + lo;
+      } else {
+        c.buf = pools[seq % n_gpu].take();
+        memcpy(c.buf, gz->at(lo), c.len);
+        gz->release_before(hi);
+      }
+      queues[seq % n_gpu]->push(std::move(c));
+      seq++;
+    });
+  } else if (map) {
     size_t p = data_off;
     // an unterminated last line is dropped (main.go:354-357)
     size_t end = map_len;

@@ -13,11 +13,16 @@
 //     byte i, reading byte (i mod distance) of the source, so even the distance-4 runs of genotype text ("0|0\t"
 //     repeated 64 times per match) move 32 bytes per step instead of waiting on a store-to-load round trip per byte;
 //   * the finished block leaves as coalesced 16-byte stores.
-// Stored, fixed and dynamic blocks are all handled; the gzip CRC32 is not verified (ISIZE is).
+// Stored, fixed and dynamic blocks are all handled.  Every member is checked against its gzip trailer: ISIZE, and the
+// CRC-32 of the text, computed from the shared-memory ring as each piece is flushed (bvcf_crc.cuh), so the check makes
+// no second pass over the text in HBM.  The bit reader is bounded: a stream that would consume more bits than its
+// payload holds (a chain of empty blocks, a missing end-of-block code, a truncated payload) fails its block, and no
+// read goes further than 11 bytes past the payload.
 // (A first version gave a THREAD per block with its text in global memory: 12 GB/s -- every byte of an overlapping
 // match waited for the previous store to come back from L2.)
 #pragma once
 #include "bvcf_common.cuh"
+#include "bvcf_crc.cuh"
 
 namespace bvcf {
 
@@ -26,13 +31,15 @@ struct InflateBlock {
   unsigned long long out_off;  // where its text goes in `out`
   uint32_t in_len;             // payload bytes
   uint32_t out_len;            // ISIZE: bytes of text
+  uint32_t crc;                // CRC-32 of the text (the gzip trailer)
+  uint32_t pad;
 };
 struct InflateParams {
   const uint8_t *comp;
   uint8_t *out;
   const InflateBlock *blocks;
   uint32_t n_blocks;
-  uint32_t *n_bad;             // blocks that failed (corrupt stream, size mismatch)
+  uint32_t *n_bad;             // blocks that failed (corrupt stream, size or CRC-32 mismatch)
 };
 
 constexpr int INF_MAXBITS = 15, INF_MAXL = 288, INF_MAXD = 30;
@@ -44,11 +51,15 @@ struct InfBits {
   int cnt;
   __device__ __forceinline__ void refill() {  // at least 32 bits afterwards
     if (cnt <= 32) {
-      // four bytes at any alignment from two aligned words; past `end` lies the next block's header (or the buffer's
-      // slack): harmless, a valid stream stops at its end-of-block symbol and the text size is checked
-      const uint32_t *wp = reinterpret_cast<const uint32_t *>((uintptr_t)p & ~(uintptr_t)3);
-      const uint32_t sh = (uint32_t)((uintptr_t)p & 3u) * 8u;
-      const uint32_t w = __funnelshift_r(wp[0], wp[1], sh);
+      // four bytes at any alignment from two aligned words; just past `end` lie the member's trailer and the next
+      // block's header (or the buffer's slack): harmless, a valid stream stops at its end-of-block symbol.  Further out
+      // nothing is read -- zeros come in, and overrun() fails the block at its next check
+      uint32_t w = 0;
+      if (p <= end + 4) {
+        const uint32_t *wp = reinterpret_cast<const uint32_t *>((uintptr_t)p & ~(uintptr_t)3);
+        const uint32_t sh = (uint32_t)((uintptr_t)p & 3u) * 8u;
+        w = __funnelshift_r(wp[0], wp[1], sh);
+      }
       buf |= (unsigned long long)w << cnt;
       cnt += 32;
       p += 4;
@@ -60,6 +71,8 @@ struct InfBits {
     buf >>= n; cnt -= n;
     return v;
   }
+  // more bits consumed than the payload holds
+  __device__ __forceinline__ bool overrun() const { return (long long)(p - end) * 8 > (long long)cnt; }
 };
 
 struct InfHuff {
@@ -166,9 +179,12 @@ struct InfOut {
   uint32_t o;          // text bytes produced
   uint32_t flushed;    // text bytes already in global memory (a multiple of INF_PIECE until the end)
   uint32_t out_len;
+  uint32_t crc;        // CRC-32 of the flushed text
+  const uint32_t *crc_tab;  // its byte table, in shared memory
 };
-// text bytes [from, to) ring -> global, all lanes; coalesced 4-byte words where the alignment allows
-__device__ __forceinline__ void inf_flush(const InfOut &w, uint32_t from, uint32_t to, int lane) {
+// text bytes [from, to) ring -> global, all lanes; coalesced 4-byte words where the alignment allows.  Their CRC-32 is
+// folded into w.crc on the way (the bytes are read from the ring, not from HBM)
+__device__ __forceinline__ void inf_flush(InfOut &w, uint32_t from, uint32_t to, int lane) {
   uint8_t *g = w.g;
   uint32_t a = from;
   // bytes up to the first 4-byte boundary of the destination
@@ -188,6 +204,9 @@ __device__ __forceinline__ void inf_flush(const InfOut &w, uint32_t from, uint32
   }
   a += 4 * nw;
   if (a + lane < to) g[a + lane] = w.ring[(a + lane) & INF_RING_MASK];
+  const uint8_t *ring = w.ring;
+  const uint32_t c = crc_warp([&](uint32_t i) { return (uint32_t)ring[(from + i) & INF_RING_MASK]; }, to - from, lane, w.crc_tab);
+  w.crc = crc_shift(w.crc, to - from) ^ c;
 }
 
 // literal/length + distance codes until the end-of-block symbol; every lane runs this in lockstep; returns 0 or an error
@@ -205,7 +224,7 @@ __device__ __forceinline__ int inf_codes(InfBits &b, const InfHuff &lc, const In
       if (lane == 0) asm volatile("st.shared.u8 [%0], %1;\n" ::"r"(w.ring_s + (w.o & INF_RING_MASK)), "r"(sym) : "memory");
       w.o++;
     } else if (sym == 256) {
-      return 0;
+      return b.overrun() ? 18 : 0;
     } else {
       sym -= 257;
       if (sym >= 29) return 3;
@@ -255,7 +274,9 @@ __device__ __forceinline__ int inf_codes(InfBits &b, const InfHuff &lc, const In
 constexpr uint32_t INF_TEXT_MAX = 65536;  // a bgzf block holds at most 64 KiB of text
 constexpr int INF_LBITS = 10, INF_DBITS = 9;  // lookup-table bits of the literal/length and the distance code
 constexpr uint32_t INF_TAB_SHORTS = 2 * (INF_MAXBITS + 1) + INF_MAXL + INF_MAXD + 2 + INF_MAXL + INF_MAXD + 2 + 16;
-constexpr uint32_t INF_SMEM = INF_RING + 2 * INF_TAB_SHORTS + 2 * ((1u << INF_LBITS) + (1u << INF_DBITS));
+constexpr uint32_t INF_LUT_BYTES = 2 * ((1u << INF_LBITS) + (1u << INF_DBITS));
+constexpr uint32_t INF_SMEM = INF_RING + 2 * INF_TAB_SHORTS + INF_LUT_BYTES + 256 * 4;  // ring, code tables, CRC-32 table
+static_assert((INF_RING + 2 * INF_TAB_SHORTS + INF_LUT_BYTES) % 4 == 0, "the CRC-32 table is word-aligned");
 
 __global__ void __launch_bounds__(32) bvcf_inflate_kernel(const InflateParams p) {
   extern __shared__ __align__(16) uint8_t s_inf[];
@@ -266,17 +287,20 @@ __global__ void __launch_bounds__(32) bvcf_inflate_kernel(const InflateParams p)
   short *tabs = reinterpret_cast<short *>(s_inf + INF_RING);
   short *lencnt = tabs, *distcnt = tabs + 16, *lensym = tabs + 32, *distsym = lensym + INF_MAXL, *lengths = distsym + INF_MAXD + 2;
   unsigned short *llut = reinterpret_cast<unsigned short *>(tabs + INF_TAB_SHORTS), *dlut = llut + (1 << INF_LBITS);
+  uint32_t *crc_tab = reinterpret_cast<uint32_t *>(s_inf + INF_RING + 2 * INF_TAB_SHORTS + INF_LUT_BYTES);
+  crc_table_init(crc_tab, lane);  // ordered before its first use by the __syncwarp() in front of every flush
   int err = blk.out_len > INF_TEXT_MAX ? 17 : 0;
   InfBits b;
   b.p = p.comp + blk.in_off; b.end = b.p + blk.in_len; b.buf = 0; b.cnt = 0;
   InfOut w;
   w.ring_s = (uint32_t)__cvta_generic_to_shared(s_inf); w.ring = s_inf; w.g = p.out + blk.out_off;
-  w.o = 0; w.flushed = 0; w.out_len = blk.out_len;
+  w.o = 0; w.flushed = 0; w.out_len = blk.out_len; w.crc = 0; w.crc_tab = crc_tab;
   InfHuff lc, dc;
   lc.count = lencnt; lc.symbol = lensym; dc.count = distcnt; dc.symbol = distsym;
   lc.lut = llut; lc.lut_bits = INF_LBITS; dc.lut = dlut; dc.lut_bits = INF_DBITS;
   int last = 1;
   if (!err) do {
+    if (b.overrun()) { err = 19; break; }  // e.g. a chain of empty blocks running past the payload
     last = (int)b.bits(1);
     const int type = (int)b.bits(2);
     if (type == 0) {  // stored
@@ -295,6 +319,9 @@ __global__ void __launch_bounds__(32) bvcf_inflate_kernel(const InflateParams p)
         w.g[w.o + i] = c;
         s_inf[(w.o + i) & INF_RING_MASK] = c;
       }
+      const uint8_t *src = b.p;
+      const uint32_t c = crc_warp([&](uint32_t i) { return (uint32_t)src[i]; }, len, lane, crc_tab);
+      w.crc = crc_shift(w.crc, len) ^ c;
       w.o += len; b.p += len;
       w.flushed = w.o;
       __syncwarp();
@@ -339,6 +366,7 @@ __global__ void __launch_bounds__(32) bvcf_inflate_kernel(const InflateParams p)
         }
       }
       if (err) break;
+      if (b.overrun()) { err = 20; break; }
       __syncwarp();
       if (lengths[256] == 0) { err = 13; break; }
       int r = inf_construct(lc, lengths, nlen);
@@ -356,6 +384,7 @@ __global__ void __launch_bounds__(32) bvcf_inflate_kernel(const InflateParams p)
     return;
   }
   inf_flush(w, w.flushed, w.o, lane);  // what is still in the ring
+  if (w.crc != blk.crc && lane == 0) atomicAdd(p.n_bad, 1u);
 }
 
 }  // namespace bvcf

@@ -55,6 +55,67 @@ struct DiagSink {
   unsigned long long line_start;   // set per record by the caller
 };
 
+// CHROM and POS ("CHROM\tPOS") of the lines of a chunk's diagnostics, gathered on the device for the host's log lines
+// when the chunk's text exists only there (bgzf input).  An entry ends before the line's second tab; a line without
+// one in its first DIAG_FIELDS_MAX bytes gives an empty entry.
+constexpr uint32_t DIAG_FIELDS_MAX = 4096;
+__device__ __forceinline__ uint32_t diag_fields_len(const uint8_t *in, unsigned long long len, unsigned long long st) {
+  const unsigned long long lim = len < st + DIAG_FIELDS_MAX ? len : st + DIAG_FIELDS_MAX;
+  int tabs = 0;
+  for (unsigned long long p = st; p < lim; p++) {
+    const uint8_t c = in[p];
+    if (c == '\n') break;
+    if (c == '\t' && ++tabs == 2) return (uint32_t)(p - st);
+  }
+  return 0;
+}
+// one CTA: every entry's length, exclusive prefix sums into off[0 .. n] (1,024 entries per step)
+__global__ void __launch_bounds__(1024) bvcf_diag_fields_len_kernel(const uint8_t *in, unsigned long long len,
+                                                                   const unsigned long long *starts, uint32_t n,
+                                                                   unsigned long long *off) {
+  __shared__ unsigned long long s_warp[32], s_base;
+  const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
+  if (t == 0) s_base = 0;
+  __syncthreads();
+  for (uint32_t b = 0; b < n; b += 1024) {
+    const uint32_t i = b + (uint32_t)t;
+    const unsigned long long l = i < n ? diag_fields_len(in, len, starts[i]) : 0ull;
+    unsigned long long v = l;  // inclusive scan: warp, then warp totals
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const unsigned long long u = __shfl_up_sync(FULL, v, d);
+      if (lane >= d) v += u;
+    }
+    if (lane == 31) s_warp[wid] = v;
+    __syncthreads();
+    if (wid == 0) {
+      unsigned long long w = s_warp[lane];
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const unsigned long long u = __shfl_up_sync(FULL, w, d);
+        if (lane >= d) w += u;
+      }
+      s_warp[lane] = w;
+    }
+    __syncthreads();
+    if (i < n) off[i] = s_base + (wid ? s_warp[wid - 1] : 0ull) + v - l;
+    __syncthreads();
+    if (t == 0) s_base += s_warp[31];
+    __syncthreads();
+  }
+  if (t == 0) off[n] = s_base;
+}
+// warp per entry: the bytes to out + off[e]
+__global__ void bvcf_diag_fields_copy_kernel(const uint8_t *in, const unsigned long long *starts, const unsigned long long *off,
+                                             uint32_t n, uint8_t *out) {
+  const uint32_t lane = threadIdx.x & 31, warps = (gridDim.x * blockDim.x) >> 5;
+  for (uint32_t e = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; e < n; e += warps) {
+    const unsigned long long o = off[e], m = off[e + 1] - o;
+    const uint8_t *src = in + starts[e];
+    for (uint32_t k = lane; k < m; k += 32) out[o + k] = src[k];
+  }
+}
+
 // site types (bystro-utils parse.Snp/Ins/Del/Mnp/Multi)
 enum { T_SNP = 0, T_INS = 1, T_DEL = 2, T_MNP = 3, T_MULTI = 4 };
 __device__ __constant__ char TYPE_TXT[5][13] = {"SNP", "INS", "DEL", "MNP", "MULTIALLELIC"};

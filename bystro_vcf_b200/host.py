@@ -171,6 +171,7 @@ class ChunkResult:
     loci: List[bytes] = field(default_factory=list)
     dosage: Optional[object] = None  # numpy int8 [rows, samples]
     retries: int = 0
+    diag_fields: List[tuple] = field(default_factory=list)    # (CHROM, POS) of each diagnostic's line, when asked for
 
 
 def _unpack_dosage(dos):
@@ -277,7 +278,38 @@ class Transformer:
             self._keep_chunk[seq] = chunk
         check(self._L.bvcf_submit(self._ctx, seq, addr, n), self._ctx, "bvcf_submit")
 
-    def collect(self, seq: int, copy: bool = True) -> ChunkResult:
+    def submit_bgzf(self, seq: int, comp, skip: int = 0, tail: bytes = b"") -> None:
+        """A chunk given as whole bgzf blocks: its text is inflate(comp)[skip:] + tail and must end with a newline.
+        comp: bytes-like or (address, length).  The blocks are inflated on the GPU and every member's CRC-32 and ISIZE
+        checked there: collect(seq) raises BvcfError for a corrupt member."""
+        if isinstance(comp, tuple):
+            addr, n = comp
+        else:
+            comp = bytes(comp) if not isinstance(comp, bytes) else comp
+            n = len(comp)
+            addr = C.cast(C.c_char_p(comp), C.c_void_p).value
+        tail = bytes(tail)
+        self._keep_chunk = getattr(self, "_keep_chunk", {})
+        self._keep_chunk[seq] = (comp, tail)
+        check(self._L.bvcf_submit_bgzf(self._ctx, seq, addr, n, skip, C.cast(C.c_char_p(tail), C.c_void_p).value, len(tail)),
+              self._ctx, "bvcf_submit_bgzf")
+
+    def _diag_fields(self, seq: int, n: int) -> List[tuple]:
+        """(CHROM, POS) of each diagnostic of collected chunk seq, gathered on the device (bvcf_diag_fields)"""
+        text, off = C.c_void_p(), C.POINTER(C.c_uint64)()
+        check(self._L.bvcf_diag_fields(self._ctx, seq, C.byref(text), C.byref(off)), self._ctx, "bvcf_diag_fields")
+        if n == 0:
+            return []
+        blob = C.string_at(text, off[n]) if off[n] else b""
+        out = []
+        for i in range(n):
+            f = blob[off[i]:off[i + 1]].split(b"\t", 1)
+            out.append((f[0].decode("latin-1"), f[1].decode("latin-1")) if len(f) == 2 else ("?", "?"))
+        return out
+
+    def collect(self, seq: int, copy: bool = True, diag_fields: bool = False) -> ChunkResult:
+        """Rows, dosage batch and diagnostics of chunk seq, in input order.  diag_fields: also the CHROM and POS of each
+        diagnostic's line (out.diag_fields), read on the device -- what a bgzf chunk's log lines need."""
         import numpy as np
 
         tsv = C.c_void_p()
@@ -293,6 +325,8 @@ class Transformer:
         out.diags = [(dg[i].line_no, dg[i].alt_no, dg[i].code) for i in range(nd.value)]
         out.diag_starts = [dg[i].line_start for i in range(nd.value)]
         out.loci, out.dosage = _unpack_dosage(dos)
+        if diag_fields:
+            out.diag_fields = self._diag_fields(seq, nd.value)
         check(self._L.bvcf_release(self._ctx, seq), self._ctx, "bvcf_release")
         if hasattr(self, "_keep_chunk"):
             self._keep_chunk.pop(seq, None)

@@ -12,17 +12,22 @@ Two partitions are provided:
   * `read_vcf_multi` the product path: the data region is cut into chunks (config.chunkBytes), chunk k goes to GPU
                      k mod N, results are written in chunk order.  Output streams while the GPUs work and host
                      memory stays bounded (a few chunks per GPU), which N contiguous shards cannot offer: shard 1's
-                     whole output would have to wait for shard 0's.
+                     whole output would have to wait for shard 0's.  A bgzf (.vcf.gz) input is cut into groups of
+                     whole blocks (bgzf.plan_groups): the compressed bytes go to the GPUs, which inflate them.
 Both are pure host logic around bvcf_submit / bvcf_collect.
 """
 from __future__ import annotations
 
 import ctypes as C
 import queue
+import re
 import threading
 from typing import BinaryIO, List, Optional, Sequence, Tuple
 
-from .host import Config, PinnedRing, Transformer, format_diag, locus_at, parse_preamble, write_sample_list
+from . import bgzf
+from ._lib import BvcfError
+from .host import (Config, NotAVcfError, PinnedRing, Transformer, format_diag, locus_at, parse_preamble,
+                   write_sample_list)
 
 
 def partition(data, begin: int, end: int, n: int) -> List[Tuple[int, int]]:
@@ -83,23 +88,29 @@ def _stage(dst: int, data, lo: int, hi: int) -> None:
 
 def _gpu_worker(cfg: Config, device: int, eol_width: int, chrom_line: bytes, data, chunks, my_ids, results, errors,
                 n_slots: int):
-    """One GPU: its chunks in order, n_slots in flight; results (chunk id, ChunkResult) into `results`."""
+    """One GPU: its chunks in order, n_slots in flight; results (chunk id, ChunkResult) into `results`.  A chunk is a
+    (lo, hi) byte range of plain text or a bgzf.Group."""
     ring = None
     try:
         c = Config(**{**cfg.__dict__, "device": device})
+        gz = bool(chunks) and isinstance(chunks[0], bgzf.Group)
         cap = max((chunks[i][1] - chunks[i][0] for i in my_ids), default=0) + 1
+        text_cap = max((chunks[i].text + len(chunks[i].tail) for i in my_ids), default=0) + 1 if gz else cap
         ring = PinnedRing(n_slots + 1, cap)
-        with Transformer(c, eol_width=eol_width, n_slots=n_slots, max_chunk_bytes=cap) as tr:
+        with Transformer(c, eol_width=eol_width, n_slots=n_slots, max_chunk_bytes=text_cap) as tr:
             tr.set_header(chrom_line)
             sub = col = 0
             while col < len(my_ids):
                 while sub < len(my_ids) and sub - col < n_slots:
-                    lo, hi = chunks[my_ids[sub]]
+                    ch = chunks[my_ids[sub]]
                     buf = ring.ptrs[sub % (n_slots + 1)]
-                    _stage(buf, data, lo, hi)
-                    tr.submit(sub, (buf, hi - lo))
+                    _stage(buf, data, ch[0], ch[1])
+                    if gz:
+                        tr.submit_bgzf(sub, (buf, ch.hi - ch.lo), ch.skip, ch.tail)
+                    else:
+                        tr.submit(sub, (buf, ch[1] - ch[0]))
                     sub += 1
-                res = tr.collect(col)
+                res = tr.collect(col, diag_fields=gz)
                 results.put((my_ids[col], res))  # blocks when the writer is behind: bounded host memory
                 col += 1
     except BaseException as e:  # surfaced by the caller
@@ -113,13 +124,33 @@ def _gpu_worker(cfg: Config, device: int, eol_width: int, chrom_line: bytes, dat
 def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Sequence[int], diag_sink=None,
                    n_slots: int = 3) -> dict:
     """readVcf (main.go:241-396) over several GPUs of one box.  `data` is the whole uncompressed VCF as a bytes-like
-    object or mmap.  Chunk k of the data region goes to devices[k mod N] (a device may be listed more than once);
-    rows, dosage batches and diagnostics leave in input order while the GPUs are still working."""
-    width, chrom_line, off = parse_preamble(bytes(data[:min(len(data), 64 << 20)]))
-    end = len(data)
-    last_nl = data.rfind(b"\n", off, end)
-    end = off if last_nl < 0 else last_nl + 1  # an unterminated last line is dropped (main.go:354-357)
-    chunks = chunk_ranges(data, off, end, max(int(config.chunkBytes), 1 << 16))
+    object or mmap, or a whole bgzf (.vcf.gz) file.  Chunk k of the data region goes to devices[k mod N] (a device may
+    be listed more than once); rows, dosage batches and diagnostics leave in input order while the GPUs are still
+    working."""
+    chunk_bytes = max(int(config.chunkBytes), 1 << 16)
+    gz = bgzf.is_bgzf(bytes(data[:18]))
+    if gz:
+        want = 1 << 20
+        while True:  # the preamble, inflated on the host
+            text0 = bgzf.inflate_host(data, want)
+            try:
+                width, chrom_line, off = parse_preamble(text0)
+                break
+            except NotAVcfError as e:
+                if (str(e) == "Not a VCF file" and re.search(rb"[\r\n]", text0)) or len(text0) < want:
+                    raise
+                want *= 4
+        try:
+            chunks = bgzf.plan_groups(data, off, chunk_bytes, 2 * chunk_bytes + (64 << 20))
+        except ValueError as e:
+            raise BvcfError(str(e)) from None
+        end = off + sum(g.text - g.skip + len(g.tail) for g in chunks)
+    else:
+        width, chrom_line, off = parse_preamble(bytes(data[:min(len(data), 64 << 20)]))
+        end = len(data)
+        last_nl = data.rfind(b"\n", off, end)
+        end = off if last_nl < 0 else last_nl + 1  # an unterminated last line is dropped (main.go:354-357)
+        chunks = chunk_ranges(data, off, end, chunk_bytes)
     n_dev = len(devices)
     totals = {"n_lines": 0, "n_records": 0, "n_rows": 0, "out_bytes": 0, "in_bytes": end - off, "n_chunks": len(chunks),
               "devices": list(devices)}
@@ -154,9 +185,11 @@ def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Se
             if arrow is not None and res.dosage is not None:
                 arrow.write(res.loci, res.dosage)
             if diag_sink is not None and res.diags:
-                lo, hi = chunks[k]
-                for (ln, alt_no, code), st in zip(res.diags, res.diag_starts):
-                    chrom, pos = locus_at(data, lo + st)
+                if gz:
+                    loci = res.diag_fields
+                else:
+                    loci = [locus_at(data, chunks[k][0] + st) for st in res.diag_starts]
+                for (ln, alt_no, code), (chrom, pos) in zip(res.diags, loci):
                     diag_sink(format_diag(chrom, pos, alt_no, code), totals["n_lines"] + ln, alt_no, code)
             totals["n_lines"] += res.n_lines
             totals["n_records"] += res.n_records

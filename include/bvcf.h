@@ -143,6 +143,17 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
                  bvcf_chunk_stats *stats);
 int bvcf_release(bvcf_ctx *ctx, uint64_t seq);
 
+/* A chunk given as whole bgzf blocks: its text is inflate(comp)[skip:] followed by tail[0..tail_len), and must end
+ * with '\n'.  The CRC-32 and ISIZE of every member are checked on the device; bvcf_collect(seq) returns BVCF_E_ARG on
+ * a corrupt member.  The caller keeps comp and tail alive until bvcf_collect(seq) returns.  max_chunk_bytes limits the
+ * inflated text plus the tail; a diagnostic's line_start is an offset into inflate(comp) followed by the tail. */
+int bvcf_submit_bgzf(bvcf_ctx *ctx, uint64_t seq, const uint8_t *comp, size_t comp_len, size_t skip,
+                     const uint8_t *tail, size_t tail_len);
+/* CHROM and POS ("CHROM<TAB>POS", back to back) of the line of each diagnostic of collected chunk seq, in the order
+ * bvcf_collect returned them; off has n_diags + 1 entries.  Gathered on the device: the text of a bgzf chunk exists
+ * only there.  Library-owned, valid until bvcf_release(seq). */
+int bvcf_diag_fields(bvcf_ctx *ctx, uint64_t seq, const uint8_t **text, const uint64_t **off);
+
 /* ---- device-resident path: input already in HBM (bench `value`, torch/cupy interop) -------- */
 
 /* (Re)allocate the context's resident input region (+ padding) and output region; returns device pointers. */
@@ -157,9 +168,10 @@ int bvcf_resident_run(bvcf_ctx *ctx, size_t len, bvcf_chunk_stats *stats, bvcf_k
 int bvcf_resident_run_at(bvcf_ctx *ctx, size_t begin, size_t len, bvcf_chunk_stats *stats, bvcf_kernel_times *times);
 
 /* bgzf-compressed input (bgzip / htslib .vcf.gz; upstream of main.go:192 the reference pipes through `pigz -d -c`,
- * README.md:10,46): only the COMPRESSED bytes cross PCIe, the DEFLATE blocks are inflated on the GPU (one thread per
- * 64 KiB block) straight into the resident input region at `dst_offset`.  `comp` must hold whole bgzf blocks.
- * text_bytes receives the uncompressed size.  BVCF_E_ARG: not bgzf, corrupt, or larger than the region. */
+ * README.md:10,46): only the COMPRESSED bytes cross PCIe, the DEFLATE blocks are inflated on the GPU (one warp per
+ * bgzf block, its CRC-32 and ISIZE checked) straight into the resident input region at `dst_offset`.  `comp` must hold
+ * whole bgzf blocks.  text_bytes receives the uncompressed size.  BVCF_E_ARG: not bgzf, corrupt (including a CRC-32
+ * mismatch), or larger than the region. */
 int bvcf_resident_inflate_bgzf(bvcf_ctx *ctx, const void *comp, size_t comp_len, size_t dst_offset, size_t *text_bytes);
 /* Host only: the uncompressed size (sum of ISIZE) and block count of a bgzf buffer of whole blocks. */
 int bvcf_bgzf_text_bytes(const void *comp, size_t comp_len, uint64_t *text_bytes, uint64_t *n_blocks);
