@@ -2,10 +2,9 @@
 
 Same flags, same stdin/stdout behaviour: header line first (main.go:199), then rows in input order; the
 reference's log.Printf lines ("chrom:pos ALT #k message", main.go:730-986) on stderr, or appended to --err.
-`--gpus N` (extension) shards the input -- plain or bgzf (.vcf.gz) -- over N GPUs of the box (shard.read_vcf_multi);
-`--bgzfOut` (extension) writes
-the rows as bgzf blocks deflated on the GPU -- with a .vcf.gz input the command stands for the whole
-`pigz -d -c in.vcf.gz | bystro-vcf ... | pigz -c > out.gz` of README.md:10."""
+`--gpus N` (extension) shards the input -- plain or bgzf (.vcf.gz) -- over N GPUs of the box (shard.read_vcf_multi, which
+also runs a .vcf.gz on one GPU); `--bgzfOut` (extension) writes the rows as bgzf blocks deflated on the GPU -- with a
+.vcf.gz input the command stands for the whole `pigz -d -c in.vcf.gz | bystro-vcf ... | pigz -c > out.gz` of README.md:10."""
 from __future__ import annotations
 
 import os
@@ -67,15 +66,9 @@ def main(argv=None) -> int:
             print("--bgzfOut runs on one GPU", file=err)
             return 1
         if gpus > 1:
-            import mmap
+            from . import shard
 
-            from .shard import read_vcf_multi
-
-            if not cfg.inPath:
-                data = inp.read()
-            else:
-                data = mmap.mmap(inp.fileno(), 0, access=mmap.ACCESS_READ)
-            read_vcf_multi(cfg, data, out, list(range(gpus)), diag_sink=log)
+            shard.read_vcf_multi(cfg, shard.whole_input(inp), out, list(range(gpus)), diag_sink=log)
         else:
             read_vcf(cfg, inp, out, diag_sink=log)
         if out is not None and cfg.bgzfOut:

@@ -187,7 +187,8 @@ def compress(data, level: int = 6, block_text: int = MAX_TEXT, threads: int = 0,
 
 
 def inflate_host(buf, max_text: int) -> bytes:
-    """the first max_text text bytes of a bgzf buffer, on the host (zlib): only used to read the VCF preamble"""
+    """the text of the whole blocks at the start of a bgzf buffer, until there are at least max_text bytes of it, inflated
+    on the host and checked against each block's CRC-32 and ISIZE: only used to read the VCF preamble"""
     out = []
     n = 0
     p = 0
@@ -195,9 +196,7 @@ def inflate_host(buf, max_text: int) -> bytes:
         bs = block_size(buf, p)
         if bs == 0 or p + bs > len(buf):
             break
-        xlen = buf[p + 10] | (buf[p + 11] << 8)
-        text = zlib.decompress(bytes(buf[p + 12 + xlen:p + bs - 8]), -15)
-        out.append(text)
-        n += len(text)
+        out.append(_payload_text(buf, p, bs))
+        n += len(out[-1])
         p += bs
     return b"".join(out)

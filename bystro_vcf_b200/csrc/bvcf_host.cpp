@@ -274,8 +274,8 @@ struct Turnstile {
 
 // ---- bgzf input (.vcf.gz as bgzip / htslib write it): the compressed bytes go to the GPU, which inflates them ----
 // Replaces the `pigz -d -c in.vcf.gz |` in front of the reference (README.md:10,46).  Groups of whole blocks are
-// uploaded and inflated straight into the resident input region (bvcf_resident_inflate_bgzf), the transform runs
-// there; rows, dosage batches and diagnostics come back.  One GPU, one group at a time.
+// uploaded and inflated on the GPU: into a slot's input buffer (bvcf_submit_bgzf), or with --bgzfOut into the resident
+// input region (bvcf_resident_inflate_bgzf).
 bool looks_bgzf(const uint8_t *p, size_t n) {
   return n >= 18 && p[0] == 0x1f && p[1] == 0x8b && p[2] == 8 && (p[3] & 4) && p[12] == 'B' && p[13] == 'C';
 }
@@ -294,28 +294,6 @@ size_t bgzf_block_size(const uint8_t *p, size_t n) {  // 0: header incomplete
     q += 4 + slen;
   }
   fatal("gzip input without the bgzf BC subfield: decompress it first (gzip -dc | ...)");
-}
-// the first text bytes of a bgzf buffer, inflated on the host: only to read the VCF preamble
-std::string bgzf_inflate_host(const uint8_t *p, size_t n, size_t want) {
-  std::string out;
-  size_t off = 0;
-  while (off < n && out.size() < want) {
-    const size_t bs = bgzf_block_size(p + off, n - off);
-    if (!bs || off + bs > n) break;
-    const size_t xlen = (size_t)p[off + 10] | ((size_t)p[off + 11] << 8);
-    const uint32_t isize = (uint32_t)p[off + bs - 4] | ((uint32_t)p[off + bs - 3] << 8) | ((uint32_t)p[off + bs - 2] << 16) | ((uint32_t)p[off + bs - 1] << 24);
-    std::string text(isize, '\0');
-    z_stream z{};
-    if (inflateInit2(&z, -15) != Z_OK) fatal("zlib: inflateInit2 failed");
-    z.next_in = const_cast<Bytef *>(p + off + 12 + xlen); z.avail_in = (uInt)(bs - 12 - xlen - 8);
-    z.next_out = (Bytef *)text.data(); z.avail_out = isize;
-    const int zr = inflate(&z, Z_FINISH);
-    inflateEnd(&z);
-    if (zr != Z_STREAM_END && isize) fatal("corrupt bgzf block in the VCF preamble");
-    out += text;
-    off += bs;
-  }
-  return out;
 }
 
 // one bgzf block (SAM spec 4.1) around `text` (< 64 KiB), deflated on the host: the TSV header line
@@ -339,24 +317,31 @@ std::vector<uint8_t> bgzf_block_host(const uint8_t *text, size_t n) {
 }
 const uint8_t BGZF_EOF[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 
+// What main.go:250-294 finds in the first bytes of the text: the EOL width, the #CHROM line, where the data lines start
+struct Preamble {
+  std::string chrom_line;
+  size_t data_off = 0;
+  int eol_width = 1;
+};
+
 // main.go:250-294 on the first bytes of the text: EOL width, the ##fileformat check, the #CHROM line.  true when found;
 // false when more text is needed (fatal at eof)
-bool find_preamble(const uint8_t *p, size_t n, bool eof, std::string &chrom_line, size_t &data_off, int &eol_width) {
+bool find_preamble(const uint8_t *p, size_t n, bool eof, Preamble &pre) {
   if (n == 0 && eof) fatal("Not a VCF file");
   const uint8_t *nl = (const uint8_t *)memchr(p, '\n', n);
   if (!nl) { if (eof) fatal("Not a VCF file"); return false; }
   size_t first_end = nl - p;
-  eol_width = 1;
-  if (first_end > 0 && p[first_end - 1] == '\r') { eol_width = 2; first_end--; }
+  pre.eol_width = 1;
+  if (first_end > 0 && p[first_end - 1] == '\r') { pre.eol_width = 2; first_end--; }
   if (!memmem(p, first_end, "##fileformat=VCFv4", 18)) fatal("Not a VCF file");  // main.go:256-264
   for (size_t q = (nl - p) + 1; q < n;) {
     const uint8_t *e = (const uint8_t *)memchr(p + q, '\n', n - q);
     if (!e) break;
     size_t cl = (e - p) - q;
-    cl = cl + 1 >= (size_t)eol_width ? cl + 1 - eol_width : 0;
+    cl = cl + 1 >= (size_t)pre.eol_width ? cl + 1 - pre.eol_width : 0;
     if (cl >= 6 && memcmp(p + q, "#CHROM", 6) == 0 && (cl == 6 || p[q + 6] == '\t')) {
-      chrom_line.assign((const char *)p + q, cl);
-      data_off = (e - p) + 1;
+      pre.chrom_line.assign((const char *)p + q, cl);
+      pre.data_off = (e - p) + 1;
       return true;
     }
     q = (e - p) + 1;
@@ -365,25 +350,58 @@ bool find_preamble(const uint8_t *p, size_t n, bool eof, std::string &chrom_line
   return false;
 }
 
-// The blocks of a bgzf input, memory-mapped or read from a pipe as they are needed.  Blocks without text (the EOF
-// block among them) are left out of the list; offsets are absolute in the compressed stream.
+// The input bytes: a memory-mapped file, or what has been read from a pipe so far.  Offsets are absolute in the stream.
+class Input {
+ public:
+  Input(int fd, const uint8_t *map, size_t map_len, std::vector<uint8_t> head)
+      : fd_(fd), map_(map), map_len_(map_len), buf_(std::move(head)), eof_(map != nullptr) {}
+  bool mapped() const { return map_ != nullptr; }
+  bool eof() const { return eof_; }
+  int fd() const { return fd_; }
+  size_t end() const { return map_ ? map_len_ : base_ + buf_.size(); }
+  const uint8_t *at(size_t abs) const { return map_ ? map_ + abs : buf_.data() + (abs - base_); }
+  void fill(size_t want) {  // bytes up to absolute offset `want` (or the end of the input)
+    while (!eof_ && end() < want) {
+      const size_t old = buf_.size(), n = std::min<size_t>(8u << 20, std::max<size_t>(want - end(), 1u << 20));
+      buf_.resize(old + n);
+      const ssize_t r = read(fd_, buf_.data() + old, n);
+      if (r < 0) { buf_.resize(old); if (errno == EINTR) continue; fatal(std::string("read: ") + strerror(errno)); }
+      buf_.resize(old + (size_t)r);
+      if (r == 0) eof_ = true;
+    }
+  }
+  // pipe input: bytes before `abs` are no longer needed
+  void release_before(size_t abs) {
+    if (map_ || abs - base_ < (64u << 20)) return;
+    buf_.erase(buf_.begin(), buf_.begin() + (abs - base_));
+    base_ = abs;
+  }
+
+ private:
+  int fd_;
+  const uint8_t *map_;
+  size_t map_len_;
+  std::vector<uint8_t> buf_;
+  size_t base_ = 0;
+  bool eof_;
+};
+
+// The blocks of a bgzf input, walked as they are needed.  Blocks without text (the EOF block among them) are left out
+// of the list; offsets are absolute in the compressed stream.
 class BgzfIn {
  public:
   struct Blk { size_t off, size; uint64_t start; uint32_t isize; };
-  BgzfIn(int fd, const uint8_t *map, size_t map_len, std::vector<uint8_t> &head) : fd_(fd), map_(map), map_len_(map_len) {
-    if (!map_) buf_.swap(head);
-    eof_ = map_ != nullptr;
-  }
+  explicit BgzfIn(Input &in) : in_(in) {}
   // block i exists (reads and walks headers until it does or the input ends; a truncated block is fatal)
   bool has(size_t i) {
     while (blk_.size() <= i && !walked_) {
-      fill(walk_ + (1u << 16) + 18);
-      if (walk_ == end()) { walked_ = true; break; }
-      size_t bs = bgzf_block_size(at(walk_), end() - walk_);
-      if (bs && walk_ + bs > end()) { fill(walk_ + bs); }
-      bs = bgzf_block_size(at(walk_), end() - walk_);
-      if (!bs || walk_ + bs > end()) fatal("bgzf input: truncated block at the end");
-      const uint8_t *e = at(walk_ + bs - 4);
+      in_.fill(walk_ + (1u << 16) + 18);
+      if (walk_ == in_.end()) { walked_ = true; break; }
+      size_t bs = bgzf_block_size(in_.at(walk_), in_.end() - walk_);
+      if (bs && walk_ + bs > in_.end()) { in_.fill(walk_ + bs); }
+      bs = bgzf_block_size(in_.at(walk_), in_.end() - walk_);
+      if (!bs || walk_ + bs > in_.end()) fatal("bgzf input: truncated block at the end");
+      const uint8_t *e = in_.at(walk_ + bs - 4);
       const uint32_t isize = (uint32_t)e[0] | ((uint32_t)e[1] << 8) | ((uint32_t)e[2] << 16) | ((uint32_t)e[3] << 24);
       if (isize) blk_.push_back({walk_, bs, text_, isize});
       text_ += isize;
@@ -393,11 +411,16 @@ class BgzfIn {
   }
   const Blk &operator[](size_t i) const { return blk_[i]; }
   size_t off(size_t i) { return has(i) ? blk_[i].off : walk_; }  // where block i starts (the end past the last)
-  const uint8_t *at(size_t abs) const { return map_ ? map_ + abs : buf_.data() + (abs - base_); }
+  // the first block whose text reaches past text byte `text_off` (the end past the last when none does)
+  size_t block_at(uint64_t text_off) {
+    size_t b = 0;
+    while (has(b) && blk_[b].start + blk_[b].isize <= text_off) b++;
+    return b;
+  }
   // block i inflated on the host, its CRC-32 and ISIZE checked
   std::string inflate_block(size_t i) {
     const Blk &b = blk_[i];
-    const uint8_t *p = at(b.off);
+    const uint8_t *p = in_.at(b.off);
     const size_t xlen = (size_t)p[10] | ((size_t)p[11] << 8);
     std::string text(b.isize, '\0');
     z_stream z{};
@@ -419,32 +442,12 @@ class BgzfIn {
     for (size_t i = 0; out.size() < want && has(i); i++) out += inflate_block(i);
     return out;
   }
-  // pipe input: bytes before `abs` are no longer needed
-  void release_before(size_t abs) {
-    if (map_ || abs - base_ < (64u << 20)) return;
-    buf_.erase(buf_.begin(), buf_.begin() + (abs - base_));
-    base_ = abs;
-  }
 
  private:
-  size_t end() const { return map_ ? map_len_ : base_ + buf_.size(); }
-  void fill(size_t want) {  // bytes up to absolute offset `want` (or the end of the input)
-    while (!eof_ && end() < want) {
-      const size_t old = buf_.size();
-      buf_.resize(old + (8u << 20));
-      const ssize_t r = read(fd_, buf_.data() + old, 8u << 20);
-      if (r < 0) { buf_.resize(old); if (errno == EINTR) continue; fatal(std::string("read: ") + strerror(errno)); }
-      buf_.resize(old + (size_t)r);
-      if (r == 0) eof_ = true;
-    }
-  }
-  int fd_;
-  const uint8_t *map_;
-  size_t map_len_;
-  std::vector<uint8_t> buf_;
-  size_t base_ = 0, walk_ = 0;
+  Input &in_;
+  size_t walk_ = 0;
   uint64_t text_ = 0;
-  bool eof_ = false, walked_ = false;
+  bool walked_ = false;
   std::vector<Blk> blk_;
 };
 
@@ -457,8 +460,7 @@ class BgzfIn {
 // receives each group in order (hi_block: one past its last block).
 template <class Emit>
 void plan_bgzf_groups(BgzfIn &in, uint64_t data_off, size_t chunk_bytes, size_t cap, Emit emit_out) {
-  size_t b = 0;
-  while (in.has(b) && in[b].start + in[b].isize <= data_off) b++;
+  size_t b = in.block_at(data_off);
   if (!in.has(b)) return;
   size_t skip = (size_t)(data_off - in[b].start);
   auto take = [&](size_t i) {
@@ -526,133 +528,139 @@ void plan_bgzf_groups(BgzfIn &in, uint64_t data_off, size_t chunk_bytes, size_t 
   }
 }
 
-// readVcf over the resident regions, for compressed streams on either side: bgzf input is inflated on the GPU
-// (compressed_in), --bgzfOut rows are deflated there
-int run_resident(const Config &config, int in_fd, const uint8_t *map, size_t map_len, std::vector<uint8_t> &head, int out_fd,
-                 bool compressed_in) {
-  // compressed bytes: the mapping, or a growing buffer read from the pipe
-  std::vector<uint8_t> &buf = head;
-  size_t consumed = 0;  // bytes of the compressed stream already handed to the GPU
-  bool eof = map != nullptr;
-  auto avail = [&]() { return map ? map_len - consumed : buf.size() - consumed; };
-  auto at = [&](size_t off) { return map ? map + consumed + off : buf.data() + consumed + off; };
-  auto fill = [&](size_t want) {
-    while (!eof && avail() < want) {
-      const size_t old = buf.size();
-      buf.resize(old + (8u << 20));
-      const ssize_t r = read(in_fd, buf.data() + old, 8u << 20);
-      if (r < 0) { if (errno == EINTR) { buf.resize(old); continue; } fatal(std::string("read: ") + strerror(errno)); }
-      buf.resize(old + (size_t)r);
-      if (r == 0) eof = true;
-    }
-  };
-  // ---- preamble (main.go:250-294) from the first blocks ----
-  std::string chrom_line;
-  size_t data_off = 0;
-  int eol_width = 1;
-  for (size_t want = 1u << 20;; want *= 4) {
-    fill(want);
-    const std::string t = compressed_in ? bgzf_inflate_host(at(0), avail(), want * 4) : std::string((const char *)at(0), std::min(avail(), want * 4));
-    if (find_preamble((const uint8_t *)t.data(), t.size(), eof, chrom_line, data_off, eol_width)) break;
-  }
-  if (!config.sampleListPath.empty() && !config.noOut) {
-    FILE *f = fopen(config.sampleListPath.c_str(), "w");
-    if (!f) fatal("Couldn't write sample list file");
+// Where the results of a run go (main.go:296-343, 398-445): the rows to the output, the dosage batches to the Arrow
+// file.  Built once from the #CHROM line: it writes the sample list and opens the dosage file -- or, when the VCF has no
+// samples, writes an empty one and asks for no dosage work.
+class Sink {
+ public:
+  Sink(const Config &c, int out_fd, const std::string &chrom_line) : c_(c), out_fd_(out_fd) {
+    std::vector<std::string> names;
     int field = 0;
-    size_t s0 = 0;
+    size_t s = 0;
     for (size_t i = 0; i <= chrom_line.size(); i++)
       if (i == chrom_line.size() || chrom_line[i] == '\t') {
-        if (field >= 9) { std::string nm = chrom_line.substr(s0, i - s0); for (auto &ch : nm) if (ch == '.') ch = '_'; fprintf(f, "%s\n", nm.c_str()); }
-        field++; s0 = i + 1;
+        if (field >= 9) {
+          names.push_back(chrom_line.substr(s, i - s));
+          for (auto &ch : names.back()) if (ch == '.') ch = '_';  // parse.NormalizeHeader
+        }
+        field++; s = i + 1;
       }
-    fclose(f);
-  }
-  std::vector<const char *> allow_c, excl_c;
-  for (auto &s : config.allowed) allow_c.push_back(s.c_str());
-  for (auto &s : config.excluded) excl_c.push_back(s.c_str());
-  bvcf_config bc{};
-  bc.empty_field = config.emptyField.c_str(); bc.field_delim = config.fieldDelimiter.c_str();
-  bc.keep_id = config.keepID; bc.keep_info = config.keepInfo; bc.keep_pos = config.keepPos;
-  std::vector<std::string> sample_names;
-  {
-    int field = 0;
-    size_t s0 = 0;
-    for (size_t i = 0; i <= chrom_line.size(); i++)
-      if (i == chrom_line.size() || chrom_line[i] == '\t') {
-        if (field >= 9) { std::string nm = chrom_line.substr(s0, i - s0); for (auto &ch : nm) if (ch == '.') ch = '_'; sample_names.push_back(nm); }
-        field++; s0 = i + 1;
-      }
-  }
-  bool want_dosage = !config.dosageMatrixOutPath.empty();
-#ifndef BVCF_NO_ARROW
-  bvcf_arrow_writer *arrow = nullptr;
-  if (want_dosage) {
-    if (sample_names.empty()) {  // main.go:308-318
-      fprintf(stderr, "No samples found in VCF file; writing empty dosage matrix file\n");
-      FILE *f = fopen(config.dosageMatrixOutPath.c_str(), "w");
-      if (!f) fatal(config.dosageMatrixOutPath + ": " + strerror(errno));
+    if (!c.sampleListPath.empty() && !c.noOut) {
+      FILE *f = fopen(c.sampleListPath.c_str(), "w");
+      if (!f) fatal("Couldn't write sample list file");
+      for (auto &nm : names) fprintf(f, "%s\n", nm.c_str());
       fclose(f);
-      want_dosage = false;
-    } else {
-      std::vector<const char *> nm;
-      for (auto &s : sample_names) nm.push_back(s.c_str());
-      char err[512];
-      arrow = bvcf_arrow_open(config.dosageMatrixOutPath.c_str(), nm.data(), (uint32_t)nm.size(), err, sizeof err);
-      if (!arrow) fatal(std::string("dosage output: ") + err);
     }
-  }
+#ifndef BVCF_NO_ARROW
+    if (c.dosageMatrixOutPath.empty()) return;
+    if (names.empty()) {  // main.go:308-318
+      fprintf(stderr, "No samples found in VCF file; writing empty dosage matrix file\n");
+      FILE *f = fopen(c.dosageMatrixOutPath.c_str(), "w");
+      if (!f) fatal(c.dosageMatrixOutPath + ": " + strerror(errno));
+      fclose(f);
+      return;
+    }
+    std::vector<const char *> nm;
+    for (auto &x : names) nm.push_back(x.c_str());
+    char err[512];
+    arrow_ = bvcf_arrow_open(c.dosageMatrixOutPath.c_str(), nm.data(), (uint32_t)nm.size(), err, sizeof err);
+    if (!arrow_) fatal(std::string("dosage output: ") + err);
 #endif
-  bc.want_tsv = !config.noOut; bc.want_dosage = want_dosage;
-  bc.allow = allow_c.data(); bc.n_allow = config.allowAll ? -1 : (int)allow_c.size();
+  }
+  bool want_dosage() const { return arrow_ != nullptr; }
+  void rows(const uint8_t *p, size_t n) {
+    if (!c_.noOut) write_all(out_fd_, p, n);
+  }
+  void dosage(const bvcf_dosage_batch &d) {
+#ifndef BVCF_NO_ARROW
+    if (arrow_ && d.n_rows && bvcf_arrow_write(arrow_, d.n_rows, d.dosage, d.loci, d.loci_off))
+      fatal(std::string("dosage output: ") + bvcf_arrow_error(arrow_));
+#endif
+  }
+  // the exit status: 1 when the Arrow file could not be finished
+  int close() {
+#ifndef BVCF_NO_ARROW
+    if (arrow_ && bvcf_arrow_close(arrow_)) return 1;
+#endif
+    return 0;
+  }
+
+ private:
+  const Config &c_;
+  int out_fd_;
+#ifndef BVCF_NO_ARROW
+  bvcf_arrow_writer *arrow_ = nullptr;
+#else
+  void *arrow_ = nullptr;
+#endif
+};
+
+// a context on CUDA device `device` for this run, its #CHROM line set
+bvcf_ctx *open_ctx(const Config &c, int device, const Preamble &pre, bool want_dosage, int n_slots, size_t max_chunk_bytes) {
+  std::vector<const char *> allow_c, excl_c;
+  for (auto &s : c.allowed) allow_c.push_back(s.c_str());
+  for (auto &s : c.excluded) excl_c.push_back(s.c_str());
+  bvcf_config bc{};
+  bc.empty_field = c.emptyField.c_str();
+  bc.field_delim = c.fieldDelimiter.c_str();
+  bc.keep_id = c.keepID; bc.keep_info = c.keepInfo; bc.keep_pos = c.keepPos;
+  bc.want_tsv = !c.noOut; bc.want_dosage = want_dosage;
+  bc.allow = allow_c.data(); bc.n_allow = c.allowAll ? -1 : (int)allow_c.size();
   bc.exclude = excl_c.data(); bc.n_exclude = (int)excl_c.size();
-  bc.eol_width = eol_width; bc.normalize_dots = 1;
+  bc.eol_width = pre.eol_width; bc.normalize_dots = 1;
+  bc.n_slots = n_slots;
+  bc.max_chunk_bytes = max_chunk_bytes;
   bvcf_ctx *ctx = nullptr;
-  int rc = bvcf_create(&ctx, config.devices.empty() ? 0 : config.devices[0], &bc);
-  if (rc) fatal(std::string("bvcf_create: ") + bvcf_strerror(rc) + " -- a CUDA device is required, there is no CPU fallback");
-  if ((rc = bvcf_set_header(ctx, chrom_line.data(), chrom_line.size()))) fatal(std::string("bvcf_set_header: ") + bvcf_strerror(rc));
+  int rc = bvcf_create(&ctx, device, &bc);
+  if (rc) fatal(std::string("bvcf_create(gpu ") + std::to_string(device) + "): " + bvcf_strerror(rc) + " -- a CUDA device is required, there is no CPU fallback");
+  if ((rc = bvcf_set_header(ctx, pre.chrom_line.data(), pre.chrom_line.size()))) fatal(std::string("bvcf_set_header: ") + bvcf_strerror(rc));
+  return ctx;
+}
+
+// readVcf for --bgzfOut: the rows are deflated where they are made, so the input goes through one GPU's resident
+// regions a group at a time -- plain text uploaded, or whole bgzf blocks inflated there (bvcf_resident_inflate_bgzf).
+// The partial line at a group's end is carried into the next group.
+void run_resident(const Config &config, Input &in, BgzfIn *gz, const Preamble &pre, Sink &sink) {
+  bvcf_ctx *ctx = open_ctx(config, config.devices.empty() ? 0 : config.devices[0], pre, sink.want_dosage(), 0, 0);
+  int rc;
   const size_t batch_text = std::max<size_t>(config.chunkBytes * 8, 64u << 20), max_line = 8u << 20;
   void *d_in, *d_out;
   if ((rc = bvcf_resident_alloc(ctx, batch_text + max_line + (1u << 20), batch_text / 4 + (64u << 20), &d_in, &d_out)))
     fatal(std::string("bvcf_resident_alloc: ") + bvcf_strerror(rc));
-  uint8_t *pin = nullptr, *out_host = nullptr;   // pinned: compressed group in, rows out
+  uint8_t *pin = nullptr, *out_host = nullptr;   // pinned: group in, compressed rows out
   size_t pin_cap = 0, out_cap = 0;
   std::vector<uint8_t> carry, tail;
-  size_t begin = data_off;
+  // the first group starts at the data lines (plain) or at the block that holds their first byte (bgzf); `begin` is
+  // where they start in it
+  size_t pos = pre.data_off, b = 0, begin = 0;
+  if (gz && gz->has(b = gz->block_at(pre.data_off))) begin = pre.data_off - (*gz)[b].start;
   for (;;) {
-    // ---- a group of whole blocks worth about batch_text bytes of text ----
-    size_t p = 0, text = 0;
-    if (!compressed_in) {
-      fill(batch_text);
-      p = std::min(avail(), batch_text);
+    // ---- a group: whole blocks worth about batch_text bytes of text, or batch_text bytes of plain text ----
+    size_t lo = pos, hi;
+    if (gz) {
+      size_t e = b;
+      for (uint64_t text = 0; text < batch_text && gz->has(e); e++) text += (*gz)[e].isize;
+      lo = gz->off(b); hi = gz->off(e);  // blocks without text in between go along
+      b = e;
+    } else {
+      in.fill(pos + batch_text);
+      hi = pos = std::min(in.end(), pos + batch_text);
     }
-    while (compressed_in && text < batch_text) {
-      fill(p + (1u << 16) + 18);
-      const size_t bs = bgzf_block_size(at(p), avail() - p);
-      if (!bs || p + bs > avail()) {
-        if (!eof) { fill(p + std::max<size_t>(bs, 1u << 16) + 18); continue; }
-        break;
-      }
-      const uint8_t *e = at(p + bs - 4);
-      text += (size_t)e[0] | ((size_t)e[1] << 8) | ((size_t)e[2] << 16) | ((size_t)e[3] << 24);
-      p += bs;
-    }
-    if (p == 0) break;
-    if (p > pin_cap) {
+    if (hi == lo) break;
+    if (hi - lo > pin_cap) {
       if (pin) bvcf_host_free(pin);
-      pin_cap = p + p / 4;
+      pin_cap = (hi - lo) + (hi - lo) / 4;
       if (bvcf_host_alloc((void **)&pin, pin_cap)) fatal("bvcf_host_alloc failed");
     }
-    memcpy(pin, at(0), p);
-    consumed += p;
-    if (!map && consumed > (64u << 20)) { buf.erase(buf.begin(), buf.begin() + consumed); consumed = 0; }
+    memcpy(pin, in.at(lo), hi - lo);
+    in.release_before(hi);
     if (!carry.empty() && (rc = bvcf_resident_upload(ctx, 0, carry.data(), carry.size()))) fatal(std::string("upload: ") + bvcf_strerror(rc));
-    size_t n_text = 0;
-    if (compressed_in) {
-      if ((rc = bvcf_resident_inflate_bgzf(ctx, pin, p, carry.size(), &n_text)))
+    size_t n_text = hi - lo;
+    if (gz) {
+      if ((rc = bvcf_resident_inflate_bgzf(ctx, pin, hi - lo, carry.size(), &n_text)))
         fatal(std::string("bgzf: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
-    } else {
-      if ((rc = bvcf_resident_upload(ctx, carry.size(), pin, p))) fatal(std::string("upload: ") + bvcf_strerror(rc));
-      n_text = p;
+    } else if ((rc = bvcf_resident_upload(ctx, carry.size(), pin, hi - lo))) {
+      fatal(std::string("upload: ") + bvcf_strerror(rc));
     }
     const size_t total = carry.size() + n_text;
     // ---- the longest newline-terminated prefix; the rest is carried into the next group ----
@@ -675,31 +683,23 @@ int run_resident(const Config &config, int in_fd, const uint8_t *map, size_t map
         out_cap = st.out_bytes + st.out_bytes / 4;
         if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
       }
-      if (config.bgzfOut) {
-        size_t comp = 0;
+      size_t comp = 0;
+      rc = bvcf_resident_download_bgzf(ctx, 0, st.out_bytes, out_host, out_cap, &comp);
+      if (rc == BVCF_E_TOO_LARGE) {  // comp: the bytes needed
+        bvcf_host_free(out_host);
+        out_cap = comp + comp / 8;
+        if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
         rc = bvcf_resident_download_bgzf(ctx, 0, st.out_bytes, out_host, out_cap, &comp);
-        if (rc == BVCF_E_TOO_LARGE) {  // comp: the bytes needed
-          bvcf_host_free(out_host);
-          out_cap = comp + comp / 8;
-          if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
-          rc = bvcf_resident_download_bgzf(ctx, 0, st.out_bytes, out_host, out_cap, &comp);
-        }
-        if (rc) fatal(std::string("download: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
-        write_all(out_fd, out_host, comp);
-      } else {
-        if ((rc = bvcf_resident_download(ctx, 0, out_host, st.out_bytes))) fatal(std::string("download: ") + bvcf_strerror(rc));
-        write_all(out_fd, out_host, st.out_bytes);
       }
+      if (rc) fatal(std::string("download: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
+      sink.rows(out_host, comp);
     }
     {  // dosage batch and diagnostics of this group
-      bvcf_dosage_batch dos;
+      bvcf_dosage_batch dos{};
       const bvcf_diag *dg = nullptr;
       size_t nd = 0;
-      if ((rc = bvcf_resident_results(ctx, want_dosage ? &dos : nullptr, &dg, &nd))) fatal(std::string("results: ") + bvcf_strerror(rc));
-#ifndef BVCF_NO_ARROW
-      if (arrow && want_dosage && dos.n_rows && bvcf_arrow_write(arrow, dos.n_rows, dos.dosage, dos.loci, dos.loci_off))
-        fatal(std::string("dosage output: ") + bvcf_arrow_error(arrow));
-#endif
+      if ((rc = bvcf_resident_results(ctx, sink.want_dosage() ? &dos : nullptr, &dg, &nd))) fatal(std::string("results: ") + bvcf_strerror(rc));
+      sink.dosage(dos);
       char line[4096];
       for (size_t k = 0; k < nd; k++) {
         const size_t n = std::min<size_t>(sizeof line, end - dg[k].line_start);
@@ -710,180 +710,24 @@ int run_resident(const Config &config, int in_fd, const uint8_t *map, size_t map
     begin = 0;
   }
   // an unterminated last line (the carry) is dropped (main.go:354-357)
-  if (config.bgzfOut && !config.noOut) write_all(out_fd, BGZF_EOF, sizeof BGZF_EOF);
+  sink.rows(BGZF_EOF, sizeof BGZF_EOF);
   if (pin) bvcf_host_free(pin);
   if (out_host) bvcf_host_free(out_host);
-  int rc_exit = 0;
-#ifndef BVCF_NO_ARROW
-  if (arrow && bvcf_arrow_close(arrow)) rc_exit = 1;
-#endif
   bvcf_destroy(ctx);
-  return rc_exit;
 }
 
-}  // namespace
-
-int main(int argc, char **argv) {
-  Config config = setup(argc, argv);
-  int in_fd = 0;
-  if (!config.inPath.empty() && (in_fd = open(config.inPath.c_str(), O_RDONLY)) < 0) fatal(config.inPath + ": " + strerror(errno));
-  // main.go:150-156 re-points os.Stderr at the file, which Go's `log` never looks at again; what the flag evidently
-  // means is honoured here: diagnostics are appended to it
-  if (!config.errPath.empty() && !freopen(config.errPath.c_str(), "a", stderr)) fatal(config.errPath + ": " + strerror(errno));
-  if (config.noOut && !config.outPath.empty()) fatal("Cannot specify --noOut and --out");                 // main.go:160
-  if (config.noOut && config.dosageMatrixOutPath.empty()) fatal("When specifying --noOut, must specify --dosageOutput");  // :164
-#ifdef BVCF_NO_ARROW
-  if (!config.dosageMatrixOutPath.empty())
-    fatal("--dosageOutput: this binary was built without libarrow (pyarrow was not found at build time); "
-          "python -m bystro_vcf_b200 writes the Arrow file");
-#endif
-  int out_fd = 1;
-  if (!config.noOut && !config.outPath.empty() &&
-      (out_fd = open(config.outPath.c_str(), O_WRONLY | O_CREAT, 0644)) < 0)  // no O_TRUNC, like main.go:172
-    fatal(config.outPath + ": " + strerror(errno));
-  if (!config.noOut) {
-    const std::string h = string_header(config) + "\n";  // main.go:199: before any input is read
-    if (config.bgzfOut) {
-      const std::vector<uint8_t> b = bgzf_block_host((const uint8_t *)h.data(), h.size());
-      write_all(out_fd, b.data(), b.size());
-    } else {
-      write_all(out_fd, (const uint8_t *)h.data(), h.size());
-    }
-  }
-
-  // ---- input: a regular file is memory-mapped, anything else (pipes) is read ----
-  const uint8_t *map = nullptr;
-  size_t map_len = 0;
-  {
-    struct stat sb;
-    if (in_fd != 0 && fstat(in_fd, &sb) == 0 && S_ISREG(sb.st_mode) && sb.st_size > 0) {
-      void *m = mmap(nullptr, (size_t)sb.st_size, PROT_READ, MAP_PRIVATE, in_fd, 0);
-      if (m != MAP_FAILED) {
-        map = (const uint8_t *)m;
-        map_len = (size_t)sb.st_size;
-        madvise(m, map_len, MADV_SEQUENTIAL);
-      }
-    }
-  }
-
-  std::vector<uint8_t> head;  // pipe input: what has been read so far
-  bool bz = false;            // .vcf.gz (bgzf) input
-  {
-    if (map) bz = looks_bgzf(map, map_len);
-    else {
-      head.resize(1 << 16);
-      size_t got = 0;
-      while (got < 18) {
-        const ssize_t r = read(in_fd, head.data() + got, head.size() - got);
-        if (r < 0) { if (errno == EINTR) continue; fatal(std::string("read: ") + strerror(errno)); }
-        if (r == 0) break;
-        got += (size_t)r;
-      }
-      head.resize(got);
-      bz = looks_bgzf(head.data(), head.size());
-    }
-    if (config.bgzfOut) {  // the rows are deflated where they are, on one GPU's resident regions
-      if (config.gpus > 1) fatal("--bgzfOut runs on one GPU");
-      const int rc = run_resident(config, in_fd, map, map_len, head, out_fd, bz);
-      if (map) munmap((void *)map, map_len);
-      if (out_fd != 1) close(out_fd);
-      return rc;
-    }
-  }
-  // ---- preamble (main.go:250-294): EOL, ##fileformat check, #CHROM line; a bgzf input's is inflated on the host ----
-  size_t data_off = 0;
-  int eol_width = 1;
-  std::string chrom_line;
-  bool eof = false;
-  std::unique_ptr<BgzfIn> gz;
-  if (bz) {
-    gz.reset(new BgzfIn(in_fd, map, map_len, head));
-    for (size_t want = 1u << 20;; want *= 4) {
-      const std::string t = gz->prefix(want);
-      if (find_preamble((const uint8_t *)t.data(), t.size(), t.size() < want, chrom_line, data_off, eol_width)) break;
-    }
-  }
-  while (!gz) {
-    const uint8_t *p;
-    size_t n;
-    if (map) {
-      p = map; n = map_len; eof = true;
-    } else {
-      const size_t old = head.size();
-      head.resize(old + (1 << 20));
-      ssize_t r = read(in_fd, head.data() + old, 1 << 20);
-      if (r < 0) fatal(std::string("read: ") + strerror(errno));
-      head.resize(old + (size_t)r);
-      if (r == 0) eof = true;
-      p = head.data(); n = head.size();
-    }
-    if (find_preamble(p, n, eof, chrom_line, data_off, eol_width)) break;
-  }
-  std::vector<std::string> sample_names;
-  {
-    int field = 0;
-    size_t s = 0;
-    for (size_t i = 0; i <= chrom_line.size(); i++)
-      if (i == chrom_line.size() || chrom_line[i] == '\t') {
-        if (field >= 9) {
-          std::string nm = chrom_line.substr(s, i - s);
-          for (auto &ch : nm) if (ch == '.') ch = '_';  // parse.NormalizeHeader
-          sample_names.push_back(nm);
-        }
-        field++; s = i + 1;
-      }
-  }
-  if (!config.sampleListPath.empty() && !config.noOut) {  // main.go:398-445
-    FILE *f = fopen(config.sampleListPath.c_str(), "w");
-    if (!f) fatal("Couldn't write sample list file");
-    for (auto &nm : sample_names) fprintf(f, "%s\n", nm.c_str());
-    fclose(f);
-  }
-  bool want_dosage = !config.dosageMatrixOutPath.empty();
-#ifndef BVCF_NO_ARROW
-  bvcf_arrow_writer *arrow = nullptr;
-  if (want_dosage) {
-    if (sample_names.empty()) {  // main.go:308-318
-      fprintf(stderr, "No samples found in VCF file; writing empty dosage matrix file\n");
-      FILE *f = fopen(config.dosageMatrixOutPath.c_str(), "w");
-      if (!f) fatal(config.dosageMatrixOutPath + ": " + strerror(errno));
-      fclose(f);
-      want_dosage = false;
-    } else {
-      std::vector<const char *> nm;
-      for (auto &s : sample_names) nm.push_back(s.c_str());
-      char err[512];
-      arrow = bvcf_arrow_open(config.dosageMatrixOutPath.c_str(), nm.data(), (uint32_t)nm.size(), err, sizeof err);
-      if (!arrow) fatal(std::string("dosage output: ") + err);
-    }
-  }
-#endif
-
+// readVcf on 1..N GPUs: a reader cuts the input into chunks (newline-aligned text, or groups of whole bgzf blocks), chunk
+// k goes to GPU k mod N, and each GPU's worker hands its results to the sink when it is the chunk's turn
+void run_streaming(const Config &config, Input &in, BgzfIn *gz, const Preamble &pre, Sink &sink) {
   // ---- one context per GPU ----
-  std::vector<const char *> allow_c, excl_c;
-  for (auto &s : config.allowed) allow_c.push_back(s.c_str());
-  for (auto &s : config.excluded) excl_c.push_back(s.c_str());
-  bvcf_config bc{};
-  bc.empty_field = config.emptyField.c_str();
-  bc.field_delim = config.fieldDelimiter.c_str();
-  bc.keep_id = config.keepID; bc.keep_info = config.keepInfo; bc.keep_pos = config.keepPos;
-  bc.want_tsv = !config.noOut; bc.want_dosage = want_dosage;
-  bc.allow = allow_c.data(); bc.n_allow = config.allowAll ? -1 : (int)allow_c.size();
-  bc.exclude = excl_c.data(); bc.n_exclude = (int)excl_c.size();
-  bc.eol_width = eol_width; bc.normalize_dots = 1;
   const int n_slots = 3;
-  bc.n_slots = n_slots;
   const size_t cap = 2 * config.chunkBytes + (64u << 20);  // a chunk grows until it holds a newline
-  bc.max_chunk_bytes = cap;
   const int n_gpu = config.gpus;
   std::vector<bvcf_ctx *> ctxs(n_gpu, nullptr);
   std::vector<BufferPool> pools(n_gpu);
   std::vector<std::unique_ptr<ChunkQueue>> queues;
   for (int g = 0; g < n_gpu; g++) {
-    int rc = bvcf_create(&ctxs[g], config.devices.empty() ? g : config.devices[g], &bc);
-    if (rc) fatal(std::string("bvcf_create(gpu ") + std::to_string(g) + "): " + bvcf_strerror(rc) + " -- a CUDA device is required, there is no CPU fallback");
-    rc = bvcf_set_header(ctxs[g], chrom_line.data(), chrom_line.size());
-    if (rc) fatal(std::string("bvcf_set_header: ") + bvcf_strerror(rc));
+    ctxs[g] = open_ctx(config, config.devices.empty() ? g : config.devices[g], pre, sink.want_dosage(), n_slots, cap);
     for (int k = 0; k < n_slots + 2; k++) {
       uint8_t *b = nullptr;
       if (bvcf_host_alloc((void **)&b, cap)) fatal("bvcf_host_alloc failed");
@@ -932,11 +776,8 @@ int main(int argc, char **argv) {
         fatal(std::string("bvcf_diag_fields: ") + bvcf_strerror(rc2) + " " + bvcf_last_error(ctx));
       }
       turn.wait_for(c.seq);  // input order
-      if (!config.noOut) write_all(out_fd, tsv, n);
-#ifndef BVCF_NO_ARROW
-      if (arrow && dos.n_rows && bvcf_arrow_write(arrow, dos.n_rows, dos.dosage, dos.loci, dos.loci_off))
-        fatal(std::string("dosage output: ") + bvcf_arrow_error(arrow));
-#endif
+      sink.rows(tsv, n);
+      sink.dosage(dos);
       if (c.gz) log_diag_fields(ftext, foff, dg, nd);
       else log_diags(c.buf, c.len, dg, nd);
       turn.done();
@@ -950,25 +791,26 @@ int main(int argc, char **argv) {
   // ---- reader: newline-aligned chunks, chunk k to GPU k mod N ----
   uint64_t seq = 0;
   if (gz) {  // groups of whole bgzf blocks: a mapped input is staged by the workers, a pipe's by the reader
-    plan_bgzf_groups(*gz, data_off, config.chunkBytes, cap, [&](size_t lo_b, size_t hi_b, size_t skip, const std::string &tail) {
+    plan_bgzf_groups(*gz, pre.data_off, config.chunkBytes, cap, [&](size_t lo_b, size_t hi_b, size_t skip, const std::string &tail) {
       const size_t lo = gz->off(lo_b), hi = gz->off(hi_b);
       if (hi - lo > cap) fatal("a bgzf group exceeds the chunk capacity; raise --chunkBytes");
       Chunk c;
       c.seq = seq; c.len = hi - lo; c.gz = true; c.skip = skip; c.tail = tail;
-      if (map) {
-        c.src = map + lo;
+      if (in.mapped()) {
+        c.src = in.at(lo);
       } else {
         c.buf = pools[seq % n_gpu].take();
-        memcpy(c.buf, gz->at(lo), c.len);
-        gz->release_before(hi);
+        memcpy(c.buf, in.at(lo), c.len);
+        in.release_before(hi);
       }
       queues[seq % n_gpu]->push(std::move(c));
       seq++;
     });
-  } else if (map) {
-    size_t p = data_off;
+  } else if (in.mapped()) {
+    const uint8_t *map = in.at(0);
+    size_t p = pre.data_off;
     // an unterminated last line is dropped (main.go:354-357)
-    size_t end = map_len;
+    size_t end = in.end();
     {
       const uint8_t *last = end > p ? (const uint8_t *)memrchr(map + p, '\n', end - p) : nullptr;
       end = last ? (size_t)(last - map) + 1 : p;
@@ -990,15 +832,15 @@ int main(int argc, char **argv) {
       seq++;
       p = q;
     }
-  } else {
+  } else {  // a pipe is read straight into the pinned buffers, after what the preamble search has read already
     uint8_t *buf = pools[0].take();
-    size_t fill = head.size() - data_off;  // bytes already in the current buffer
+    size_t fill = in.end() - pre.data_off;  // bytes already in the current buffer
     if (fill > cap) fatal("header buffer larger than a chunk");
-    memcpy(buf, head.data() + data_off, fill);
-    head.clear(); head.shrink_to_fit();
+    memcpy(buf, in.at(pre.data_off), fill);
+    bool eof = in.eof();
     while (!eof || fill) {
       while (!eof && fill < config.chunkBytes) {
-        ssize_t r = read(in_fd, buf + fill, std::min(cap - fill, config.chunkBytes - fill));
+        ssize_t r = read(in.fd(), buf + fill, std::min(cap - fill, config.chunkBytes - fill));
         if (r < 0) { if (errno == EINTR) continue; fatal(std::string("read: ") + strerror(errno)); }
         if (r == 0) { eof = true; break; }
         fill += (size_t)r;
@@ -1007,7 +849,7 @@ int main(int argc, char **argv) {
       if (!last_nl) {
         if (eof) break;  // an unterminated last line is dropped (main.go:354-357)
         if (fill >= cap) fatal("a single line exceeds the chunk capacity; raise --chunkBytes");
-        ssize_t r = read(in_fd, buf + fill, cap - fill);
+        ssize_t r = read(in.fd(), buf + fill, cap - fill);
         if (r <= 0) { eof = true; continue; }
         fill += (size_t)r;
         continue;
@@ -1026,11 +868,85 @@ int main(int argc, char **argv) {
   }
   for (auto &q : queues) q->close();
   for (auto &t : threads) t.join();
-  int rc_exit = 0;
-#ifndef BVCF_NO_ARROW
-  if (arrow && bvcf_arrow_close(arrow)) rc_exit = 1;
-#endif
   for (auto c : ctxs) bvcf_destroy(c);
+}
+
+}  // namespace
+
+int main(int argc, char **argv) {
+  Config config = setup(argc, argv);
+  int in_fd = 0;
+  if (!config.inPath.empty() && (in_fd = open(config.inPath.c_str(), O_RDONLY)) < 0) fatal(config.inPath + ": " + strerror(errno));
+  // main.go:150-156 re-points os.Stderr at the file, which Go's `log` never looks at again; what the flag evidently
+  // means is honoured here: diagnostics are appended to it
+  if (!config.errPath.empty() && !freopen(config.errPath.c_str(), "a", stderr)) fatal(config.errPath + ": " + strerror(errno));
+  if (config.noOut && !config.outPath.empty()) fatal("Cannot specify --noOut and --out");                 // main.go:160
+  if (config.noOut && config.dosageMatrixOutPath.empty()) fatal("When specifying --noOut, must specify --dosageOutput");  // :164
+#ifdef BVCF_NO_ARROW
+  if (!config.dosageMatrixOutPath.empty())
+    fatal("--dosageOutput: this binary was built without libarrow (pyarrow was not found at build time); "
+          "python -m bystro_vcf_b200 writes the Arrow file");
+#endif
+  int out_fd = 1;
+  if (!config.noOut && !config.outPath.empty() &&
+      (out_fd = open(config.outPath.c_str(), O_WRONLY | O_CREAT, 0644)) < 0)  // no O_TRUNC, like main.go:172
+    fatal(config.outPath + ": " + strerror(errno));
+  if (!config.noOut) {
+    const std::string h = string_header(config) + "\n";  // main.go:199: before any input is read
+    if (config.bgzfOut) {
+      const std::vector<uint8_t> b = bgzf_block_host((const uint8_t *)h.data(), h.size());
+      write_all(out_fd, b.data(), b.size());
+    } else {
+      write_all(out_fd, (const uint8_t *)h.data(), h.size());
+    }
+  }
+
+  // ---- input: a regular file is memory-mapped, anything else (pipes) is read ----
+  const uint8_t *map = nullptr;
+  size_t map_len = 0;
+  struct stat sb;
+  if (in_fd != 0 && fstat(in_fd, &sb) == 0 && S_ISREG(sb.st_mode) && sb.st_size > 0) {
+    void *m = mmap(nullptr, (size_t)sb.st_size, PROT_READ, MAP_PRIVATE, in_fd, 0);
+    if (m != MAP_FAILED) {
+      map = (const uint8_t *)m;
+      map_len = (size_t)sb.st_size;
+      madvise(m, map_len, MADV_SEQUENTIAL);
+    }
+  }
+  std::vector<uint8_t> head;  // pipe input: enough bytes to tell a bgzf input
+  if (!map) {
+    head.resize(1 << 16);
+    size_t got = 0;
+    while (got < 18) {
+      const ssize_t r = read(in_fd, head.data() + got, head.size() - got);
+      if (r < 0) { if (errno == EINTR) continue; fatal(std::string("read: ") + strerror(errno)); }
+      if (r == 0) break;
+      got += (size_t)r;
+    }
+    head.resize(got);
+  }
+  Input in(in_fd, map, map_len, std::move(head));
+  std::unique_ptr<BgzfIn> gz;  // .vcf.gz (bgzf) input
+  if (looks_bgzf(in.at(0), in.end())) gz.reset(new BgzfIn(in));
+  // the rows are deflated where they are, on one GPU's resident regions
+  if (config.bgzfOut && config.gpus > 1) fatal("--bgzfOut runs on one GPU");
+
+  // ---- preamble (main.go:250-294): EOL, ##fileformat check, #CHROM line; a bgzf input's is inflated on the host ----
+  Preamble pre;
+  for (size_t want = 1u << 20;; want *= 4) {
+    if (gz) {
+      const std::string t = gz->prefix(want);
+      if (find_preamble((const uint8_t *)t.data(), t.size(), t.size() < want, pre)) break;
+    } else {
+      in.fill(want);
+      if (find_preamble(in.at(0), in.end(), in.eof(), pre)) break;
+    }
+  }
+
+  Sink sink(config, out_fd, pre.chrom_line);
+  if (config.bgzfOut) run_resident(config, in, gz.get(), pre, sink);
+  else run_streaming(config, in, gz.get(), pre, sink);
+  const int rc_exit = sink.close();
   if (map) munmap((void *)map, map_len);
   if (out_fd != 1) close(out_fd);
   return rc_exit;

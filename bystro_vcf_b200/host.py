@@ -502,27 +502,83 @@ class PinnedRing:
         self.ptrs = []
 
 
-def write_sample_list(config: Config, chrom_line: bytes, normalize: bool = True) -> None:
-    """writeSampleListIfWanted / makeSampleList main.go:398-445"""
-    if not config.sampleListPath:
-        return
-    f = chrom_line.split(b"\t")
-    with open(config.sampleListPath, "wb") as fh:
-        if len(f) >= 10:
-            for s in f[9:]:
-                fh.write((s.replace(b".", b"_") if normalize else s) + b"\n")
+def read_preamble(buf, gz: bool, reader: Optional[BinaryIO] = None):
+    """parse_preamble on the first bytes of an input: (eol_width, chrom_line, data_off), data_off counted in text bytes.
+    buf holds the input read so far -- a bytearray that grows from `reader` until the #CHROM line is in sight, or the
+    whole input (bytes, mmap) when there is no reader.  A bgzf input's first blocks are inflated on the host, each one
+    checked against its CRC-32 (BvcfError when one fails)."""
+    from . import bgzf
+
+    want = 1 << 20
+    while True:
+        while reader is not None and len(buf) < want:
+            more = reader.read(want - len(buf))
+            if not more:
+                reader = None
+            buf += more
+        try:
+            text = bgzf.inflate_host(buf, want) if gz else bytes(buf[:want])
+        except ValueError as e:
+            raise BvcfError(str(e)) from None
+        try:
+            return parse_preamble(text)
+        except NotAVcfError as e:
+            if (str(e) == "Not a VCF file" and re.search(rb"[\r\n]", text)) or (reader is None and len(text) < want):
+                raise
+            want *= 4
+
+
+class Sink:
+    """Where the results of a run go (main.go:296-343, 398-445): rows to the writer, dosage batches to the Arrow file, the
+    reference's log lines to diag_sink(text, line_no, alt_no, code), and the totals.  Built once from the #CHROM line:
+    it writes the sample list and opens the dosage file -- or, when the VCF has no samples, writes an empty one."""
+
+    def __init__(self, config: Config, chrom_line: bytes, writer: Optional[BinaryIO] = None, diag_sink=None):
+        self.config, self.writer, self.diag_sink = config, writer, diag_sink
+        names = [s.replace(b".", b"_") if config.normalizeHeader else s for s in chrom_line.split(b"\t")[9:]]
+        if config.sampleListPath and not config.noOut:  # writeSampleListIfWanted / makeSampleList main.go:398-445
+            with open(config.sampleListPath, "wb") as fh:
+                fh.write(b"".join(s + b"\n" for s in names))
+        self.arrow = None
+        if config.dosageMatrixOutPath and not names:
+            open(config.dosageMatrixOutPath, "wb").close()  # main.go:308-318: no samples, an empty dosage file
+        elif config.dosageMatrixOutPath:
+            from .dosage import DosageWriter  # Arrow IPC framing (SURVEY 8f-2)
+
+            self.arrow = DosageWriter(config.dosageMatrixOutPath, names)
+        self.totals = {"n_lines": 0, "n_records": 0, "n_rows": 0, "out_bytes": 0}
+
+    def put(self, res: ChunkResult, loci) -> None:
+        """one chunk's results, in input order.  res.tsv is written as it is (bgzf blocks with bgzfOut); loci yields the
+        (CHROM, POS) of each diagnostic's line -- read from the chunk's text with locus_at, or res.diag_fields."""
+        if self.writer is not None and not self.config.noOut:
+            self.writer.write(res.tsv)
+        if self.arrow is not None and res.dosage is not None:
+            self.arrow.write(res.loci, res.dosage)
+        if self.diag_sink is not None and res.diags:
+            for (ln, alt_no, code), (chrom, pos) in zip(res.diags, loci):
+                self.diag_sink(format_diag(chrom, pos, alt_no, code), self.totals["n_lines"] + ln, alt_no, code)
+        self.totals["n_lines"] += res.n_lines
+        self.totals["n_records"] += res.n_records
+        self.totals["n_rows"] += res.n_rows
+        self.totals["out_bytes"] += len(res.tsv)
+
+    def close(self) -> None:
+        if self.arrow is not None:
+            self.arrow.close()
+            self.arrow = None
 
 
 def _read_vcf_resident(config: Config, head: bytes, reader: BinaryIO, writer: Optional[BinaryIO], batch_text: int = 512 << 20,
-                       diag_sink=None, compressed_in: bool = True) -> dict:
-    """readVcf (main.go:241-396) over the resident regions, for compressed streams on either side.
-    compressed_in: groups of whole bgzf blocks are uploaded COMPRESSED and inflated on the GPU straight into the
-    resident input region (replaces the `pigz -d -c |` in front of the reference, README.md:10); otherwise groups
-    of plain text are uploaded.  The transform runs there; rows, dosage batches and diagnostics come back -- the
-    rows as bgzf blocks deflated on the GPU when config.bgzfOut (replaces the `| pigz -c` behind it)."""
+                       diag_sink=None) -> dict:
+    """readVcf (main.go:241-396) for bgzfOut: the rows are deflated where they are made (replaces the `| pigz -c` behind
+    the reference, README.md:10), so the input goes through one GPU's resident regions a group at a time -- plain text
+    uploaded, or whole bgzf blocks inflated on the GPU.  The partial line at a group's end is carried into the next."""
     from . import bgzf
 
     buf = bytearray(head)
+    gz = bgzf.is_bgzf(bytes(buf[:18]))
+    width, chrom_line, data_off = read_preamble(buf, gz, reader)
     eof = False
 
     def fill(n: int):
@@ -534,220 +590,150 @@ def _read_vcf_resident(config: Config, head: bytes, reader: BinaryIO, writer: Op
             else:
                 buf.extend(more)
 
-    # ---- preamble: inflate the first blocks on the host until the #CHROM line is in sight ----
-    want = 1 << 20
-    while True:
-        fill(want)
-        text0 = bgzf.inflate_host(buf, want * 4) if compressed_in else bytes(buf)
-        try:
-            width, chrom_line, data_off = parse_preamble(text0)
-            break
-        except NotAVcfError as e:
-            if (str(e) == "Not a VCF file" and re.search(rb"[\r\n]", text0)) or eof:
-                raise
-            want *= 4
-    totals = {"n_lines": 0, "n_records": 0, "n_rows": 0, "out_bytes": 0, "in_bytes": 0, "compressed_bytes": 0}
-    if not config.noOut:
-        write_sample_list(config, chrom_line, config.normalizeHeader)
+    compressed_bytes = in_bytes = 0
     max_line = 8 << 20  # room for the carried partial line
-    arrow = None
-    n_samples_hdr = max(len(chrom_line.split(b"\t")) - 9, 0)
-    if config.dosageMatrixOutPath and n_samples_hdr == 0:
-        open(config.dosageMatrixOutPath, "wb").close()  # main.go:308-318
-    elif config.dosageMatrixOutPath:
-        from .dosage import DosageWriter
-
-        names = [s.replace(b".", b"_") if config.normalizeHeader else s for s in chrom_line.split(b"\t")[9:]]
-        arrow = DosageWriter(config.dosageMatrixOutPath, names)
-    with Transformer(config, eol_width=width) as tr:
-        tr.set_header(chrom_line)
-        tr.resident_alloc(batch_text + max_line + (1 << 20), batch_text // 4 + (64 << 20))
-        carry = b""
-        begin = data_off  # the first group holds the meta lines and the header: they are skipped on the device
-        while True:
-            # ---- a group of whole blocks worth about batch_text bytes of text ----
-            p = text = 0
-            if not compressed_in:
-                fill(batch_text)
-                p = min(len(buf), batch_text)
-            while compressed_in and text < batch_text:
-                fill(p + (1 << 16) + 18)
-                bs = bgzf.block_size(buf, p)
-                if bs == 0 or p + bs > len(buf):
-                    if not eof:
-                        fill(p + max(bs, 1 << 16) + 18)
-                        continue
+    sink = Sink(config, chrom_line, writer, diag_sink)
+    try:
+        with Transformer(config, eol_width=width) as tr:
+            tr.set_header(chrom_line)
+            tr.resident_alloc(batch_text + max_line + (1 << 20), batch_text // 4 + (64 << 20))
+            carry = b""
+            begin = data_off  # the first group holds the meta lines and the header: they are skipped on the device
+            while True:
+                # ---- a group: whole blocks worth about batch_text bytes of text, or batch_text bytes of plain text ----
+                p = text = 0
+                if not gz:
+                    fill(batch_text)
+                    p = min(len(buf), batch_text)
+                while gz and text < batch_text:
+                    fill(p + (1 << 16) + 18)
+                    bs = bgzf.block_size(buf, p)
+                    if bs == 0 or p + bs > len(buf):
+                        if not eof:
+                            fill(p + max(bs, 1 << 16) + 18)
+                            continue
+                        if p < len(buf):
+                            raise BvcfError("bgzf input: truncated block at the end")
+                        break
+                    text += int.from_bytes(buf[p + bs - 4:p + bs], "little")
+                    p += bs
+                if p == 0:
                     break
-                text += int.from_bytes(buf[p + bs - 4:p + bs], "little")
-                p += bs
-            if p == 0:
-                break
-            group = bytes(buf[:p])
-            del buf[:p]
-            if carry:
-                tr.resident_upload(0, carry)
-            if compressed_in:
-                n_text = tr.resident_inflate_bgzf(group, len(carry))
-            else:
-                tr.resident_upload(len(carry), group)
-                n_text = len(group)
-            total = len(carry) + n_text
-            totals["compressed_bytes"] += len(group)
-            # ---- the longest newline-terminated prefix; what follows it is carried into the next group ----
-            tail_n = min(total - begin, max_line)
-            tail = tr.resident_peek(total - tail_n, tail_n) if tail_n > 0 else b""
-            k = tail.rfind(b"\n")
-            if k < 0:
-                if tail_n == total - begin:  # no complete line in this group at all
-                    carry = carry + tr.resident_peek(len(carry), n_text) if begin == 0 else tr.resident_peek(begin, total - begin)
-                    begin = 0
-                    continue
-                raise BvcfError("a single line exceeds %d bytes" % max_line)
-            end = total - tail_n + k + 1
-            stats, _ = tr.resident_run(end, want_times=False, begin=begin)
-            if writer is not None and not config.noOut and stats["out_bytes"]:
-                if config.bgzfOut:
-                    writer.write(tr.resident_download_bgzf(0, stats["out_bytes"]))
+                group = bytes(buf[:p])
+                del buf[:p]
+                if carry:
+                    tr.resident_upload(0, carry)
+                if gz:
+                    n_text = tr.resident_inflate_bgzf(group, len(carry))
                 else:
-                    writer.write(tr.resident_download(0, stats["out_bytes"]))
-            if arrow is not None or diag_sink is not None:
+                    tr.resident_upload(len(carry), group)
+                    n_text = len(group)
+                total = len(carry) + n_text
+                compressed_bytes += len(group)
+                # ---- the longest newline-terminated prefix; what follows it is carried into the next group ----
+                tail_n = min(total - begin, max_line)
+                tail = tr.resident_peek(total - tail_n, tail_n) if tail_n > 0 else b""
+                k = tail.rfind(b"\n")
+                if k < 0:
+                    if tail_n == total - begin:  # no complete line in this group at all
+                        carry = carry + tr.resident_peek(len(carry), n_text) if begin == 0 else tr.resident_peek(begin, total - begin)
+                        begin = 0
+                        continue
+                    raise BvcfError("a single line exceeds %d bytes" % max_line)
+                end = total - tail_n + k + 1
+                stats, _ = tr.resident_run(end, want_times=False, begin=begin)
+                rows = b""
+                if writer is not None and not config.noOut and stats["out_bytes"]:
+                    rows = tr.resident_download_bgzf(0, stats["out_bytes"])
                 loci, dosage, diags = tr.resident_results()
-                if arrow is not None and dosage is not None:
-                    arrow.write(loci, dosage)
-                if diag_sink is not None:
-                    for ln, alt_no, code, st in diags:
-                        chrom, pos = locus_at(tr.resident_peek(st, min(4096, end - st)), 0)
-                        diag_sink(format_diag(chrom, pos, alt_no, code), totals["n_lines"] + ln, alt_no, code)
-            for key in ("n_lines", "n_records", "n_rows", "out_bytes"):
-                totals[key] += stats[key]
-            totals["in_bytes"] += end - begin
-            carry = tail[k + 1:]
-            begin = 0
-        # an unterminated last line (carry) is dropped (main.go:354-357)
-    if arrow is not None:
-        arrow.close()
-    return totals
+                res = ChunkResult(tsv=rows, n_lines=stats["n_lines"], n_records=stats["n_records"], n_rows=stats["n_rows"],
+                                  diags=[d[:3] for d in diags], diag_starts=[d[3] for d in diags], loci=loci, dosage=dosage)
+                sink.put(res, (locus_at(tr.resident_peek(st, min(4096, end - st)), 0) for st in res.diag_starts))
+                in_bytes += end - begin
+                carry = tail[k + 1:]
+                begin = 0
+            # an unterminated last line (carry) is dropped (main.go:354-357)
+    finally:
+        sink.close()
+    return {**sink.totals, "in_bytes": in_bytes, "compressed_bytes": compressed_bytes}
 
 
-_read_vcf_bgzf = _read_vcf_resident  # the name round 2 first gave it
-
-
-def read_vcf(config: Config, reader: BinaryIO, writer: Optional[BinaryIO], transformer: Optional[Transformer] = None,
-             diag_sink=None) -> dict:
+def read_vcf(config: Config, reader: BinaryIO, writer: Optional[BinaryIO], diag_sink=None) -> dict:
     """readVcf (main.go:241-396) on the GPU: header discovery on the host, every data line on the device.
 
     reader/writer are binary file objects (the reference's *bufio.Reader / *bufio.Writer).  Rows are
     written in input order.  The TSV header line is NOT written here (main() does that, main.go:199).
-    diag_sink(text, line_no, alt_no, code) receives the reference's log.Printf line for every skipped allele."""
+    diag_sink(text, line_no, alt_no, code) receives the reference's log.Printf line for every skipped allele.
+    A .vcf.gz (bgzf) input runs on the streaming path of shard.read_vcf_multi with config.device as its one GPU."""
+    from . import bgzf, shard
+
     chunk_bytes = max(int(config.chunkBytes), 1 << 16)
-    head = reader.read(1 << 20)
-    from . import bgzf
-
-    if bgzf.is_bgzf(head):  # .vcf.gz: the compressed bytes go to the GPU, which inflates them (SURVEY 8f-3)
-        if transformer is not None:
-            raise BvcfError("read_vcf: pass no transformer for bgzf input")
-        return _read_vcf_resident(config, head, reader, writer, diag_sink=diag_sink)
+    head = bytearray(reader.read(1 << 20))
     if config.bgzfOut:  # the rows are deflated where they are: on the device
-        if transformer is not None:
-            raise BvcfError("read_vcf: pass no transformer with bgzfOut")
-        return _read_vcf_resident(config, head, reader, writer, diag_sink=diag_sink, compressed_in=False)
-    while True:  # make sure the whole preamble (meta lines + #CHROM line) is in `head`
-        try:
-            width, chrom_line, off = parse_preamble(head)
-            break
-        except NotAVcfError as e:
-            first_line_done = re.search(rb"[\r\n]", head) is not None
-            if str(e) == "Not a VCF file" and first_line_done:
-                raise
-            more = reader.read(1 << 20)
-            if not more:
-                raise
-            head += more
-    own = transformer is None
-    tr = transformer or Transformer(config, eol_width=width, max_chunk_bytes=2 * chunk_bytes + (64 << 20))
-    totals = {"n_lines": 0, "n_records": 0, "n_rows": 0, "out_bytes": 0, "in_bytes": 0}
-    arrow = None
+        return _read_vcf_resident(config, head, reader, writer, diag_sink=diag_sink)
+    if bgzf.is_bgzf(bytes(head[:18])):  # .vcf.gz: the compressed bytes go to the GPU, which inflates them (SURVEY 8f-3)
+        return shard.read_vcf_multi(config, shard.whole_input(reader, head), writer, [config.device], diag_sink=diag_sink)
+    width, chrom_line, off = read_preamble(head, False, reader)
+    # chunks are staged in pinned host buffers (bvcf_host_alloc) and read into them directly: a pageable source
+    # would make the driver bounce every H2D copy through its own staging buffer
+    cap = 2 * chunk_bytes + (64 << 20)
+    in_bytes = 0
+    sink = Sink(config, chrom_line, writer, diag_sink)
     try:
-        tr.set_header(chrom_line)
-        if not config.noOut:
-            write_sample_list(config, chrom_line, config.normalizeHeader)
-        n_samples_hdr = max(len(chrom_line.split(b"\t")) - 9, 0)
-        if config.dosageMatrixOutPath and n_samples_hdr == 0:
-            # main.go:308-318: no samples -> an empty dosage file, and no dosage work
-            open(config.dosageMatrixOutPath, "wb").close()
-        elif config.dosageMatrixOutPath:
-            from .dosage import DosageWriter  # Arrow IPC framing (SURVEY 8f-2)
+        with Transformer(config, eol_width=width, max_chunk_bytes=cap) as tr:
+            tr.set_header(chrom_line)
+            ring = PinnedRing(tr.n_slots + 1, cap)
+            seq_in = seq_out = 0
+            pending = {}  # seq -> the chunk's text (a view of its ring buffer) while it is in flight
 
-            names = [s.replace(b".", b"_") if config.normalizeHeader else s for s in chrom_line.split(b"\t")[9:]]
-            arrow = DosageWriter(config.dosageMatrixOutPath, names)
-        # chunks are staged in pinned host buffers (bvcf_host_alloc) and read into them directly: a pageable source
-        # would make the driver bounce every H2D copy through its own staging buffer
-        cap = 2 * chunk_bytes + (64 << 20) if transformer is None else max(2 * chunk_bytes, 1 << 20)
-        ring = PinnedRing(tr.n_slots + 1, cap)
-        seq_in = seq_out = 0
-        pending = {}  # seq -> (address, length) of the chunk while it is in flight
+            def drain(upto: int):
+                nonlocal seq_out
+                while seq_out < upto:
+                    res = tr.collect(seq_out)
+                    text = pending.pop(seq_out)
+                    sink.put(res, (locus_at(text, st) for st in res.diag_starts))
+                    seq_out += 1
 
-        def drain(upto: int):
-            nonlocal seq_out
-            while seq_out < upto:
-                res = tr.collect(seq_out)
-                addr, blen = pending.pop(seq_out, (0, 0))
-                if writer is not None and not config.noOut:
-                    writer.write(res.tsv)
-                if arrow is not None and res.dosage is not None:
-                    arrow.write(res.loci, res.dosage)
-                if diag_sink is not None and res.diags:
-                    for (ln, alt_no, code), st in zip(res.diags, res.diag_starts):
-                        chrom, pos = locus_at(C.string_at(addr + st, min(4096, blen - st)), 0)
-                        diag_sink(format_diag(chrom, pos, alt_no, code), totals["n_lines"] + ln, alt_no, code)
-                totals["n_lines"] += res.n_lines
-                totals["n_records"] += res.n_records
-                totals["n_rows"] += res.n_rows
-                totals["out_bytes"] += len(res.tsv)
-                seq_out += 1
-
-        try:
-            slot = 0
-            fill = len(head) - off  # bytes waiting in the current buffer
-            if fill > cap:
-                raise BvcfError("the VCF preamble does not fit a chunk buffer; raise chunkBytes")
-            C.memmove(ring.ptrs[0], head[off:], fill)
-            eof = False
-            while not eof or fill:
-                view = ring.views[slot]
-                while not eof and fill < chunk_bytes:
-                    n = reader.readinto(view[fill:min(cap, chunk_bytes)])
-                    if not n:
-                        eof = True
-                        break
-                    fill += n
-                cut = ring.last_newline(slot, fill)
-                if cut < 0:
-                    if eof:
-                        break  # an unterminated last line is dropped (main.go:354-357)
-                    if fill >= cap:
-                        raise BvcfError("a single line exceeds the chunk capacity; raise chunkBytes")
-                    n = reader.readinto(view[fill:cap])
-                    if not n:
-                        eof = True
-                    fill += n or 0
-                    continue
-                nxt = (slot + 1) % len(ring.ptrs)
-                if seq_in - seq_out >= tr.n_slots:
-                    drain(seq_out + 1)  # frees the next ring buffer too (n_slots + 1 buffers, n_slots in flight)
-                C.memmove(ring.ptrs[nxt], ring.ptrs[slot] + cut, fill - cut)  # carry the partial line
-                pending[seq_in] = (ring.ptrs[slot], cut)
-                tr.submit(seq_in, (ring.ptrs[slot], cut))
-                totals["in_bytes"] += cut
-                seq_in += 1
-                fill -= cut
-                slot = nxt
-            drain(seq_in)
-        finally:
-            ring.close()
+            try:
+                slot = 0
+                fill = len(head) - off  # bytes waiting in the current buffer
+                if fill > cap:
+                    raise BvcfError("the VCF preamble does not fit a chunk buffer; raise chunkBytes")
+                C.memmove(ring.ptrs[0], bytes(head[off:]), fill)
+                eof = False
+                while not eof or fill:
+                    view = ring.views[slot]
+                    while not eof and fill < chunk_bytes:
+                        n = reader.readinto(view[fill:min(cap, chunk_bytes)])
+                        if not n:
+                            eof = True
+                            break
+                        fill += n
+                    cut = ring.last_newline(slot, fill)
+                    if cut < 0:
+                        if eof:
+                            break  # an unterminated last line is dropped (main.go:354-357)
+                        if fill >= cap:
+                            raise BvcfError("a single line exceeds the chunk capacity; raise chunkBytes")
+                        n = reader.readinto(view[fill:cap])
+                        if not n:
+                            eof = True
+                        fill += n or 0
+                        continue
+                    nxt = (slot + 1) % len(ring.ptrs)
+                    if seq_in - seq_out >= tr.n_slots:
+                        drain(seq_out + 1)  # frees the next ring buffer too (n_slots + 1 buffers, n_slots in flight)
+                    C.memmove(ring.ptrs[nxt], ring.ptrs[slot] + cut, fill - cut)  # carry the partial line
+                    pending[seq_in] = view[:cut]
+                    tr.submit(seq_in, (ring.ptrs[slot], cut))
+                    in_bytes += cut
+                    seq_in += 1
+                    fill -= cut
+                    slot = nxt
+                drain(seq_in)
+            finally:
+                pending.clear()
+                ring.close()
     finally:
-        if arrow is not None:
-            arrow.close()
-        if own:
-            tr.close()
-    return totals
+        sink.close()
+    return {**sink.totals, "in_bytes": in_bytes}

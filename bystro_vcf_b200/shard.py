@@ -19,15 +19,16 @@ Both are pure host logic around bvcf_submit / bvcf_collect.
 from __future__ import annotations
 
 import ctypes as C
+import mmap
+import os
 import queue
-import re
+import stat
 import threading
 from typing import BinaryIO, List, Optional, Sequence, Tuple
 
 from . import bgzf
 from ._lib import BvcfError
-from .host import (Config, NotAVcfError, PinnedRing, Transformer, format_diag, locus_at, parse_preamble,
-                   write_sample_list)
+from .host import Config, PinnedRing, Sink, Transformer, locus_at, read_preamble
 
 
 def partition(data, begin: int, end: int, n: int) -> List[Tuple[int, int]]:
@@ -121,6 +122,18 @@ def _gpu_worker(cfg: Config, device: int, eol_width: int, chrom_line: bytes, dat
             ring.close()
 
 
+def whole_input(reader: BinaryIO, head: bytes = b""):
+    """The whole input of `reader`, of which `head` has been read already: the file mapped read-only when the reader is
+    a regular file read from its start, otherwise head + the rest read."""
+    try:
+        st = os.fstat(reader.fileno())
+        if stat.S_ISREG(st.st_mode) and st.st_size > 0 and reader.tell() == len(head):
+            return mmap.mmap(reader.fileno(), 0, access=mmap.ACCESS_READ)
+    except (AttributeError, OSError, ValueError):  # io.BytesIO and other readers without a file behind them
+        pass
+    return bytes(head) + reader.read()
+
+
 def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Sequence[int], diag_sink=None,
                    n_slots: int = 3) -> dict:
     """readVcf (main.go:241-396) over several GPUs of one box.  `data` is the whole uncompressed VCF as a bytes-like
@@ -129,42 +142,19 @@ def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Se
     working."""
     chunk_bytes = max(int(config.chunkBytes), 1 << 16)
     gz = bgzf.is_bgzf(bytes(data[:18]))
+    width, chrom_line, off = read_preamble(data, gz)
     if gz:
-        want = 1 << 20
-        while True:  # the preamble, inflated on the host
-            text0 = bgzf.inflate_host(data, want)
-            try:
-                width, chrom_line, off = parse_preamble(text0)
-                break
-            except NotAVcfError as e:
-                if (str(e) == "Not a VCF file" and re.search(rb"[\r\n]", text0)) or len(text0) < want:
-                    raise
-                want *= 4
         try:
             chunks = bgzf.plan_groups(data, off, chunk_bytes, 2 * chunk_bytes + (64 << 20))
         except ValueError as e:
             raise BvcfError(str(e)) from None
         end = off + sum(g.text - g.skip + len(g.tail) for g in chunks)
     else:
-        width, chrom_line, off = parse_preamble(bytes(data[:min(len(data), 64 << 20)]))
-        end = len(data)
-        last_nl = data.rfind(b"\n", off, end)
+        last_nl = data.rfind(b"\n", off, len(data))
         end = off if last_nl < 0 else last_nl + 1  # an unterminated last line is dropped (main.go:354-357)
         chunks = chunk_ranges(data, off, end, chunk_bytes)
     n_dev = len(devices)
-    totals = {"n_lines": 0, "n_records": 0, "n_rows": 0, "out_bytes": 0, "in_bytes": end - off, "n_chunks": len(chunks),
-              "devices": list(devices)}
-    if not config.noOut:
-        write_sample_list(config, chrom_line, config.normalizeHeader)
-    arrow = None
-    n_samples = max(len(chrom_line.split(b"\t")) - 9, 0)
-    if config.dosageMatrixOutPath and n_samples == 0:
-        open(config.dosageMatrixOutPath, "wb").close()  # main.go:308-318
-    elif config.dosageMatrixOutPath:
-        from .dosage import DosageWriter
-
-        names = [s.replace(b".", b"_") if config.normalizeHeader else s for s in chrom_line.split(b"\t")[9:]]
-        arrow = DosageWriter(config.dosageMatrixOutPath, names)
+    sink = Sink(config, chrom_line, writer, diag_sink)
     errors: list = []
     queues = [queue.Queue(maxsize=n_slots + 1) for _ in range(n_dev)]
     threads = []
@@ -180,24 +170,9 @@ def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Se
             if cid is None:
                 raise errors[0]
             assert cid == k
-            if writer is not None and not config.noOut:
-                writer.write(res.tsv)
-            if arrow is not None and res.dosage is not None:
-                arrow.write(res.loci, res.dosage)
-            if diag_sink is not None and res.diags:
-                if gz:
-                    loci = res.diag_fields
-                else:
-                    loci = [locus_at(data, chunks[k][0] + st) for st in res.diag_starts]
-                for (ln, alt_no, code), (chrom, pos) in zip(res.diags, loci):
-                    diag_sink(format_diag(chrom, pos, alt_no, code), totals["n_lines"] + ln, alt_no, code)
-            totals["n_lines"] += res.n_lines
-            totals["n_records"] += res.n_records
-            totals["n_rows"] += res.n_rows
-            totals["out_bytes"] += len(res.tsv)
+            sink.put(res, res.diag_fields if gz else (locus_at(data, chunks[k][0] + st) for st in res.diag_starts))
     finally:
-        if arrow is not None:
-            arrow.close()
+        sink.close()
         for q in queues:  # unblock workers if we are bailing out
             while True:
                 try:
@@ -208,4 +183,4 @@ def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Se
             t.join(timeout=60)
     if errors:
         raise errors[0]
-    return totals
+    return {**sink.totals, "in_bytes": end - off, "n_chunks": len(chunks), "devices": list(devices)}

@@ -318,9 +318,12 @@ def test_gpu_inflate_rejects_corrupt_blocks():
             tr.resident_inflate_bgzf(b"not bgzf at all, just text\n")
 
 
-def test_bgzf_vcf_matches_plain(chr1_fixture):
-    """a .vcf.gz (bgzf) through read_vcf: compressed bytes to the device, inflated there, rows identical to the plain path;
-    groups smaller than the file, so partial lines are carried from group to group"""
+def test_bgzf_vcf_resident_and_streaming_match_plain(chr1_fixture):
+    """a .vcf.gz (bgzf) through the resident (bgzfOut) driver: compressed bytes to the device, inflated there, rows
+    identical to the plain path; groups smaller than the file, so partial lines are carried from group to group.  Then
+    through read_vcf, which runs it on the streaming path."""
+    import dataclasses
+    import gzip
     import io
 
     from bystro_vcf_b200 import Config, bgzf, host, read_vcf
@@ -335,8 +338,9 @@ def test_bgzf_vcf_matches_plain(chr1_fixture):
     st0 = read_vcf(c, io.BytesIO(vcf), plain)
     for batch in (512 << 20, 7 << 20):
         out = io.BytesIO()
-        st = host._read_vcf_bgzf(c, comp[:1 << 20], io.BytesIO(comp[1 << 20:]), out, batch_text=batch)
-        assert out.getvalue() == plain.getvalue()
+        st = host._read_vcf_resident(dataclasses.replace(c, bgzfOut=True), comp[:1 << 20], io.BytesIO(comp[1 << 20:]), out,
+                                     batch_text=batch)
+        assert gzip.decompress(out.getvalue()) == plain.getvalue()
         assert st["n_rows"] == st0["n_rows"] and st["compressed_bytes"] <= len(comp)
     out = io.BytesIO()
     read_vcf(c, io.BytesIO(comp), out)  # auto-detected

@@ -94,13 +94,13 @@ def test_parse_preamble():
         B.parse_preamble(b"##fileformat=VCFv4.2\n1\t2\n")
 
 
-def test_sample_list_like_reference(tmp_path):
+def test_sink_writes_sample_list_like_reference(tmp_path):
     """main_test.go:171-293"""
     p = tmp_path / "s.list"
-    host.write_sample_list(B.Config(sampleListPath=str(p)), "\t".join(V.HDR_S4).encode())
+    host.Sink(B.Config(sampleListPath=str(p)), "\t".join(V.HDR_S4).encode())
     assert p.read_text().split() == ["Sample1", "Sample2", "Sample3", "Sample4"]
     p2 = tmp_path / "none.list"
-    host.write_sample_list(B.Config(sampleListPath=str(p2)), "\t".join(V.HDR8).encode())
+    host.Sink(B.Config(sampleListPath=str(p2)), "\t".join(V.HDR8).encode())
     assert p2.read_text() == ""
 
 
