@@ -15,15 +15,15 @@ EOF_BLOCK = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000
 MAX_TEXT = 65280  # text bytes per block (bgzip's choice: the compressed block always fits 64 KiB)
 
 
-def is_bgzf(head: bytes) -> bool:
-    return len(head) >= 18 and head[:4] == MAGIC and head[12:14] == b"BC"
-
-
-def block_size(buf, p: int) -> int:
-    """total size of the bgzf block that starts at buf[p] (0 when its header is not complete yet)"""
+def _header(buf, p: int) -> int:
+    """The header of the bgzf block at buf[p]: a gzip member with FLG.FEXTRA whose extra field holds a BC subfield with
+    SLEN 2 -- anywhere in the field (SAM spec 4.1).  The subfields are walked in order, one that runs past the end of the
+    field ends the walk, and the first BC subfield gives BSIZE - 1.  The C++ host (bgzf_header) and the library
+    (bgzf_walk) follow the same rule.  Returns the block size, or 0 when the header is not complete yet; raises
+    ValueError when it is not a bgzf header."""
     if len(buf) - p < 18:
         return 0
-    if bytes(buf[p:p + 4]) != MAGIC:
+    if buf[p] != 0x1F or buf[p + 1] != 0x8B or buf[p + 2] != 8 or not buf[p + 3] & 4:
         raise ValueError("not a bgzf block")
     xlen = buf[p + 10] | (buf[p + 11] << 8)
     if len(buf) - p < 12 + xlen:
@@ -31,6 +31,8 @@ def block_size(buf, p: int) -> int:
     q, end = p + 12, p + 12 + xlen
     while q + 4 <= end:
         slen = buf[q + 2] | (buf[q + 3] << 8)
+        if q + 4 + slen > end:
+            break
         if buf[q] == 66 and buf[q + 1] == 67 and slen == 2:
             bsize = (buf[q + 4] | (buf[q + 5] << 8)) + 1
             if bsize < 12 + xlen + 8:
@@ -38,6 +40,19 @@ def block_size(buf, p: int) -> int:
             return bsize
         q += 4 + slen
     raise ValueError("gzip member without the bgzf BC subfield")
+
+
+def is_bgzf(head) -> bool:
+    """the first bytes of an input start with a whole bgzf header"""
+    try:
+        return _header(head, 0) > 0
+    except ValueError:
+        return False
+
+
+def block_size(buf, p: int) -> int:
+    """total size of the bgzf block that starts at buf[p] (0 when its header is not complete yet)"""
+    return _header(buf, p)
 
 
 def _payload_text(buf, p: int, bs: int) -> bytes:
@@ -55,14 +70,18 @@ def _payload_text(buf, p: int, bs: int) -> bytes:
 
 def blocks(buf) -> List[tuple]:
     """(offset, size, ISIZE) of every block of a whole bgzf file.  A truncated last block or bytes that are not a bgzf
-    block raise ValueError."""
+    block raise ValueError.  A block that claims ISIZE 0 (normally only the EOF block) is inflated here, and raises
+    ValueError unless it holds no text and CRC-32 0: its text would otherwise be dropped without a word."""
     out = []
     p, n = 0, len(buf)
     while p < n:
         bs = block_size(buf, p)
         if bs == 0 or p + bs > n:
             raise ValueError("truncated bgzf block at byte %d" % p)
-        out.append((p, bs, int.from_bytes(buf[p + bs - 4:p + bs], "little")))
+        isize = int.from_bytes(buf[p + bs - 4:p + bs], "little")
+        if isize == 0:
+            _payload_text(buf, p, bs)
+        out.append((p, bs, isize))
         p += bs
     return out
 

@@ -70,9 +70,15 @@ std::vector<std::string> split_trim(const std::string &s) {
   return out;
 }
 
+// The reader thread and the GPU workers may fail at once: the first message wins, and the process ends without running
+// exit-time teardown (the CUDA runtime's among it) under threads that are still inside CUDA calls.  Output goes
+// through write(2), so nothing is left in a stdio buffer.
 [[noreturn]] void fatal(const std::string &msg) {  // log.Fatal
+  static std::mutex m;
+  m.lock();
   fprintf(stderr, "%s\n", msg.c_str());
-  exit(1);
+  fflush(stderr);
+  _exit(1);
 }
 
 // Go `flag` syntax: -x / --x, --x=v / --x v; bool flags --x or --x=true|false; stops at the first non-flag.
@@ -276,24 +282,34 @@ struct Turnstile {
 // Replaces the `pigz -d -c in.vcf.gz |` in front of the reference (README.md:10,46).  Groups of whole blocks are
 // uploaded and inflated on the GPU: into a slot's input buffer (bvcf_submit_bgzf), or with --bgzfOut into the resident
 // input region (bvcf_resident_inflate_bgzf).
-bool looks_bgzf(const uint8_t *p, size_t n) {
-  return n >= 18 && p[0] == 0x1f && p[1] == 0x8b && p[2] == 8 && (p[3] & 4) && p[12] == 'B' && p[13] == 'C';
-}
-size_t bgzf_block_size(const uint8_t *p, size_t n) {  // 0: header incomplete
+// The header of the bgzf block at p (the rule of bgzf.py block_size and of bgzf_walk in bvcf_api.cu): a gzip member with
+// FLG.FEXTRA whose extra field holds a BC subfield with SLEN 2 -- anywhere in the field (SAM spec 4.1).  The subfields
+// are walked in order, one that runs past the end of the field ends the walk, and the first BC subfield gives BSIZE - 1.
+// Returns the block size, 0 when the header is not complete in n bytes, BGZF_NOT_GZIP / BGZF_NO_BC / BGZF_TOO_SMALL.
+enum : long long { BGZF_NOT_GZIP = -1, BGZF_NO_BC = -2, BGZF_TOO_SMALL = -3 };
+long long bgzf_header(const uint8_t *p, size_t n) {
   if (n < 18) return 0;
-  if (p[0] != 0x1f || p[1] != 0x8b || p[2] != 8 || !(p[3] & 4)) fatal("bgzf input: bytes that are not a bgzf block");
+  if (p[0] != 0x1f || p[1] != 0x8b || p[2] != 8 || !(p[3] & 4)) return BGZF_NOT_GZIP;
   const size_t xlen = (size_t)p[10] | ((size_t)p[11] << 8);
   if (n < 12 + xlen) return 0;
   for (size_t q = 12; q + 4 <= 12 + xlen;) {
     const size_t slen = (size_t)p[q + 2] | ((size_t)p[q + 3] << 8);
+    if (q + 4 + slen > 12 + xlen) break;
     if (p[q] == 'B' && p[q + 1] == 'C' && slen == 2) {
       const size_t bsize = ((size_t)p[q + 4] | ((size_t)p[q + 5] << 8)) + 1;
-      if (bsize < 12 + xlen + 8) fatal("bgzf input: a block smaller than its header and trailer");
-      return bsize;
+      return bsize < 12 + xlen + 8 ? BGZF_TOO_SMALL : (long long)bsize;
     }
     q += 4 + slen;
   }
-  fatal("gzip input without the bgzf BC subfield: decompress it first (gzip -dc | ...)");
+  return BGZF_NO_BC;
+}
+bool looks_bgzf(const uint8_t *p, size_t n) { return bgzf_header(p, n) > 0; }
+size_t bgzf_block_size(const uint8_t *p, size_t n) {  // 0: header incomplete
+  const long long r = bgzf_header(p, n);
+  if (r == BGZF_NOT_GZIP) fatal("bgzf input: bytes that are not a bgzf block");
+  if (r == BGZF_NO_BC) fatal("gzip input without the bgzf BC subfield: decompress it first (gzip -dc | ...)");
+  if (r == BGZF_TOO_SMALL) fatal("bgzf input: a block smaller than its header and trailer");
+  return (size_t)r;
 }
 
 // one bgzf block (SAM spec 4.1) around `text` (< 64 KiB), deflated on the host: the TSV header line
@@ -403,7 +419,10 @@ class BgzfIn {
       if (!bs || walk_ + bs > in_.end()) fatal("bgzf input: truncated block at the end");
       const uint8_t *e = in_.at(walk_ + bs - 4);
       const uint32_t isize = (uint32_t)e[0] | ((uint32_t)e[1] << 8) | ((uint32_t)e[2] << 16) | ((uint32_t)e[3] << 24);
+      // a block that claims no text is checked here (normally only the 28-byte EOF block): one that inflates to text
+      // would otherwise have that text dropped without a word
       if (isize) blk_.push_back({walk_, bs, text_, isize});
+      else inflate_checked({walk_, bs, text_, 0});
       text_ += isize;
       walk_ += bs;
     }
@@ -418,8 +437,17 @@ class BgzfIn {
     return b;
   }
   // block i inflated on the host, its CRC-32 and ISIZE checked
-  std::string inflate_block(size_t i) {
-    const Blk &b = blk_[i];
+  std::string inflate_block(size_t i) { return inflate_checked(blk_[i]); }
+  // the first `want` text bytes (fewer at the end of the input): the preamble
+  std::string prefix(size_t want) {
+    std::string out;
+    for (size_t i = 0; out.size() < want && has(i); i++) out += inflate_block(i);
+    return out;
+  }
+
+ private:
+  // the text of block b, inflated with zlib; a block that fails its CRC-32 or ISIZE is fatal
+  std::string inflate_checked(const Blk &b) {
     const uint8_t *p = in_.at(b.off);
     const size_t xlen = (size_t)p[10] | ((size_t)p[11] << 8);
     std::string text(b.isize, '\0');
@@ -436,14 +464,7 @@ class BgzfIn {
       fatal("bgzf input: a corrupt block (inflate, CRC-32 or ISIZE check failed)");
     return text;
   }
-  // the first `want` text bytes (fewer at the end of the input): the preamble
-  std::string prefix(size_t want) {
-    std::string out;
-    for (size_t i = 0; out.size() < want && has(i); i++) out += inflate_block(i);
-    return out;
-  }
 
- private:
   Input &in_;
   size_t walk_ = 0;
   uint64_t text_ = 0;

@@ -369,10 +369,11 @@ __global__ void __launch_bounds__(32) bvcf_inflate_kernel(const InflateParams p)
       if (b.overrun()) { err = 20; break; }
       __syncwarp();
       if (lengths[256] == 0) { err = 13; break; }
+      // an incomplete code is allowed only as a single code of one bit (RFC 1951 3.2.7, as zlib and puff.c read it)
       int r = inf_construct(lc, lengths, nlen);
-      if (r < 0 || (r > 0 && nlen - lc.count[0] != 1)) { err = 14; break; }
+      if (r < 0 || (r > 0 && !(lc.count[1] == 1 && nlen - lc.count[0] == 1))) { err = 14; break; }
       r = inf_construct(dc, lengths + nlen, ndist);
-      if (r < 0 || (r > 0 && ndist - dc.count[0] != 1)) { err = 15; break; }
+      if (r < 0 || (r > 0 && !(dc.count[1] == 1 && ndist - dc.count[0] == 1))) { err = 15; break; }
       err = inf_codes(b, lc, dc, w, lane);
     } else {
       err = 16;

@@ -577,7 +577,7 @@ def _read_vcf_resident(config: Config, head: bytes, reader: BinaryIO, writer: Op
     from . import bgzf
 
     buf = bytearray(head)
-    gz = bgzf.is_bgzf(bytes(buf[:18]))
+    gz = bgzf.is_bgzf(buf)
     width, chrom_line, data_off = read_preamble(buf, gz, reader)
     eof = False
 
@@ -671,7 +671,7 @@ def read_vcf(config: Config, reader: BinaryIO, writer: Optional[BinaryIO], diag_
     head = bytearray(reader.read(1 << 20))
     if config.bgzfOut:  # the rows are deflated where they are: on the device
         return _read_vcf_resident(config, head, reader, writer, diag_sink=diag_sink)
-    if bgzf.is_bgzf(bytes(head[:18])):  # .vcf.gz: the compressed bytes go to the GPU, which inflates them (SURVEY 8f-3)
+    if bgzf.is_bgzf(head):  # .vcf.gz: the compressed bytes go to the GPU, which inflates them (SURVEY 8f-3)
         return shard.read_vcf_multi(config, shard.whole_input(reader, head), writer, [config.device], diag_sink=diag_sink)
     width, chrom_line, off = read_preamble(head, False, reader)
     # chunks are staged in pinned host buffers (bvcf_host_alloc) and read into them directly: a pageable source

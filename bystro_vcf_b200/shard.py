@@ -141,7 +141,7 @@ def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Se
     be listed more than once); rows, dosage batches and diagnostics leave in input order while the GPUs are still
     working."""
     chunk_bytes = max(int(config.chunkBytes), 1 << 16)
-    gz = bgzf.is_bgzf(bytes(data[:18]))
+    gz = bgzf.is_bgzf(data)
     width, chrom_line, off = read_preamble(data, gz)
     if gz:
         try:

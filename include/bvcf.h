@@ -173,7 +173,8 @@ int bvcf_resident_run_at(bvcf_ctx *ctx, size_t begin, size_t len, bvcf_chunk_sta
  * whole bgzf blocks.  text_bytes receives the uncompressed size.  BVCF_E_ARG: not bgzf, corrupt (including a CRC-32
  * mismatch), or larger than the region. */
 int bvcf_resident_inflate_bgzf(bvcf_ctx *ctx, const void *comp, size_t comp_len, size_t dst_offset, size_t *text_bytes);
-/* Host only: the uncompressed size (sum of ISIZE) and block count of a bgzf buffer of whole blocks. */
+/* Host only: the uncompressed size (sum of ISIZE) and block count of a bgzf buffer of whole blocks.  Every member is
+ * counted, those with ISIZE 0 (the EOF block among them) too: the GPU inflates and checks them like any other. */
 int bvcf_bgzf_text_bytes(const void *comp, size_t comp_len, uint64_t *text_bytes, uint64_t *n_blocks);
 
 /* bgzf-compressed output (downstream of the reference stands `| pigz -c`, README.md:10,71): the rows in
