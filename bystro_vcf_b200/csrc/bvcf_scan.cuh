@@ -115,28 +115,30 @@ __device__ __forceinline__ uint32_t pack_quad(const uint32_t t[4], bool dots) {
   }
   return t[0] | (t[1] << 4) | (t[2] << 8) | (t[3] << 12);  // digits: every allele byte is already a nibble
 }
-// ALT #1 bookkeeping of one quad payload (diploid fields only: the vector path)
-__device__ __forceinline__ void acc_quad(LineAcc &a, uint32_t pl, bool dots) {
-  const uint32_t y = pl ^ 0x11111111u;
-  uint32_t one = ~(((y & 0x77777777u) + 0x77777777u) | y) & 0x88888888u;  // bit 3 of every nibble equal to 1
-  uint32_t big = pl & 0xEEEEEEEEu;                                         // nibbles >= 2
+__device__ __forceinline__ uint32_t nibbles_eq(uint32_t pl, uint32_t rep) {  // bit 3 of every nibble equal to rep's
+  const uint32_t y = pl ^ rep;
+  return ~(((y & 0x77777777u) + 0x77777777u) | y) & 0x88888888u;
+}
+// ALT #1 bookkeeping of the quad payloads of two windows (diploid fields only: the vector path; pb = 0 for one
+// window).  Window B's marks are moved one bit below A's, so one popc counts both.
+__device__ __forceinline__ void acc_quad_pair(LineAcc &a, uint32_t pa, uint32_t pb, bool dots) {
+  uint32_t oa = nibbles_eq(pa, 0x11111111u), ob = nibbles_eq(pb, 0x11111111u);
   if (dots) {
-    const uint32_t d = pl ^ 0xEEEEEEEEu;
-    const uint32_t dot = ~(((d & 0x77777777u) + 0x77777777u) | d) & 0x88888888u;  // nibbles equal to 0xE
-    const uint32_t mf = (dot | (dot >> 16)) & 0x8888u;    // samples with a '.' token: missing (main.go:1113,1150)
-    const uint32_t nm = __popc(mf);
+    const uint32_t da = nibbles_eq(pa, 0xEEEEEEEEu), db = nibbles_eq(pb, 0xEEEEEEEEu);
+    const uint32_t fa = (da | (da >> 16)) & 0x8888u, fb = (db | (db >> 16)) & 0x8888u;  // samples with a '.' token:
+    const uint32_t nm = __popc(fa | (fb >> 1));                                        // missing (main.go:1113,1150)
     a.miss_l += nm;
     a.an_l -= 2 * nm;
-    const uint32_t gone = ((mf | (mf << 16)) >> 3) * 15u;  // all eight bits of both nibbles of a missing sample
-    one &= ~gone;
-    big &= ~gone;
+    const uint32_t ga = ((fa | (fa << 16)) >> 3) * 15u, gb = ((fb | (fb << 16)) >> 3) * 15u;  // both nibbles of them
+    oa &= ~ga; ob &= ~gb;
+    pa &= ~ga; pb &= ~gb;
   }
-  const uint32_t both = one & (one >> 16);
-  const uint32_t n1 = __popc(one), n2 = __popc(both);
+  const uint32_t one = oa | (ob >> 1);
+  const uint32_t n1 = __popc(one), n2 = __popc(one & (one >> 16));
   a.ac_l += n1;
   a.hom_l += n2;
   a.het_l += n1 - 2 * n2;
-  a.flag_l |= big;
+  a.flag_l |= (pa | pb) & 0xEEEEEEEEu;  // nibbles >= 2
 }
 __device__ __forceinline__ void classify_push_words4(const ScanParams &p, WarpState &st, uint32_t *my_events,
                                                      const uint32_t t[4], int samp0, bool dots, int lane) {
@@ -151,7 +153,7 @@ __device__ __forceinline__ void classify_push_words4(const ScanParams &p, WarpSt
   } else if (lane == 0) {
     p.ctr->ev_overflow = 1;
   }
-  if (pl) acc_quad(st.a, pl, dots);
+  acc_quad_pair(st.a, pl, 0u, dots);
   st.ev_w += n;
 }
 
@@ -162,18 +164,16 @@ __device__ __forceinline__ void classify_push_pair(const ScanParams &p, WarpStat
   const uint32_t pa = pack_quad(ta, dots), pb = pack_quad(tb, dots);
   const uint32_t ba = __ballot_sync(FULL, pa != 0), bb = __ballot_sync(FULL, pb != 0);
   if ((ba | bb) == 0) return;
-  const uint32_t na = 2 * __popc(ba), n = na + 2 * __popc(bb);
-  const uint32_t lt = (1u << lane) - 1u;
+  const uint32_t qa = __popc(ba), n = 2 * (qa + __popc(bb));
   if (st.ev_w + n <= p.evcap_words) {
-    uint32_t *dst = my_events + st.ev_w;
-    if (pa) *reinterpret_cast<uint2 *>(dst + 2 * __popc(ba & lt)) = make_uint2((uint32_t)(samp0 + (int)EV_BASE_BIAS), pa);
-    if (pb)
-      *reinterpret_cast<uint2 *>(dst + na + 2 * __popc(bb & lt)) = make_uint2((uint32_t)(samp0 + 128 + (int)EV_BASE_BIAS), pb);
+    uint2 *dst = reinterpret_cast<uint2 *>(my_events + st.ev_w);  // one address for both stores
+    const uint32_t lt = (1u << lane) - 1u, e = (uint32_t)(samp0 + (int)EV_BASE_BIAS);
+    if (pa) dst[__popc(ba & lt)] = make_uint2(e, pa);
+    if (pb) dst[qa + __popc(bb & lt)] = make_uint2(e + 128u, pb);
   } else if (lane == 0) {
     p.ctr->ev_overflow = 1;
   }
-  if (pa) acc_quad(st.a, pa, dots);
-  if (pb) acc_quad(st.a, pb, dots);
+  acc_quad_pair(st.a, pa, pb, dots);
   st.ev_w += n;
 }
 
