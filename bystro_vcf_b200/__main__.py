@@ -26,7 +26,11 @@ def main(argv=None) -> int:
             gpus = max(1, int(s.split("=", 1)[1]))
             del a[i]
             break
-    cfg = setup(a)
+    try:
+        cfg = setup(a)
+    except ValueError as e:  # a flag error: one line, before anything is read or written
+        print(str(e), file=sys.stderr)
+        return 1
     err = sys.stderr
     if cfg.errPath:
         # main.go:150-156 opens the file read-only and re-points os.Stderr, which Go's `log` package never

@@ -81,7 +81,7 @@ SYMBOLS = [
     "bvcf_resident_run", "bvcf_resident_download", "bvcf_resident_peek", "bvcf_resident_line_index", "bvcf_strerror",
     "bvcf_last_error", "bvcf_abi_version", "bvcf_launch_count", "bvcf_resident_run_at", "bvcf_resident_inflate_bgzf",
     "bvcf_bgzf_text_bytes", "bvcf_resident_download_bgzf", "bvcf_resident_write_output", "bvcf_resident_results",
-    "bvcf_submit_bgzf", "bvcf_diag_fields",
+    "bvcf_submit_bgzf", "bvcf_diag_fields", "bvcf_resident_download_bgzf_level",
 ]
 
 _lib = None
@@ -139,6 +139,8 @@ def lib():
     L.bvcf_resident_write_output.argtypes = [vp, sz, vp, sz]
     L.bvcf_resident_download_bgzf.restype = C.c_int
     L.bvcf_resident_download_bgzf.argtypes = [vp, sz, sz, vp, sz, C.POINTER(sz)]
+    L.bvcf_resident_download_bgzf_level.restype = C.c_int
+    L.bvcf_resident_download_bgzf_level.argtypes = [vp, sz, sz, C.c_int, vp, sz, C.POINTER(sz)]
     L.bvcf_resident_download.restype = C.c_int
     L.bvcf_resident_download.argtypes = [vp, sz, vp, sz]
     L.bvcf_resident_peek.restype = C.c_int

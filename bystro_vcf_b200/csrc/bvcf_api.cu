@@ -1220,7 +1220,12 @@ int bvcf_diag_fields(bvcf_ctx *ctx, uint64_t seq, const uint8_t **text, const ui
 
 // ---- bgzf output (SURVEY 8f-4) -----------------------------------------------------------------------------
 int bvcf_resident_download_bgzf(bvcf_ctx *ctx, size_t offset, size_t len, void *host, size_t host_cap, size_t *comp_len) {
-  if (!ctx || !host || !comp_len) return BVCF_E_ARG;
+  return bvcf_resident_download_bgzf_level(ctx, offset, len, 1, host, host_cap, comp_len);
+}
+
+int bvcf_resident_download_bgzf_level(bvcf_ctx *ctx, size_t offset, size_t len, int level, void *host, size_t host_cap,
+                                      size_t *comp_len) {
+  if (!ctx || !host || !comp_len || level < 1 || level > 9) return BVCF_E_ARG;
   if (offset + len > ctx->r_out.cap) return BVCF_E_ARG;
   *comp_len = 0;
   if (len == 0) return BVCF_OK;
@@ -1237,13 +1242,20 @@ int bvcf_resident_download_bgzf(bvcf_ctx *ctx, size_t offset, size_t len, void *
   DeflateParams dp{};
   dp.text = (const uint8_t *)ctx->r_out.p + offset; dp.text_len = len; dp.slots = (uint8_t *)ctx->r_def_slots.p;
   dp.sizes = (uint32_t *)ctx->r_def_sizes.p; dp.n_blocks = nb;
-  bvcf_deflate_kernel<<<nb, 32, 0, st>>>(dp);
+  if (level == 1) bvcf_deflate_kernel<<<nb, 32, 0, st>>>(dp);
+  else bvcf_deflate_dyn_kernel<<<nb, 32, def_dyn_smem(DEF_LEVELS[level]), st>>>(dp, DEF_LEVELS[level]);
   std::vector<uint32_t> sizes(nb);
   CK(cudaMemcpyAsync(sizes.data(), dp.sizes, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   std::vector<unsigned long long> offs(nb);
   unsigned long long total = 0;
-  for (uint32_t i = 0; i < nb; i++) { offs[i] = total; total += sizes[i]; }
+  for (uint32_t i = 0; i < nb; i++) {
+    if (sizes[i] == 0) {  // bvcf_deflate_dyn_kernel's emitted bits disagree with its own count: a bug, never bad data
+      ctx->last_error = "bgzf block " + std::to_string(i) + ": the deflate kernel's output disagrees with its size";
+      return BVCF_E_CUDA;
+    }
+    offs[i] = total; total += sizes[i];
+  }
   if (total > host_cap) { *comp_len = (size_t)total; return BVCF_E_TOO_LARGE; }  // comp_len says how much room it takes
   if ((rc = dev_reserve(ctx, ctx->r_def_out, (size_t)total + 16))) return rc;
   CK(cudaMemcpyAsync(ctx->r_def_offs.p, offs.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));

@@ -50,6 +50,7 @@ struct Config {  // main.go:63-80
   std::vector<int> devices;  // --devices a,b,...: CUDA device of each worker (a device may be listed twice); default 0..gpus-1
   size_t chunkBytes = 64u << 20;
   bool bgzfOut = false;  // --bgzfOut: the rows leave as bgzf blocks deflated on the GPU (the `| pigz -c` of README.md:10,71)
+  int bgzfLevel = 1;     // --bgzfLevel N: 1..9 as `bgzip -l` / `pigz -N` take it (bvcf_resident_download_bgzf_level)
 };
 
 std::string trim(const std::string &s) {  // strings.TrimSpace
@@ -81,6 +82,40 @@ std::vector<std::string> split_trim(const std::string &s) {
   _exit(1);
 }
 
+// strconv.ParseInt(s, 0, 64), what Go's `flag` package reads an int flag with: a sign, then 0x / 0o / 0b / 0 (octal)
+// prefixes or decimal digits, underscores between digits
+bool go_int(const std::string &s, long long *out) {
+  size_t i = 0;
+  const bool neg = !s.empty() && s[0] == '-';
+  if (!s.empty() && (s[0] == '-' || s[0] == '+')) i = 1;
+  int base = 10;
+  if (s.size() > i + 1 && s[i] == '0') {
+    const char b = (char)tolower((unsigned char)s[i + 1]);
+    if (b == 'x') base = 16, i += 2;
+    else if (b == 'o') base = 8, i += 2;
+    else if (b == 'b') base = 2, i += 2;
+    else base = 8, i += 1;
+  }
+  if (i >= s.size()) return false;
+  unsigned long long v = 0;
+  bool digit_before = base == 8 && s[i - 1] == '0';  // "0_7" is octal 7
+  for (; i < s.size(); i++) {
+    if (s[i] == '_') {
+      if (!digit_before || i + 1 >= s.size() || s[i + 1] == '_') return false;
+      continue;
+    }
+    const int c = tolower((unsigned char)s[i]);
+    const int d = isdigit(c) ? c - '0' : (c >= 'a' && c <= 'z') ? c - 'a' + 10 : 99;
+    if (d >= base) return false;
+    if (v > (~0ull - (unsigned)d) / (unsigned)base) return false;
+    v = v * (unsigned)base + (unsigned)d;
+    digit_before = true;
+  }
+  if (v > (neg ? (1ull << 63) : (1ull << 63) - 1)) return false;
+  *out = neg ? (long long)(0 - v) : (long long)v;
+  return true;
+}
+
 // Go `flag` syntax: -x / --x, --x=v / --x v; bool flags --x or --x=true|false; stops at the first non-flag.
 Config setup(int argc, char **argv) {  // main.go:82-126
   Config c;
@@ -93,7 +128,8 @@ Config setup(int argc, char **argv) {  // main.go:82-126
   struct BF { const char *name; bool *dst; };
   const BF bf[] = {{"noOut", &c.noOut}, {"keepId", &c.keepID}, {"keepQual", &c.keepQual}, {"keepPos", &c.keepPos},
                    {"keepInfo", &c.keepInfo}, {"bgzfOut", &c.bgzfOut}};
-  std::string gpus, chunk, devices;
+  std::string gpus, chunk, devices, level;
+  bool level_given = false;
   for (int i = 1; i < argc; i++) {
     std::string s = argv[i];
     if (s.size() < 2 || s[0] != '-') break;
@@ -118,6 +154,7 @@ Config setup(int argc, char **argv) {  // main.go:82-126
     if (name == "gpus") dst = &gpus;          // extension: number of GPUs to use
     if (name == "chunkBytes") dst = &chunk;   // extension: host chunk size
     if (name == "devices") dst = &devices;    // extension: explicit CUDA device per worker
+    if (name == "bgzfLevel") { dst = &level; level_given = true; }  // extension: --bgzfOut's compression level
     if (!dst) fatal("flag provided but not defined: -" + name);
     if (!has_val) {
       if (++i >= argc) fatal("flag needs an argument: -" + name);
@@ -133,6 +170,13 @@ Config setup(int argc, char **argv) {  // main.go:82-126
   if (!devices.empty()) {
     for (auto &d : split_trim(devices)) c.devices.push_back(atoi(d.c_str()));
     c.gpus = (int)c.devices.size();
+  }
+  if (level_given) {
+    long long v;
+    if (!go_int(level, &v)) fatal("invalid value \"" + level + "\" for flag -bgzfLevel: parse error");
+    if (v < 1 || v > 9) fatal("--bgzfLevel must be 1..9, not " + std::to_string(v));
+    if (!c.bgzfOut) fatal("--bgzfLevel needs --bgzfOut");
+    c.bgzfLevel = (int)v;
   }
   return c;
 }
@@ -705,12 +749,12 @@ void run_resident(const Config &config, Input &in, BgzfIn *gz, const Preamble &p
         if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
       }
       size_t comp = 0;
-      rc = bvcf_resident_download_bgzf(ctx, 0, st.out_bytes, out_host, out_cap, &comp);
+      rc = bvcf_resident_download_bgzf_level(ctx, 0, st.out_bytes, config.bgzfLevel, out_host, out_cap, &comp);
       if (rc == BVCF_E_TOO_LARGE) {  // comp: the bytes needed
         bvcf_host_free(out_host);
         out_cap = comp + comp / 8;
         if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
-        rc = bvcf_resident_download_bgzf(ctx, 0, st.out_bytes, out_host, out_cap, &comp);
+        rc = bvcf_resident_download_bgzf_level(ctx, 0, st.out_bytes, config.bgzfLevel, out_host, out_cap, &comp);
       }
       if (rc) fatal(std::string("download: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
       sink.rows(out_host, comp);

@@ -79,6 +79,9 @@ class Config:
     # not in the reference: the rows leave as bgzf blocks deflated on the GPU (stands in for the `| pigz -c` behind the
     # reference, README.md:10,71); --bgzfOut
     bgzfOut: bool = False
+    # --bgzfLevel N: how hard the GPU deflates those rows, 1..9 as `bgzip -l` / `pigz -N` take it; 1 is the fast
+    # single-candidate kernel with fixed codes, 2..9 search more and write dynamic Huffman codes
+    bgzfLevel: int = 1
 
 
 _STRING_FLAGS = {"in": "inPath", "fam": "famPath", "err": "errPath", "out": "outPath", "dosageOutput": "dosageMatrixOutPath",
@@ -86,6 +89,20 @@ _STRING_FLAGS = {"in": "inPath", "fam": "famPath", "err": "errPath", "out": "out
                  "cpuProfile": "cpuProfile", "allowFilter": None, "excludeFilter": None}
 _BOOL_FLAGS = {"noOut": "noOut", "keepId": "keepID", "keepQual": "keepQual", "keepPos": "keepPos", "keepInfo": "keepInfo",
                "bgzfOut": "bgzfOut"}
+_INT_FLAGS = {"bgzfLevel": "bgzfLevel"}
+
+
+def _go_int(val: str) -> Optional[int]:
+    """strconv.ParseInt(val, 0, 64), what Go's `flag` package reads an int flag with (0x.., 0o.., 0b.., 0.. octal,
+    underscores between digits); None when val is not such an integer"""
+    digits = val.lstrip("+-")
+    if val != val.strip() or len(val) - len(digits) > 1:
+        return None
+    try:
+        v = int(val, 8) if len(digits) > 1 and digits[0] == "0" and digits[1] in "01234567_" else int(val, 0)
+    except ValueError:
+        return None
+    return v if -(1 << 63) <= v < (1 << 63) else None
 
 
 def setup(args: Optional[Sequence[str]] = None) -> Config:
@@ -96,6 +113,7 @@ def setup(args: Optional[Sequence[str]] = None) -> Config:
     a = list(sys.argv[1:] if args is None else args)
     cfg = Config()
     allow, exclude = "PASS,.", ""
+    level_given = False
     i = 0
     while i < len(a):
         s = a[i]
@@ -121,6 +139,17 @@ def setup(args: Optional[Sequence[str]] = None) -> Config:
                 else:
                     raise ValueError(f"invalid boolean value {val!r} for -{name}")
             setattr(cfg, _BOOL_FLAGS[name], b)
+        elif name in _INT_FLAGS:
+            if val is None:
+                i += 1
+                if i >= len(a):
+                    raise ValueError(f"flag needs an argument: -{name}")
+                val = a[i]
+            v = _go_int(val)
+            if v is None:
+                raise ValueError(f'invalid value "{val}" for flag -{name}: parse error')
+            setattr(cfg, _INT_FLAGS[name], v)
+            level_given = True
         elif name in _STRING_FLAGS:
             if val is None:
                 i += 1
@@ -140,6 +169,10 @@ def setup(args: Optional[Sequence[str]] = None) -> Config:
         cfg.allowedFilters = {v.strip(): True for v in allow.split(",")}
     if exclude != "":  # main.go:117-123
         cfg.excludedFilters = {v.strip(): True for v in exclude.split(",")}
+    if not 1 <= cfg.bgzfLevel <= 9:
+        raise ValueError(f"--bgzfLevel must be 1..9, not {cfg.bgzfLevel}")
+    if level_given and not cfg.bgzfOut:
+        raise ValueError("--bgzfLevel needs --bgzfOut")
     return cfg
 
 
@@ -388,14 +421,14 @@ class Transformer:
     def resident_write_output(self, offset: int, data: bytes) -> None:
         check(self._L.bvcf_resident_write_output(self._ctx, offset, data, len(data)), self._ctx, "bvcf_resident_write_output")
 
-    def resident_download_bgzf(self, offset: int, length: int) -> bytes:
-        """rows [offset, offset + length) of the resident output, deflated on the GPU: whole bgzf blocks (append
-        bgzf.EOF_BLOCK at the end of a file)"""
+    def resident_download_bgzf(self, offset: int, length: int, level: int = 1) -> bytes:
+        """rows [offset, offset + length) of the resident output, deflated on the GPU at `level` (1..9, see
+        bvcf_resident_download_bgzf_level): whole bgzf blocks (append bgzf.EOF_BLOCK at the end of a file)"""
         cap = length + length // 4 + (1 << 16)
         buf = C.create_string_buffer(cap)
         n = C.c_size_t()
-        check(self._L.bvcf_resident_download_bgzf(self._ctx, offset, length, buf, cap, C.byref(n)), self._ctx,
-              "bvcf_resident_download_bgzf")
+        check(self._L.bvcf_resident_download_bgzf_level(self._ctx, offset, length, level, buf, cap, C.byref(n)), self._ctx,
+              "bvcf_resident_download_bgzf_level")
         return buf.raw[:n.value]
 
     def resident_download(self, offset: int, length: int) -> bytes:
@@ -644,7 +677,7 @@ def _read_vcf_resident(config: Config, head: bytes, reader: BinaryIO, writer: Op
                 stats, _ = tr.resident_run(end, want_times=False, begin=begin)
                 rows = b""
                 if writer is not None and not config.noOut and stats["out_bytes"]:
-                    rows = tr.resident_download_bgzf(0, stats["out_bytes"])
+                    rows = tr.resident_download_bgzf(0, stats["out_bytes"], config.bgzfLevel)
                 loci, dosage, diags = tr.resident_results()
                 res = ChunkResult(tsv=rows, n_lines=stats["n_lines"], n_records=stats["n_records"], n_rows=stats["n_rows"],
                                   diags=[d[:3] for d in diags], diag_starts=[d[3] for d in diags], loci=loci, dosage=dosage)

@@ -183,6 +183,11 @@ int bvcf_bgzf_text_bytes(const void *comp, size_t comp_len, uint64_t *text_bytes
  * pieces of a file and end it with the 28-byte bgzf EOF block.  BVCF_E_TOO_LARGE: host_cap is too small, *comp_len
  * says what is needed. */
 int bvcf_resident_download_bgzf(bvcf_ctx *ctx, size_t offset, size_t len, void *host, size_t host_cap, size_t *comp_len);
+/* The same at a compression level, as `bgzip -l` / `pigz -N` take one: 1 is bvcf_resident_download_bgzf (the bytes are
+ * the same); 2..9 search more match candidates per position (from 4 on, lazily) and pick per block the cheapest of
+ * dynamic Huffman codes, fixed codes and a stored block.  Any other level: BVCF_E_ARG. */
+int bvcf_resident_download_bgzf_level(bvcf_ctx *ctx, size_t offset, size_t len, int level, void *host, size_t host_cap,
+                                      size_t *comp_len);
 
 /* Put host bytes into the resident output region (a host that wants its own text -- the TSV header line, say --
  * to leave through bvcf_resident_download_bgzf with the rows). */
