@@ -53,14 +53,23 @@ struct Scratch {
   uint32_t slow_cap = 0;      // slow-path list entries (grown on slow_overflow)
 };
 
-struct Slot {
+// One run of the pipeline over text on the device: a streaming slot's chunk, or the resident path's input.  A run that
+// reports an overflow grows what overflowed and runs again with the same buffers (grow_for_retry).
+struct Run {
   cudaStream_t stream = nullptr;
-  cudaEvent_t done = nullptr;
-  DevBuf d_in, d_out, d_dosage, d_loci, d_loci_off, d_diags;
-  DevBuf d_comp, d_blocks, d_fields, d_field_off, d_diag_starts;  // bgzf chunks; diagnostic fields
-  Scratch sc;
   RunCounters *d_ctr = nullptr;
   RunCounters *h_ctr = nullptr;  // pinned
+  Scratch sc;
+  DevBuf d_in, d_out, d_dosage, d_loci, d_loci_off, d_diags;
+  uint32_t diag_cap = 0;         // entries of d_diags the run was enqueued with
+  DevBuf d_comp, d_blocks;       // bgzf input: compressed bytes and block table
+  uint32_t *d_bad = nullptr;     // blocks that failed to inflate
+};
+
+struct Slot {
+  Run run;
+  cudaEvent_t done = nullptr;
+  DevBuf d_fields, d_field_off, d_diag_starts;  // diagnostic fields
   uint8_t *h_out = nullptr;      // pinned
   size_t h_out_cap = 0;
   int8_t *h_dosage = nullptr;    // pinned
@@ -76,14 +85,12 @@ struct Slot {
   const uint8_t *h_src = nullptr;
   size_t len = 0;
   uint32_t retries = 0;
-  uint32_t diag_cap = 0;         // entries of d_diags the chunk was enqueued with
   // bgzf chunk: the text is inflate(comp) [0, text_len) then the tail; data lines start at `skip`
   bool bgzf = false;
   size_t skip = 0, text_len = 0, tail_len = 0;
   uint8_t *h_stage = nullptr;    // pinned: compressed bytes, block table, tail
   size_t h_stage_cap = 0;
-  uint32_t *d_bad = nullptr;     // blocks that failed to inflate
-  uint32_t *h_bad = nullptr;     // pinned copy
+  uint32_t *h_bad = nullptr;     // pinned: [0] blocks that failed to inflate, [1] last text byte
   std::vector<InflateBlock> blocks;
   std::vector<uint8_t> h_fields;
   std::vector<uint64_t> h_field_off, h_diag_starts;
@@ -104,16 +111,13 @@ struct bvcf_ctx {
   DevBuf d_filt_blob, d_filt_off, d_names, d_name_off, d_name8, d_name16;
   std::vector<Slot> slots;
   // resident path
-  DevBuf r_in, r_out, r_dosage, r_loci, r_loci_off, r_comp, r_blocks, r_def_slots, r_def_sizes, r_def_offs, r_def_out, r_diags;
+  Run res;
+  DevBuf r_def_slots, r_def_sizes, r_def_offs, r_def_out;
   std::vector<bvcf_diag> r_h_diags;
   std::vector<int8_t> r_h_dosage;
   std::vector<uint8_t> r_h_loci;
   std::vector<uint64_t> r_h_loci_off;
-  uint32_t *r_d_bad = nullptr;
   size_t r_in_bytes = 0;
-  Scratch r_sc;
-  cudaStream_t r_stream = nullptr;
-  RunCounters *r_d_ctr = nullptr, *r_h_ctr = nullptr;
   std::vector<cudaEvent_t> ev_pool;
   double ev_factor = 0.5;  // event slice bytes per range byte
   uint32_t diag_cap = DIAG_CAP0;   // diagnostics a chunk may report (grown on demand, never truncated)
@@ -161,9 +165,7 @@ constexpr uint64_t IN_SLACK = 8192;
 uint32_t choose_range_bytes(uint64_t total) {
   uint64_t r = total / (148ull * 32 * 3);
   r = round_up(std::max<uint64_t>(r, 1), 512);
-  uint64_t cap_r = 256 * 1024;
-  if (const char *e = getenv("BVCF_RANGE_KB")) cap_r = std::max(16, atoi(e)) * 1024ull;  // experiments
-  r = std::min<uint64_t>(std::max<uint64_t>(r, 16 * 1024), cap_r);
+  r = std::min<uint64_t>(std::max<uint64_t>(r, 16 * 1024), 256 * 1024);
   return (uint32_t)r;
 }
 
@@ -184,7 +186,7 @@ int scratch_reserve(bvcf_ctx *ctx, Scratch &sc, uint64_t total_bytes, uint64_t s
   sc.sub_bytes = sub;
   sc.n_ranges = (uint32_t)(sub / sc.range_bytes);
   // a record needs at least H bytes (H - 1 tabs + the newline); with H < 16 the first guess is 16 and slot_overflow
-  // lowers it (bvcf_collect / bvcf_resident_run re-run the chunk)
+  // lowers it (grow_for_retry) and the chunk runs again
   sc.slots = sc.range_bytes / std::max<uint32_t>((uint32_t)std::max(H, 1), ctx->min_line_bytes) + 2;
   uint64_t evb = (uint64_t)(sc.range_bytes * ctx->ev_factor) + 16 * 1024;
   if (ctx->dcfg.n_samples == 0) evb = 64;
@@ -228,22 +230,54 @@ void scratch_free(Scratch &sc) {
     dev_free(*b);
 }
 
+bool run_init(Run &r) {
+  return cudaStreamCreateWithFlags(&r.stream, cudaStreamNonBlocking) == cudaSuccess &&
+         cudaMalloc(&r.d_ctr, sizeof(RunCounters)) == cudaSuccess && cudaMallocHost(&r.h_ctr, sizeof(RunCounters)) == cudaSuccess;
+}
+void run_free(Run &r) {
+  if (r.stream) cudaStreamDestroy(r.stream);
+  for (DevBuf *b : {&r.d_in, &r.d_out, &r.d_dosage, &r.d_loci, &r.d_loci_off, &r.d_diags, &r.d_comp, &r.d_blocks}) dev_free(*b);
+  scratch_free(r.sc);
+  if (r.d_bad) cudaFree(r.d_bad);
+  if (r.d_ctr) cudaFree(r.d_ctr);
+  if (r.h_ctr) cudaFreeHost(r.h_ctr);
+}
+
+// geometry and scratch for data lines in [begin, len), and a diagnostics buffer of the context's current capacity
+int run_reserve(bvcf_ctx *ctx, Run &r, uint64_t begin, uint64_t len) {
+  int rc;
+  if ((rc = scratch_reserve(ctx, r.sc, len - (begin & ~511ull), ctx->cfg.resident_subchunk_bytes))) return rc;
+  r.diag_cap = ctx->diag_cap;
+  return dev_reserve(ctx, r.d_diags, (size_t)r.diag_cap * DIAG_WORDS * 4);
+}
+
+// rows the dosage matrix and the locus offsets have room for (0 without --dosageOutput)
+uint64_t dosage_rows(const bvcf_ctx *ctx, const Run &r) {
+  const DevCfg &dc = ctx->dcfg;
+  if (!dc.want_dosage || dc.n_samples <= 0) return 0;
+  return std::min<uint64_t>(r.d_dosage.cap / (uint64_t)dc.n_samples, r.d_loci_off.cap / 8);
+}
+
 constexpr int N_STAGE_EV = 8;  // 0..5 stage boundaries, 6..7 inside the rows stage (compose | offsets | copy-out)
 struct StageEvents {  // optional per-stage timing of one sub-chunk
   cudaEvent_t e[N_STAGE_EV];
 };
 
-// Enqueue the whole pipeline for data lines in [0, len) of d_in.  Never synchronises.
-int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t *d_in, uint64_t begin, uint64_t len, uint64_t buf_len,
-                     uint8_t *d_out, uint64_t out_cap, RunCounters *d_ctr, int8_t *d_dosage, uint64_t dosage_cap_rows,
-                     uint8_t *d_loci, uint64_t loci_cap, unsigned long long *d_loci_off, uint32_t *d_diags,
-                     uint32_t diag_cap, std::vector<StageEvents> *timing) {
+// Enqueue the whole pipeline for data lines in [begin, len) of r.d_in, from zeroed counters to their copy in r.h_ctr.
+// Never synchronises.
+int enqueue_pipeline(bvcf_ctx *ctx, Run &r, uint64_t begin, uint64_t len, uint64_t buf_len, std::vector<StageEvents> *timing) {
   const DevCfg &dc = ctx->dcfg;
+  Scratch &sc = r.sc;
+  const cudaStream_t st = r.stream;
+  const uint8_t *d_in = (const uint8_t *)r.d_in.p;
+  RunCounters *d_ctr = r.d_ctr;
+  int8_t *d_dosage = (int8_t *)r.d_dosage.p;
+  const uint64_t dosage_cap_rows = dosage_rows(ctx, r);
+  CK(cudaMemsetAsync(d_ctr, 0, sizeof(RunCounters), st));
   // data lines live in [begin, len); ranges tile the region from begin rounded down to 512 bytes
   const uint64_t a0 = begin & ~511ull;
   const uint64_t total_ranges = (len - a0 + sc.range_bytes - 1) / sc.range_bytes;
-  int smem = SCAN_WARPS * RING;
-  if (const char *e = getenv("BVCF_SCAN_SMEM_KB")) smem = std::max(smem, atoi(e) * 1024);  // experiments: cap CTAs/SM
+  const int smem = SCAN_WARPS * RING;
   cudaFuncSetAttribute(bvcf_scan_genotype_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   cudaFuncSetAttribute(bvcf_scan_genotype_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   int n_sm = 148;
@@ -311,28 +345,24 @@ int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t 
     }
     if (se) CK(cudaEventRecord(se->e[3], st));
     // 4. rows: FILTER + getAlleles + row text + short name lists, one pass (tile of 128 records per CTA)
-    static const bool no_vec = getenv("BVCF_NO_NAMES_VEC") != nullptr;  // experiments
-    const bool vec = (dc.name8 || dc.name16) && dc.want_tsv && !no_vec && dc.n_samples > 0;
+    const bool vec = (dc.name8 || dc.name16) && dc.want_tsv && dc.n_samples > 0;
     TileParams tp{};
     tp.in = d_in; tp.cfg = dc; tp.lines = cp.dense; tp.events = sp.events; tp.stats = (const LineStats *)sc.stats1.p;
-    tp.out = d_out; tp.out_cap = out_cap; tp.ctr = d_ctr;
+    tp.out = (uint8_t *)r.d_out.p; tp.out_cap = r.d_out.cap; tp.ctr = d_ctr;
     tp.tile_agg = (TileAgg *)sc.tile_agg.p; tp.tile_base = (TileBase *)sc.tile_base.p;
     tp.tile_partial = (unsigned long long *)sc.tile_partial.p;
     tp.scratch = (uint8_t *)sc.tile_scratch.p; tp.scratch_cap = sc.scratch_cap;
     tp.slow = (SlowRec *)sc.slow.p; tp.slow_cap = sc.slow_cap;
     tp.row_desc = (RowDesc *)sc.row_desc.p; tp.row_desc_cap = dc.n_samples > 0 ? sc.row_cap : 0;
     tp.long_words = vec ? 8192u : 0u;  // rows beyond 4,096 quads: a CTA per row
-    {
-      // rows of up to 16 quads: a lane per row.  Measured on 600,000 chr1-shape variants (names stage): no mid class
-      // 0.349 ms, 16 quads 0.345, 32 quads 0.359, 64 quads 0.408, 128 quads 0.49 -- a lane's own event list and its
-      // scattered 8-byte stores cost more than the idle lanes of a warp-per-row sweep once rows hold a few dozen names
-      static const int mid_q = getenv("BVCF_MID_QUADS") ? atoi(getenv("BVCF_MID_QUADS")) : 16;  // experiments
-      tp.mid_words = (dc.want_tsv && dc.n_samples > 0) ? 2u * (uint32_t)std::max(mid_q, 0) : 0u;
-      if (!vec) tp.mid_words = 0;  // names_big_kernel serves every list
-    }
+    // rows of up to 16 quads: a lane per row.  Measured on 600,000 chr1-shape variants (names stage): no mid class
+    // 0.349 ms, 16 quads 0.345, 32 quads 0.359, 64 quads 0.408, 128 quads 0.49 -- a lane's own event list and its
+    // scattered 8-byte stores cost more than the idle lanes of a warp-per-row sweep once rows hold a few dozen names.
+    // Without the vector kernels names_big_kernel serves every list.
+    tp.mid_words = vec ? 2u * 16u : 0u;
     tp.dosage = d_dosage; tp.dosage_cap_rows = dosage_cap_rows;
-    tp.loci = d_loci; tp.loci_cap = loci_cap; tp.loci_off = d_loci_off;
-    tp.diag.diags = d_diags; tp.diag.cap = diag_cap; tp.diag.ctr = d_ctr;
+    tp.loci = (uint8_t *)r.d_loci.p; tp.loci_cap = r.d_loci.cap; tp.loci_off = (unsigned long long *)r.d_loci_off.p;
+    tp.diag.diags = (uint32_t *)r.d_diags.p; tp.diag.cap = r.diag_cap; tp.diag.ctr = d_ctr;
     {
       auto launch = [&](auto kern, uint32_t arena, uint32_t rows, int minb) {
         const uint32_t smem = TILE_WARPS * tile_smem_warp(arena, rows);
@@ -342,29 +372,20 @@ int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t 
       // (5, 6 and 8 resident CTAs per SM were measured too: the spills of a 96 / 80 / 64-register build cost more than
       // the extra warps hide -- rows 0.42 -> 0.51 / 0.52 / 0.55 ms on 600,000 chr1-shape variants)
       // L2 prefetch of the next tile's lines / scratch block: measured, no gain (compose 0.323 -> 0.329 ms, copy-out
-      // 0.116 -> 0.124 ms on 600,000 chr1-shape variants: the waits are dependent L1/L2 hits, not DRAM), so off
-      static const int pf = getenv("BVCF_PREFETCH") ? atoi(getenv("BVCF_PREFETCH")) : 0;  // experiments: bit 0 compose, bit 1 copy-out
-      static const bool sites_old = getenv("BVCF_SITES_OLD") != nullptr;  // experiments: the thread-per-record composer
-      if (dc.n_samples == 0 && !sites_old) {
-        static const int sv = getenv("BVCF_SITES_VAR") ? atoi(getenv("BVCF_SITES_VAR")) : 0;  // experiments
+      // 0.116 -> 0.124 ms on 600,000 chr1-shape variants: the waits are dependent L1/L2 hits, not DRAM), so none
+      if (dc.n_samples == 0) {
         // 8 resident CTAs (64 registers, 3.5 KiB arena + 96 rows per warp) against 5 (80 registers, 6 KiB + 128 rows):
         // 19.5 against 23.3 ms on 50 M lines -- the kernel waits on dependent loads and taken branches, warps hide both
         // (REF / ALT held in registers, which pays at 128 registers, spills at 64: 20.3 ms; 7 CTAs x 72 registers with
         // them: 20.9 ms; 8 CTAs without: 19.5 ms)
-        if (sv == 5) launch(bvcf_compose_sites_kernel<5, 6144, 128, true>, 6144, 128, 5);
-        else launch(bvcf_compose_sites_kernel<8, 3584, 96, false>, 3584, 96, 8);
-      } else if (dc.n_samples == 0) {
-        if (pf & 1) launch(bvcf_compose_kernel<4, 8192, 160, true>, 8192, 160, 4);
-        else launch(bvcf_compose_kernel<4, 8192, 160, false>, 8192, 160, 4);
+        launch(bvcf_compose_sites_kernel<8, 3584, 96>, 3584, 96, 8);
       } else {
         // the build for the default flags: TSV rows, no --keepPos/Id/Info, no dosage matrix, 7-character names joined by
         // one character -- a smaller kernel (see "Code size" in DESIGN.md)
-        static const bool no_spec = getenv("BVCF_NO_SPEC") != nullptr;  // experiments
-        const bool spec = !no_spec && dc.want_tsv && !dc.keep_pos && !dc.keep_id && !dc.keep_info && !dc.want_dosage && dc.name8 &&
+        const bool spec = dc.want_tsv && !dc.keep_pos && !dc.keep_id && !dc.keep_info && !dc.want_dosage && dc.name8 &&
                           dc.delim_len == 1 && dc.name_fixed_w == 7;
-        if (pf & 1) launch(bvcf_compose_kernel<4, 10240, 48, true>, 10240, 48, 4);
-        else if (spec) launch(bvcf_compose_kernel<4, 10240, 48, false, true>, 10240, 48, 4);
-        else launch(bvcf_compose_kernel<4, 10240, 48, false>, 10240, 48, 4);
+        if (spec) launch(bvcf_compose_kernel<4, 10240, 48, true>, 10240, 48, 4);
+        else launch(bvcf_compose_kernel<4, 10240, 48>, 10240, 48, 4);
       }
       if (se) CK(cudaEventRecord(se->e[6], st));
       bvcf_tile_reduce_kernel<<<TSCAN_BLOCKS, TSCAN_THREADS, 0, st>>>(tp);
@@ -375,8 +396,7 @@ int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t 
         bvcf_dosage_zero_kernel<<<(unsigned)n_sm * 8, 256, 0, st>>>(tp);
         ctx->launches += 1;
       }
-      if (pf & 2) bvcf_copyout_kernel<true><<<(unsigned)n_sm * 16, TILE_WARPS * 32, 0, st>>>(tp);
-      else bvcf_copyout_kernel<false><<<(unsigned)n_sm * 16, TILE_WARPS * 32, 0, st>>>(tp);
+      bvcf_copyout_kernel<<<(unsigned)n_sm * 16, TILE_WARPS * 32, 0, st>>>(tp);
     }
     bvcf_slow_rows_kernel<<<(unsigned)n_sm, 64, 0, st>>>(tp);
     ctx->launches += 6;
@@ -386,7 +406,7 @@ int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t 
     if (dc.n_samples > 0) {
       NamesParams np{};
       np.in = d_in; np.cfg = dc; np.lines = cp.dense; np.events = sp.events; np.row_desc = (const RowDesc *)sc.row_desc.p;
-      np.row_desc_cap = sc.row_cap; np.out = d_out; np.ctr = d_ctr; np.dosage = d_dosage; np.dosage_cap_rows = dosage_cap_rows;
+      np.row_desc_cap = sc.row_cap; np.out = tp.out; np.ctr = d_ctr; np.dosage = d_dosage; np.dosage_cap_rows = dosage_cap_rows;
       np.long_words = tp.long_words;
       if (vec) {
         const unsigned g1 = (unsigned)n_sm * 18, g2 = (unsigned)n_sm * 2;
@@ -422,6 +442,7 @@ int enqueue_pipeline(bvcf_ctx *ctx, Scratch &sc, cudaStream_t st, const uint8_t 
     if (se) CK(cudaEventRecord(se->e[5], st));
   }
   CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(r.h_ctr, d_ctr, sizeof(RunCounters), cudaMemcpyDeviceToHost, st));
   return 0;
 }
 
@@ -492,73 +513,118 @@ void decode_diags(const uint32_t *raw, uint32_t nd, std::vector<bvcf_diag> &out)
   }
 }
 
-// A bgzf chunk's compressed bytes, block table and tail are in the slot's pinned staging buffer: upload them, inflate the
-// blocks into d_in, put the tail after the text.  Only the first attempt does this -- a retry finds the text on the device.
-int slot_inflate(bvcf_ctx *ctx, Slot &s, size_t comp_len) {
-  const size_t nb = s.blocks.size(), tab_off = round_up(comp_len, 16), tail_off = tab_off + nb * sizeof(InflateBlock);
+// Enqueue the inflate of `nb` bgzf blocks into r.d_in: their compressed bytes and block table are copied from the host
+// (pinned memory makes the copies asynchronous), and r.d_bad counts the blocks that fail.
+int enqueue_inflate(bvcf_ctx *ctx, Run &r, const uint8_t *comp, size_t comp_len, const InflateBlock *blocks, size_t nb) {
   int rc;
-  if ((rc = dev_reserve(ctx, s.d_comp, comp_len + 16))) return rc;  // the bit reader may look 11 bytes past the payload
-  if ((rc = dev_reserve(ctx, s.d_blocks, nb * sizeof(InflateBlock)))) return rc;
-  if (!s.d_bad) CK(cudaMalloc(&s.d_bad, 4));
-  if (!s.h_bad) CK(cudaMallocHost(&s.h_bad, 8));  // [0] bad blocks, [1] last text byte
-  s.h_bad[0] = s.h_bad[1] = 0;
-  CK(cudaMemsetAsync(s.d_bad, 0, 4, s.stream));
+  if ((rc = dev_reserve(ctx, r.d_comp, comp_len + 16))) return rc;  // the bit reader may look 11 bytes past the payload
+  if ((rc = dev_reserve(ctx, r.d_blocks, nb * sizeof(InflateBlock)))) return rc;
+  if (!r.d_bad) CK(cudaMalloc(&r.d_bad, 4));
+  CK(cudaMemsetAsync(r.d_bad, 0, 4, r.stream));
   if (nb) {
-    CK(cudaMemcpyAsync(s.d_comp.p, s.h_stage, comp_len, cudaMemcpyHostToDevice, s.stream));
-    CK(cudaMemcpyAsync(s.d_blocks.p, s.h_stage + tab_off, nb * sizeof(InflateBlock), cudaMemcpyHostToDevice, s.stream));
+    CK(cudaMemcpyAsync(r.d_comp.p, comp, comp_len, cudaMemcpyHostToDevice, r.stream));  // the compressed bytes cross PCIe
+    CK(cudaMemcpyAsync(r.d_blocks.p, blocks, nb * sizeof(InflateBlock), cudaMemcpyHostToDevice, r.stream));
     InflateParams ip{};
-    ip.comp = (const uint8_t *)s.d_comp.p; ip.out = (uint8_t *)s.d_in.p; ip.blocks = (const InflateBlock *)s.d_blocks.p;
-    ip.n_blocks = (uint32_t)nb; ip.n_bad = s.d_bad;
+    ip.comp = (const uint8_t *)r.d_comp.p; ip.out = (uint8_t *)r.d_in.p; ip.blocks = (const InflateBlock *)r.d_blocks.p;
+    ip.n_blocks = (uint32_t)nb; ip.n_bad = r.d_bad;
     cudaFuncSetAttribute(bvcf_inflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)INF_SMEM);
-    bvcf_inflate_kernel<<<ip.n_blocks, 32, INF_SMEM, s.stream>>>(ip);
+    bvcf_inflate_kernel<<<ip.n_blocks, 32, INF_SMEM, r.stream>>>(ip);
     ctx->launches++;
   }
+  return 0;
+}
+
+int inflate_result(bvcf_ctx *ctx, uint32_t n_bad) {
+  if (!n_bad) return BVCF_OK;
+  ctx->last_error = std::to_string(n_bad) + " bgzf block(s) failed to inflate or failed their CRC-32 / ISIZE check";
+  return BVCF_E_ARG;
+}
+
+// A bgzf chunk's compressed bytes, block table and tail are in the slot's pinned staging buffer: inflate the blocks into
+// d_in, put the tail after the text.  Only the first attempt does this -- a retry finds the text on the device.
+int slot_inflate(bvcf_ctx *ctx, Slot &s, size_t comp_len) {
+  Run &r = s.run;
+  const size_t nb = s.blocks.size(), tab_off = round_up(comp_len, 16), tail_off = tab_off + nb * sizeof(InflateBlock);
+  if (!s.h_bad) CK(cudaMallocHost(&s.h_bad, 8));
+  s.h_bad[0] = s.h_bad[1] = 0;
+  int rc;
+  if ((rc = enqueue_inflate(ctx, r, s.h_stage, comp_len, (const InflateBlock *)(s.h_stage + tab_off), nb))) return rc;
   if (s.tail_len)
-    CK(cudaMemcpyAsync((uint8_t *)s.d_in.p + s.text_len, s.h_stage + tail_off, s.tail_len, cudaMemcpyHostToDevice, s.stream));
-  CK(cudaMemcpyAsync(s.h_bad, s.d_bad, 4, cudaMemcpyDeviceToHost, s.stream));
+    CK(cudaMemcpyAsync((uint8_t *)r.d_in.p + s.text_len, s.h_stage + tail_off, s.tail_len, cudaMemcpyHostToDevice, r.stream));
+  CK(cudaMemcpyAsync(s.h_bad, r.d_bad, 4, cudaMemcpyDeviceToHost, r.stream));
   if (s.len > s.skip && !s.tail_len)  // the text must end with a newline: its last byte, for bvcf_collect
-    CK(cudaMemcpyAsync(s.h_bad + 1, (const uint8_t *)s.d_in.p + s.len - 1, 1, cudaMemcpyDeviceToHost, s.stream));
+    CK(cudaMemcpyAsync(s.h_bad + 1, (const uint8_t *)r.d_in.p + s.len - 1, 1, cudaMemcpyDeviceToHost, r.stream));
   else
     s.h_bad[1] = '\n';
   return 0;
 }
 
 int slot_enqueue(bvcf_ctx *ctx, Slot &s, bool upload, size_t comp_len = 0) {
+  Run &r = s.run;
   const uint64_t len = s.len;
   const uint64_t buf_len = round_up(len, 1024) + 2048;
   int rc;
-  if ((rc = dev_reserve(ctx, s.d_in, buf_len + IN_SLACK))) return rc;
-  if ((rc = scratch_reserve(ctx, s.sc, len - (s.skip & ~511ull), ctx->cfg.resident_subchunk_bytes))) return rc;
-  if (s.d_out.cap == 0) {
-    if ((rc = dev_reserve(ctx, s.d_out, std::max<size_t>(len / 2, 1 << 20)))) return rc;
+  if ((rc = dev_reserve(ctx, r.d_in, buf_len + IN_SLACK))) return rc;
+  if ((rc = run_reserve(ctx, r, s.skip, len))) return rc;
+  if (r.d_out.cap == 0) {
+    if ((rc = dev_reserve(ctx, r.d_out, std::max<size_t>(len / 2, 1 << 20)))) return rc;
   }
   const DevCfg &dc = ctx->dcfg;
-  uint64_t dos_rows = 0;
-  if (dc.want_dosage && dc.n_samples > 0) {
-    dos_rows = std::min<uint64_t>(s.d_dosage.cap / (uint64_t)dc.n_samples, s.d_loci_off.cap / 8);
-    if (dos_rows == 0) {
-      const uint64_t est = std::max<uint64_t>(len / std::max(1, dc.H) * 2, 1024);
-      if ((rc = dev_reserve(ctx, s.d_dosage, est * dc.n_samples))) return rc;
-      if ((rc = dev_reserve(ctx, s.d_loci_off, est * 8))) return rc;
-      if ((rc = dev_reserve(ctx, s.d_loci, est * LOCI_GUESS))) return rc;
-      dos_rows = est;
-    }
+  if (dc.want_dosage && dc.n_samples > 0 && dosage_rows(ctx, r) == 0) {  // first guess: two rows per shortest line
+    const uint64_t est = std::max<uint64_t>(len / std::max(1, dc.H) * 2, 1024);
+    if ((rc = dev_reserve(ctx, r.d_dosage, est * dc.n_samples))) return rc;
+    if ((rc = dev_reserve(ctx, r.d_loci_off, est * 8))) return rc;
+    if ((rc = dev_reserve(ctx, r.d_loci, est * LOCI_GUESS))) return rc;
   }
-  s.diag_cap = ctx->diag_cap;
-  if ((rc = dev_reserve(ctx, s.d_diags, (size_t)s.diag_cap * DIAG_WORDS * 4))) return rc;
   if (upload && s.bgzf) {
     if ((rc = slot_inflate(ctx, s, comp_len))) return rc;
   } else if (upload) {
-    CK(cudaMemcpyAsync(s.d_in.p, s.h_src, len, cudaMemcpyHostToDevice, s.stream));
+    CK(cudaMemcpyAsync(r.d_in.p, s.h_src, len, cudaMemcpyHostToDevice, r.stream));
   }
-  CK(cudaMemsetAsync((uint8_t *)s.d_in.p + len, '\n', buf_len - len, s.stream));
-  CK(cudaMemsetAsync(s.d_ctr, 0, sizeof(RunCounters), s.stream));
-  rc = enqueue_pipeline(ctx, s.sc, s.stream, (const uint8_t *)s.d_in.p, s.skip, len, buf_len, (uint8_t *)s.d_out.p, s.d_out.cap,
-                        s.d_ctr, (int8_t *)s.d_dosage.p, dos_rows, (uint8_t *)s.d_loci.p, s.d_loci.cap,
-                        (unsigned long long *)s.d_loci_off.p, (uint32_t *)s.d_diags.p, s.diag_cap, nullptr);
-  if (rc) return rc;
-  CK(cudaMemcpyAsync(s.h_ctr, s.d_ctr, sizeof(RunCounters), cudaMemcpyDeviceToHost, s.stream));
-  CK(cudaEventRecord(s.done, s.stream));
+  CK(cudaMemsetAsync((uint8_t *)r.d_in.p + len, '\n', buf_len - len, r.stream));
+  if ((rc = enqueue_pipeline(ctx, r, s.skip, len, buf_len, nullptr))) return rc;
+  CK(cudaEventRecord(s.done, r.stream));
+  return 0;
+}
+
+// After a run: grow whatever its counters report too small.  `again` says the run must go again -- at once for short
+// lines and dense genotype blocks, whose later stages did not run -- and the 9th retry is an error.
+int grow_for_retry(bvcf_ctx *ctx, Run &r, const RunCounters &c, uint32_t &retries, bool &again) {
+  const DevCfg &dc = ctx->dcfg;
+  again = true;
+  if (c.slot_overflow) {                                              // lines shorter than assumed: more line slots
+    if (ctx->min_line_bytes <= 1) return BVCF_E_TOO_LARGE;
+    ctx->min_line_bytes /= 2;
+    return ++retries > 8 ? BVCF_E_TOO_LARGE : 0;
+  }
+  if (c.ev_overflow) {                                                // dense genotype block: more event slots
+    ctx->ev_factor *= 4;
+    return ++retries > 8 ? BVCF_E_TOO_LARGE : 0;
+  }
+  again = false;
+  int rc;
+  if (c.row_overflow) { r.sc.row_cap = r.sc.row_cap * 4 + c.row_cursor; again = true; }  // MNP/multi-ALT heavy block
+  if (c.out_overflow) {
+    if ((rc = dev_reserve(ctx, r.d_out, (size_t)(c.out_cursor + c.out_cursor / 8 + 4096)))) return rc;
+    again = true;
+  }
+  if (dc.want_dosage && dc.n_samples > 0) {  // dosage rows, locus offsets and locus bytes grow to what the run reported
+    if (c.row_cursor * (uint64_t)dc.n_samples > r.d_dosage.cap || c.row_cursor * 8 > r.d_loci_off.cap) {
+      if ((rc = dev_reserve(ctx, r.d_dosage, (size_t)(c.row_cursor + 64) * dc.n_samples))) return rc;
+      if ((rc = dev_reserve(ctx, r.d_loci_off, (size_t)(c.row_cursor + 64) * 8))) return rc;
+      again = true;
+    }
+    if (c.loci_cursor > r.d_loci.cap) {
+      if ((rc = dev_reserve(ctx, r.d_loci, (size_t)(c.loci_cursor + c.loci_cursor / 8 + 4096)))) return rc;
+      again = true;
+    }
+  }
+  // every log line or none.  Compared with the capacity this run had: another slot may have raised ctx->diag_cap since,
+  // and this run's buffer is still the old size
+  if (c.n_diags > r.diag_cap) { ctx->diag_cap = std::max(ctx->diag_cap, c.n_diags + c.n_diags / 4); again = true; }
+  if (c.scratch_overflow) { r.sc.scratch_cap = c.scratch_cursor + c.scratch_cursor / 4 + (1ull << 20); again = true; }
+  if (c.slow_overflow) { r.sc.slow_cap = c.n_slow + c.n_slow / 4 + 1024; again = true; }
+  if (again && ++retries > 8) return BVCF_E_TOO_LARGE;
   return 0;
 }
 
@@ -649,14 +715,10 @@ int bvcf_create(bvcf_ctx **out, int cuda_device, const bvcf_config *cfg) {
 
   ctx->slots.resize(ctx->cfg.n_slots);
   for (auto &s : ctx->slots) {
-    if (cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess) return fail(BVCF_E_CUDA);
+    if (!run_init(s.run)) return fail(BVCF_E_CUDA);
     if (cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming) != cudaSuccess) return fail(BVCF_E_CUDA);
-    if (cudaMalloc(&s.d_ctr, sizeof(RunCounters)) != cudaSuccess) return fail(BVCF_E_CUDA);
-    if (cudaMallocHost(&s.h_ctr, sizeof(RunCounters)) != cudaSuccess) return fail(BVCF_E_CUDA);
   }
-  if (cudaStreamCreateWithFlags(&ctx->r_stream, cudaStreamNonBlocking) != cudaSuccess) return fail(BVCF_E_CUDA);
-  if (cudaMalloc(&ctx->r_d_ctr, sizeof(RunCounters)) != cudaSuccess) return fail(BVCF_E_CUDA);
-  if (cudaMallocHost(&ctx->r_h_ctr, sizeof(RunCounters)) != cudaSuccess) return fail(BVCF_E_CUDA);
+  if (!run_init(ctx->res)) return fail(BVCF_E_CUDA);
   *out = ctx;
   return BVCF_OK;
 }
@@ -666,31 +728,20 @@ void bvcf_destroy(bvcf_ctx *ctx) {
   cudaSetDevice(ctx->device);
   cudaDeviceSynchronize();
   for (auto &s : ctx->slots) {
-    if (s.stream) cudaStreamDestroy(s.stream);
+    run_free(s.run);
     if (s.done) cudaEventDestroy(s.done);
-    for (DevBuf *b : {&s.d_in, &s.d_out, &s.d_dosage, &s.d_loci, &s.d_loci_off, &s.d_diags, &s.d_comp, &s.d_blocks, &s.d_fields,
-                      &s.d_field_off, &s.d_diag_starts})
-      dev_free(*b);
-    if (s.d_bad) cudaFree(s.d_bad);
+    for (DevBuf *b : {&s.d_fields, &s.d_field_off, &s.d_diag_starts}) dev_free(*b);
     if (s.h_bad) cudaFreeHost(s.h_bad);
     if (s.h_stage) cudaFreeHost(s.h_stage);
-    scratch_free(s.sc);
-    if (s.d_ctr) cudaFree(s.d_ctr);
-    if (s.h_ctr) cudaFreeHost(s.h_ctr);
     if (s.h_out) cudaFreeHost(s.h_out);
     if (s.h_dosage) cudaFreeHost(s.h_dosage);
     if (s.h_loci) cudaFreeHost(s.h_loci);
     if (s.h_loci_off) cudaFreeHost(s.h_loci_off);
   }
-  for (DevBuf *b : {&ctx->d_filt_blob, &ctx->d_filt_off, &ctx->d_names, &ctx->d_name_off, &ctx->d_name8, &ctx->d_name16, &ctx->r_in, &ctx->r_out,
-                    &ctx->r_dosage, &ctx->r_loci, &ctx->r_loci_off, &ctx->r_comp, &ctx->r_blocks, &ctx->r_def_slots,
-                    &ctx->r_def_sizes, &ctx->r_def_offs, &ctx->r_def_out, &ctx->r_diags})
+  for (DevBuf *b : {&ctx->d_filt_blob, &ctx->d_filt_off, &ctx->d_names, &ctx->d_name_off, &ctx->d_name8, &ctx->d_name16,
+                    &ctx->r_def_slots, &ctx->r_def_sizes, &ctx->r_def_offs, &ctx->r_def_out})
     dev_free(*b);
-  scratch_free(ctx->r_sc);
-  if (ctx->r_stream) cudaStreamDestroy(ctx->r_stream);
-  if (ctx->r_d_ctr) cudaFree(ctx->r_d_ctr);
-  if (ctx->r_d_bad) cudaFree(ctx->r_d_bad);
-  if (ctx->r_h_ctr) cudaFreeHost(ctx->r_h_ctr);
+  run_free(ctx->res);
   for (auto e : ctx->ev_pool) cudaEventDestroy(e);
   delete ctx;
 }
@@ -797,65 +848,20 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
   cudaSetDevice(ctx->device);
   ctx->last_error.clear();
   const DevCfg &dc = ctx->dcfg;
-  static const bool trace = getenv("BVCF_TRACE") != nullptr;  // experiments: where a collect spends its time
+  static const bool trace = getenv("BVCF_TRACE") != nullptr;  // instrumentation: where a collect spends its time
   const auto t_begin = std::chrono::steady_clock::now();
+  Run &r = s->run;
   for (;;) {
     CK(cudaEventSynchronize(s->done));
-    if (s->bgzf && s->h_bad[0]) {  // a corrupt member: whatever the pipeline made of its text is not looked at
-      ctx->last_error = std::to_string(s->h_bad[0]) + " bgzf block(s) failed to inflate or failed their CRC-32 / ISIZE check";
-      return BVCF_E_ARG;
-    }
+    int rc;
+    if (s->bgzf && (rc = inflate_result(ctx, s->h_bad[0]))) return rc;  // a corrupt member: the rows made of it are not looked at
     if (s->bgzf && s->len > s->skip && (s->h_bad[1] & 0xFFu) != '\n') return BVCF_E_NOT_ALIGNED;
-    const RunCounters &c = *s->h_ctr;
-    bool again = false;
-    if (c.slot_overflow) {                                              // lines shorter than assumed: more line slots
-      if (ctx->min_line_bytes <= 1) return BVCF_E_TOO_LARGE;
-      ctx->min_line_bytes /= 2;
-      s->retries++;
-      if (s->retries > 8) return BVCF_E_TOO_LARGE;
-      const int rc = slot_enqueue(ctx, *s, false);
-      if (rc) return rc;
-      continue;
-    }
-    if (c.ev_overflow) {                                                // dense genotype block: more event slots
-      ctx->ev_factor *= 4;
-      s->retries++;
-      if (s->retries > 8) return BVCF_E_TOO_LARGE;
-      const int rc = slot_enqueue(ctx, *s, false);
-      if (rc) return rc;
-      continue;
-    }
-    if (c.row_overflow) { s->sc.row_cap = s->sc.row_cap * 4 + c.row_cursor; again = true; }  // MNP/multi-ALT heavy block
-    if (c.out_overflow) {
-      int rc = dev_reserve(ctx, s->d_out, (size_t)(c.out_cursor + c.out_cursor / 8 + 4096));
-      if (rc) return rc;
-      again = true;
-    }
-    if (dc.want_dosage && dc.n_samples > 0) {  // dosage rows, locus offsets and locus bytes grow to what the chunk reported
-      if (c.row_cursor * (uint64_t)dc.n_samples > s->d_dosage.cap || c.row_cursor * 8 > s->d_loci_off.cap) {
-        int rc = dev_reserve(ctx, s->d_dosage, (size_t)(c.row_cursor + 64) * dc.n_samples);
-        if (rc) return rc;
-        if ((rc = dev_reserve(ctx, s->d_loci_off, (size_t)(c.row_cursor + 64) * 8))) return rc;
-        again = true;
-      }
-      if (c.loci_cursor > s->d_loci.cap) {
-        int rc = dev_reserve(ctx, s->d_loci, (size_t)(c.loci_cursor + c.loci_cursor / 8 + 4096));
-        if (rc) return rc;
-        again = true;
-      }
-    }
-    // every log line or none.  Compared with the capacity this chunk ran with: another slot may have raised ctx->diag_cap
-    // since, and this slot's buffer is still the old size
-    if (c.n_diags > s->diag_cap) { ctx->diag_cap = std::max(ctx->diag_cap, c.n_diags + c.n_diags / 4); again = true; }
-    if (c.scratch_overflow) { s->sc.scratch_cap = c.scratch_cursor + c.scratch_cursor / 4 + (1ull << 20); again = true; }
-    if (c.slow_overflow) { s->sc.slow_cap = c.n_slow + c.n_slow / 4 + 1024; again = true; }
+    bool again;
+    if ((rc = grow_for_retry(ctx, r, *r.h_ctr, s->retries, again))) return rc;
     if (!again) break;
-    s->retries++;
-    if (s->retries > 8) return BVCF_E_TOO_LARGE;
-    const int rc = slot_enqueue(ctx, *s, false);  // input is still on the device
-    if (rc) return rc;
+    if ((rc = slot_enqueue(ctx, *s, false))) return rc;  // input is still on the device
   }
-  const RunCounters c = *s->h_ctr;
+  const RunCounters c = *r.h_ctr;
   // rows back to pinned host memory
   if (c.out_cursor > s->h_out_cap) {
     if (s->h_out) cudaFreeHost(s->h_out);
@@ -865,7 +871,7 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
     CK(cudaMallocHost(&s->h_out, cap));
     s->h_out_cap = cap;
   }
-  if (c.out_cursor) CK(cudaMemcpyAsync(s->h_out, s->d_out.p, c.out_cursor, cudaMemcpyDeviceToHost, s->stream));
+  if (c.out_cursor) CK(cudaMemcpyAsync(s->h_out, r.d_out.p, c.out_cursor, cudaMemcpyDeviceToHost, r.stream));
   const bool dos = dc.want_dosage && dc.n_samples > 0;
   if (dos && c.row_cursor) {
     const size_t nb = (size_t)c.row_cursor * dc.n_samples;
@@ -875,7 +881,7 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
       CK(cudaMallocHost(&s->h_dosage, nb + nb / 4));
       s->h_dosage_cap = nb + nb / 4;
     }
-    CK(cudaMemcpyAsync(s->h_dosage, s->d_dosage.p, nb, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(s->h_dosage, r.d_dosage.p, nb, cudaMemcpyDeviceToHost, r.stream));
     if (c.loci_cursor > s->h_loci_cap) {
       if (s->h_loci) cudaFreeHost(s->h_loci);
       s->h_loci = nullptr; s->h_loci_cap = 0;
@@ -890,19 +896,19 @@ int bvcf_collect(bvcf_ctx *ctx, uint64_t seq, const uint8_t **tsv, size_t *tsv_l
       CK(cudaMallocHost(&s->h_loci_off, cap * 8));
       s->h_loci_off_cap = cap;
     }
-    CK(cudaMemcpyAsync(s->h_loci, s->d_loci.p, c.loci_cursor, cudaMemcpyDeviceToHost, s->stream));
-    CK(cudaMemcpyAsync(s->h_loci_off, s->d_loci_off.p, c.row_cursor * 8, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(s->h_loci, r.d_loci.p, c.loci_cursor, cudaMemcpyDeviceToHost, r.stream));
+    CK(cudaMemcpyAsync(s->h_loci_off, r.d_loci_off.p, c.row_cursor * 8, cudaMemcpyDeviceToHost, r.stream));
   }
   // <= diag_cap: larger counts re-ran the chunk above.  A caller that takes no diagnostics does not pay for them: on
   // sites-only input with 9 % rejected alleles their copy, decode and sort was 3.6 ms of every 128 MiB chunk, more than
   // its PCIe time
-  const uint32_t nd = (diags || n_diags) ? std::min(c.n_diags, s->diag_cap) : 0u;
+  const uint32_t nd = (diags || n_diags) ? std::min(c.n_diags, r.diag_cap) : 0u;
   if (nd) {
     s->h_diag_raw.resize((size_t)nd * DIAG_WORDS);
-    CK(cudaMemcpyAsync(s->h_diag_raw.data(), s->d_diags.p, (size_t)nd * DIAG_WORDS * 4, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(s->h_diag_raw.data(), r.d_diags.p, (size_t)nd * DIAG_WORDS * 4, cudaMemcpyDeviceToHost, r.stream));
   }
   const auto t_kernels = std::chrono::steady_clock::now();
-  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaStreamSynchronize(r.stream));
   const auto t_copied = std::chrono::steady_clock::now();
   if (tsv) *tsv = s->h_out;
   if (tsv_len) *tsv_len = (size_t)c.out_cursor;
@@ -950,12 +956,12 @@ int bvcf_resident_alloc(bvcf_ctx *ctx, size_t in_bytes, size_t out_capacity, voi
   cudaSetDevice(ctx->device);
   const uint64_t buf_len = round_up(in_bytes, 1024) + 2048;
   int rc;
-  if ((rc = dev_reserve(ctx, ctx->r_in, buf_len + IN_SLACK))) return rc;
-  if ((rc = dev_reserve(ctx, ctx->r_out, std::max<size_t>(out_capacity, 4096)))) return rc;
-  CK(cudaMemset((uint8_t *)ctx->r_in.p + in_bytes, '\n', ctx->r_in.cap - in_bytes));
+  if ((rc = dev_reserve(ctx, ctx->res.d_in, buf_len + IN_SLACK))) return rc;
+  if ((rc = dev_reserve(ctx, ctx->res.d_out, std::max<size_t>(out_capacity, 4096)))) return rc;
+  CK(cudaMemset((uint8_t *)ctx->res.d_in.p + in_bytes, '\n', ctx->res.d_in.cap - in_bytes));
   ctx->r_in_bytes = in_bytes;
-  if (d_in) *d_in = ctx->r_in.p;
-  if (d_out) *d_out = ctx->r_out.p;
+  if (d_in) *d_in = ctx->res.d_in.p;
+  if (d_out) *d_out = ctx->res.d_out.p;
   return BVCF_OK;
 }
 
@@ -963,7 +969,7 @@ int bvcf_resident_upload(bvcf_ctx *ctx, size_t offset, const void *host, size_t 
   if (!ctx || !host) return BVCF_E_ARG;
   if (offset + len > ctx->r_in_bytes) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
-  CK(cudaMemcpy((uint8_t *)ctx->r_in.p + offset, host, len, cudaMemcpyHostToDevice));
+  CK(cudaMemcpy((uint8_t *)ctx->res.d_in.p + offset, host, len, cudaMemcpyHostToDevice));
   return BVCF_OK;
 }
 
@@ -976,67 +982,28 @@ int bvcf_resident_run_at(bvcf_ctx *ctx, size_t begin, size_t len, bvcf_chunk_sta
   if (!ctx->header_set) return BVCF_E_STATE;
   if (len > ctx->r_in_bytes || begin > len) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
-  const DevCfg &dc = ctx->dcfg;
+  Run &r = ctx->res;
   uint32_t retries = 0;
   uint64_t launches0 = ctx->launches;
   std::vector<StageEvents> timing;
   for (;;) {
     int rc;
-    if ((rc = scratch_reserve(ctx, ctx->r_sc, len - (begin & ~511ull), ctx->cfg.resident_subchunk_bytes))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->r_diags, (size_t)ctx->diag_cap * DIAG_WORDS * 4))) return rc;
+    // dosage rows and locus bytes start from nothing and grow to what the first run reports: a guess from the input
+    // size would be far too large for tens of gigabytes of wide lines
+    if ((rc = run_reserve(ctx, r, begin, len))) return rc;
     // the bytes after `len` must not look like data: pad (idempotent)
-    const uint64_t buf_len = std::min<uint64_t>((ctx->r_in.cap - IN_SLACK) / 1024 * 1024, round_up(len, 1024) + 2048);
-    CK(cudaMemsetAsync(ctx->r_d_ctr, 0, sizeof(RunCounters), ctx->r_stream));
-    uint64_t dos_rows = 0;
-    if (dc.want_dosage && dc.n_samples > 0)
-      dos_rows = std::min<uint64_t>(ctx->r_dosage.cap / (uint64_t)dc.n_samples, ctx->r_loci_off.cap / 8);
+    const uint64_t buf_len = std::min<uint64_t>((r.d_in.cap - IN_SLACK) / 1024 * 1024, round_up(len, 1024) + 2048);
     for (auto &t : timing)
       for (auto e : t.e) ctx->ev_pool.push_back(e);
     timing.clear();
     launches0 = ctx->launches;
-    rc = enqueue_pipeline(ctx, ctx->r_sc, ctx->r_stream, (const uint8_t *)ctx->r_in.p, begin, len, buf_len,
-                          (uint8_t *)ctx->r_out.p, ctx->r_out.cap, ctx->r_d_ctr, (int8_t *)ctx->r_dosage.p, dos_rows,
-                          (uint8_t *)ctx->r_loci.p, ctx->r_loci.cap, (unsigned long long *)ctx->r_loci_off.p,
-                          (uint32_t *)ctx->r_diags.p, ctx->diag_cap, times ? &timing : nullptr);
-    if (rc) return rc;
-    CK(cudaMemcpyAsync(ctx->r_h_ctr, ctx->r_d_ctr, sizeof(RunCounters), cudaMemcpyDeviceToHost, ctx->r_stream));
-    CK(cudaStreamSynchronize(ctx->r_stream));
-    const RunCounters &c = *ctx->r_h_ctr;
-    bool again = false;
-    if (c.slot_overflow) {  // lines shorter than assumed: more line slots, run again
-      if (ctx->min_line_bytes <= 1) return BVCF_E_TOO_LARGE;
-      ctx->min_line_bytes /= 2;
-      if (++retries > 8) return BVCF_E_TOO_LARGE;
-      continue;
-    }
-    if (c.ev_overflow) {  // dense genotype block: more event slots, run again
-      ctx->ev_factor *= 4;
-      if (++retries > 8) return BVCF_E_TOO_LARGE;
-      continue;
-    }
-    if (c.row_overflow) { ctx->r_sc.row_cap = ctx->r_sc.row_cap * 4 + c.row_cursor; again = true; }
-    if (c.scratch_overflow) { ctx->r_sc.scratch_cap = c.scratch_cursor + c.scratch_cursor / 4 + (1ull << 20); again = true; }
-    if (c.n_diags > ctx->diag_cap) { ctx->diag_cap = c.n_diags + c.n_diags / 4; again = true; }
-    if (c.slow_overflow) { ctx->r_sc.slow_cap = c.n_slow + c.n_slow / 4 + 1024; again = true; }
-    if (c.out_overflow) {
-      if ((rc = dev_reserve(ctx, ctx->r_out, (size_t)(c.out_cursor + c.out_cursor / 8 + 4096)))) return rc;
-      again = true;
-    }
-    if (dc.want_dosage && dc.n_samples > 0) {
-      if (c.row_cursor * (uint64_t)dc.n_samples > ctx->r_dosage.cap || c.row_cursor * 8 > ctx->r_loci_off.cap) {
-        if ((rc = dev_reserve(ctx, ctx->r_dosage, (size_t)(c.row_cursor + 64) * dc.n_samples))) return rc;
-        if ((rc = dev_reserve(ctx, ctx->r_loci_off, (size_t)(c.row_cursor + 64) * 8))) return rc;
-        again = true;
-      }
-      if (c.loci_cursor > ctx->r_loci.cap) {
-        if ((rc = dev_reserve(ctx, ctx->r_loci, (size_t)(c.loci_cursor + c.loci_cursor / 8 + 4096)))) return rc;
-        again = true;
-      }
-    }
+    if ((rc = enqueue_pipeline(ctx, r, begin, len, buf_len, times ? &timing : nullptr))) return rc;
+    CK(cudaStreamSynchronize(r.stream));
+    bool again;
+    if ((rc = grow_for_retry(ctx, r, *r.h_ctr, retries, again))) return rc;
     if (!again) break;
-    if (++retries > 8) return BVCF_E_TOO_LARGE;
   }
-  const RunCounters &c = *ctx->r_h_ctr;
+  const RunCounters &c = *r.h_ctr;
   ctx->r_last_records = c.n_records;
   ctx->r_last_len = len;
   if (stats) {
@@ -1122,23 +1089,12 @@ int bvcf_resident_inflate_bgzf(bvcf_ctx *ctx, const void *comp, size_t comp_len,
   if (blocks.empty()) return BVCF_OK;
   if (blocks.size() >= (1ull << 32)) return BVCF_E_TOO_LARGE;
   for (auto &b : blocks) b.out_off += dst_offset;
-  if ((rc = dev_reserve(ctx, ctx->r_comp, comp_len + 16))) return rc;
-  if ((rc = dev_reserve(ctx, ctx->r_blocks, blocks.size() * sizeof(InflateBlock)))) return rc;
-  if (!ctx->r_d_bad) CK(cudaMalloc(&ctx->r_d_bad, 4));
-  CK(cudaMemcpyAsync(ctx->r_comp.p, comp, comp_len, cudaMemcpyHostToDevice, ctx->r_stream));  // the compressed bytes cross PCIe
-  CK(cudaMemcpyAsync(ctx->r_blocks.p, blocks.data(), blocks.size() * sizeof(InflateBlock), cudaMemcpyHostToDevice, ctx->r_stream));
-  CK(cudaMemsetAsync(ctx->r_d_bad, 0, 4, ctx->r_stream));
-  InflateParams ip{};
-  ip.comp = (const uint8_t *)ctx->r_comp.p; ip.out = (uint8_t *)ctx->r_in.p; ip.blocks = (const InflateBlock *)ctx->r_blocks.p;
-  ip.n_blocks = (uint32_t)blocks.size(); ip.n_bad = ctx->r_d_bad;
-  cudaFuncSetAttribute(bvcf_inflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)INF_SMEM);
-  bvcf_inflate_kernel<<<ip.n_blocks, 32, INF_SMEM, ctx->r_stream>>>(ip);
-  ctx->launches++;
+  Run &r = ctx->res;
+  if ((rc = enqueue_inflate(ctx, r, (const uint8_t *)comp, comp_len, blocks.data(), blocks.size()))) return rc;
   uint32_t bad = 0;
-  CK(cudaMemcpyAsync(&bad, ctx->r_d_bad, 4, cudaMemcpyDeviceToHost, ctx->r_stream));
-  CK(cudaStreamSynchronize(ctx->r_stream));
-  if (bad) { ctx->last_error = std::to_string(bad) + " bgzf block(s) failed to inflate or failed their CRC-32 / ISIZE check"; return BVCF_E_ARG; }
-  return BVCF_OK;
+  CK(cudaMemcpyAsync(&bad, r.d_bad, 4, cudaMemcpyDeviceToHost, r.stream));
+  CK(cudaStreamSynchronize(r.stream));
+  return inflate_result(ctx, bad);
 }
 
 int bvcf_submit_bgzf(bvcf_ctx *ctx, uint64_t seq, const uint8_t *comp, size_t comp_len, size_t skip, const uint8_t *tail,
@@ -1185,6 +1141,7 @@ int bvcf_diag_fields(bvcf_ctx *ctx, uint64_t seq, const uint8_t **text, const ui
   Slot *s = find_slot(ctx, seq);
   if (!s) return BVCF_E_STATE;
   cudaSetDevice(ctx->device);
+  const Run &r = s->run;
   const size_t n = s->h_diags.size();
   s->h_field_off.assign(n + 1, 0);
   if (n) {
@@ -1194,22 +1151,22 @@ int bvcf_diag_fields(bvcf_ctx *ctx, uint64_t seq, const uint8_t **text, const ui
     int rc;
     if ((rc = dev_reserve(ctx, s->d_diag_starts, n * 8))) return rc;
     if ((rc = dev_reserve(ctx, s->d_field_off, (n + 1) * 8))) return rc;
-    CK(cudaMemcpyAsync(s->d_diag_starts.p, s->h_diag_starts.data(), n * 8, cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(s->d_diag_starts.p, s->h_diag_starts.data(), n * 8, cudaMemcpyHostToDevice, r.stream));
     const unsigned long long *st = (const unsigned long long *)s->d_diag_starts.p;
     unsigned long long *fo = (unsigned long long *)s->d_field_off.p;
-    bvcf_diag_fields_len_kernel<<<1, 1024, 0, s->stream>>>((const uint8_t *)s->d_in.p, s->len, st, (uint32_t)n, fo);
+    bvcf_diag_fields_len_kernel<<<1, 1024, 0, r.stream>>>((const uint8_t *)r.d_in.p, s->len, st, (uint32_t)n, fo);
     ctx->launches++;
-    CK(cudaMemcpyAsync(s->h_field_off.data(), fo, (n + 1) * 8, cudaMemcpyDeviceToHost, s->stream));
-    CK(cudaStreamSynchronize(s->stream));
+    CK(cudaMemcpyAsync(s->h_field_off.data(), fo, (n + 1) * 8, cudaMemcpyDeviceToHost, r.stream));
+    CK(cudaStreamSynchronize(r.stream));
     const size_t total = (size_t)s->h_field_off[n];
     s->h_fields.resize(total);
     if (total) {
       if ((rc = dev_reserve(ctx, s->d_fields, total))) return rc;
-      bvcf_diag_fields_copy_kernel<<<(unsigned)std::min<size_t>((n + 7) / 8, 1184), 256, 0, s->stream>>>(
-          (const uint8_t *)s->d_in.p, st, fo, (uint32_t)n, (uint8_t *)s->d_fields.p);
+      bvcf_diag_fields_copy_kernel<<<(unsigned)std::min<size_t>((n + 7) / 8, 1184), 256, 0, r.stream>>>(
+          (const uint8_t *)r.d_in.p, st, fo, (uint32_t)n, (uint8_t *)s->d_fields.p);
       ctx->launches++;
-      CK(cudaMemcpyAsync(s->h_fields.data(), s->d_fields.p, total, cudaMemcpyDeviceToHost, s->stream));
-      CK(cudaStreamSynchronize(s->stream));
+      CK(cudaMemcpyAsync(s->h_fields.data(), s->d_fields.p, total, cudaMemcpyDeviceToHost, r.stream));
+      CK(cudaStreamSynchronize(r.stream));
     }
     CK(cudaGetLastError());
   }
@@ -1226,7 +1183,7 @@ int bvcf_resident_download_bgzf(bvcf_ctx *ctx, size_t offset, size_t len, void *
 int bvcf_resident_download_bgzf_level(bvcf_ctx *ctx, size_t offset, size_t len, int level, void *host, size_t host_cap,
                                       size_t *comp_len) {
   if (!ctx || !host || !comp_len || level < 1 || level > 9) return BVCF_E_ARG;
-  if (offset + len > ctx->r_out.cap) return BVCF_E_ARG;
+  if (offset + len > ctx->res.d_out.cap) return BVCF_E_ARG;
   *comp_len = 0;
   if (len == 0) return BVCF_OK;
   cudaSetDevice(ctx->device);
@@ -1237,10 +1194,10 @@ int bvcf_resident_download_bgzf_level(bvcf_ctx *ctx, size_t offset, size_t len, 
   if ((rc = dev_reserve(ctx, ctx->r_def_slots, (size_t)nb * DEF_SLOT))) return rc;
   if ((rc = dev_reserve(ctx, ctx->r_def_sizes, (size_t)nb * 4))) return rc;
   if ((rc = dev_reserve(ctx, ctx->r_def_offs, (size_t)nb * 8))) return rc;
-  cudaStream_t st = ctx->r_stream;
+  cudaStream_t st = ctx->res.stream;
   CK(cudaMemsetAsync(ctx->r_def_slots.p, 0, (size_t)nb * DEF_SLOT, st));  // the token bits are OR-ed in
   DeflateParams dp{};
-  dp.text = (const uint8_t *)ctx->r_out.p + offset; dp.text_len = len; dp.slots = (uint8_t *)ctx->r_def_slots.p;
+  dp.text = (const uint8_t *)ctx->res.d_out.p + offset; dp.text_len = len; dp.slots = (uint8_t *)ctx->r_def_slots.p;
   dp.sizes = (uint32_t *)ctx->r_def_sizes.p; dp.n_blocks = nb;
   if (level == 1) bvcf_deflate_kernel<<<nb, 32, 0, st>>>(dp);
   else bvcf_deflate_dyn_kernel<<<nb, 32, def_dyn_smem(DEF_LEVELS[level]), st>>>(dp, DEF_LEVELS[level]);
@@ -1273,7 +1230,7 @@ int bvcf_resident_download_bgzf_level(bvcf_ctx *ctx, size_t offset, size_t len, 
 int bvcf_resident_results(bvcf_ctx *ctx, bvcf_dosage_batch *dosage, const bvcf_diag **diags, size_t *n_diags) {
   if (!ctx) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
-  const RunCounters &c = *ctx->r_h_ctr;
+  const RunCounters &c = *ctx->res.h_ctr;
   const DevCfg &dc = ctx->dcfg;
   if (dosage) {
     memset(dosage, 0, sizeof(*dosage));
@@ -1282,9 +1239,9 @@ int bvcf_resident_results(bvcf_ctx *ctx, bvcf_dosage_batch *dosage, const bvcf_d
       ctx->r_h_dosage.resize((size_t)c.row_cursor * dc.n_samples);
       ctx->r_h_loci.resize((size_t)c.loci_cursor);
       ctx->r_h_loci_off.resize((size_t)c.row_cursor + 1);
-      CK(cudaMemcpy(ctx->r_h_dosage.data(), ctx->r_dosage.p, ctx->r_h_dosage.size(), cudaMemcpyDeviceToHost));
-      if (c.loci_cursor) CK(cudaMemcpy(ctx->r_h_loci.data(), ctx->r_loci.p, (size_t)c.loci_cursor, cudaMemcpyDeviceToHost));
-      CK(cudaMemcpy(ctx->r_h_loci_off.data(), ctx->r_loci_off.p, (size_t)c.row_cursor * 8, cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(ctx->r_h_dosage.data(), ctx->res.d_dosage.p, ctx->r_h_dosage.size(), cudaMemcpyDeviceToHost));
+      if (c.loci_cursor) CK(cudaMemcpy(ctx->r_h_loci.data(), ctx->res.d_loci.p, (size_t)c.loci_cursor, cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(ctx->r_h_loci_off.data(), ctx->res.d_loci_off.p, (size_t)c.row_cursor * 8, cudaMemcpyDeviceToHost));
       ctx->r_h_loci_off[c.row_cursor] = c.loci_cursor;
       dosage->n_rows = c.row_cursor;
       dosage->dosage = ctx->r_h_dosage.data();
@@ -1293,10 +1250,10 @@ int bvcf_resident_results(bvcf_ctx *ctx, bvcf_dosage_batch *dosage, const bvcf_d
     }
   }
   ctx->r_h_diags.clear();
-  const uint32_t nd = std::min<uint32_t>(c.n_diags, ctx->diag_cap);
-  if (nd && ctx->r_diags.p) {
+  const uint32_t nd = std::min<uint32_t>(c.n_diags, ctx->res.diag_cap);
+  if (nd && ctx->res.d_diags.p) {
     std::vector<uint32_t> raw((size_t)nd * DIAG_WORDS);
-    CK(cudaMemcpy(raw.data(), ctx->r_diags.p, raw.size() * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(raw.data(), ctx->res.d_diags.p, raw.size() * 4, cudaMemcpyDeviceToHost));
     decode_diags(raw.data(), nd, ctx->r_h_diags);
   }
   if (diags) *diags = ctx->r_h_diags.data();
@@ -1306,25 +1263,25 @@ int bvcf_resident_results(bvcf_ctx *ctx, bvcf_dosage_batch *dosage, const bvcf_d
 
 int bvcf_resident_write_output(bvcf_ctx *ctx, size_t offset, const void *host, size_t len) {
   if (!ctx || !host) return BVCF_E_ARG;
-  if (offset + len > ctx->r_out.cap) return BVCF_E_ARG;
+  if (offset + len > ctx->res.d_out.cap) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
-  CK(cudaMemcpy((uint8_t *)ctx->r_out.p + offset, host, len, cudaMemcpyHostToDevice));
+  CK(cudaMemcpy((uint8_t *)ctx->res.d_out.p + offset, host, len, cudaMemcpyHostToDevice));
   return BVCF_OK;
 }
 
 int bvcf_resident_download(bvcf_ctx *ctx, size_t offset, void *host, size_t len) {
   if (!ctx || !host) return BVCF_E_ARG;
-  if (offset + len > ctx->r_out.cap) return BVCF_E_ARG;
+  if (offset + len > ctx->res.d_out.cap) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
-  CK(cudaMemcpy(host, (uint8_t *)ctx->r_out.p + offset, len, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(host, (uint8_t *)ctx->res.d_out.p + offset, len, cudaMemcpyDeviceToHost));
   return BVCF_OK;
 }
 
 int bvcf_resident_peek(bvcf_ctx *ctx, size_t offset, void *host, size_t len) {
   if (!ctx || !host) return BVCF_E_ARG;
-  if (offset + len > ctx->r_in.cap) return BVCF_E_ARG;
+  if (offset + len > ctx->res.d_in.cap) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
-  CK(cudaMemcpy(host, (uint8_t *)ctx->r_in.p + offset, len, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(host, (uint8_t *)ctx->res.d_in.p + offset, len, cudaMemcpyDeviceToHost));
   return BVCF_OK;
 }
 
@@ -1333,11 +1290,11 @@ int bvcf_resident_line_index(bvcf_ctx *ctx, uint64_t *starts, uint32_t *lens, ui
   if (!ctx) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
   // valid for single-sub-chunk runs: the dense table of the last sub-chunk
-  const size_t n = (size_t)std::min<uint64_t>(ctx->r_h_ctr->chunk_records, cap);
-  if (n_records) *n_records = ctx->r_h_ctr->chunk_records;
+  const size_t n = (size_t)std::min<uint64_t>(ctx->res.h_ctr->chunk_records, cap);
+  if (n_records) *n_records = ctx->res.h_ctr->chunk_records;
   if (n == 0) return BVCF_OK;
   std::vector<LineRec> tmp(n);
-  CK(cudaMemcpy(tmp.data(), ctx->r_sc.dense.p, n * sizeof(LineRec), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(tmp.data(), ctx->res.sc.dense.p, n * sizeof(LineRec), cudaMemcpyDeviceToHost));
   for (size_t i = 0; i < n; i++) {
     if (starts) starts[i] = tmp[i].start;
     if (lens) lens[i] = tmp[i].len;

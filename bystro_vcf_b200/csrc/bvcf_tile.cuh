@@ -747,9 +747,9 @@ constexpr uint32_t TILE_BLOCK_HDR = 32u * (uint32_t)sizeof(LaneRec);
 
 // ---- compose ------------------------------------------------------------------------------------------------
 // MINB resident CTAs per SM (sets the register budget), ARENA staging bytes and ROWS row descriptors per warp.
-// Records with samples give about one row each (wide text: 10 KiB, 48 rows); sites-only input gives 1.6 short rows per
-// record at BASELINE's 30 % multi-allelic / MNP mix (8 KiB, 160 rows).
-template <int MINB, uint32_t ARENA, uint32_t ROWS, bool PREFETCH, bool SPEC = false>
+// Records with samples give about one row each (wide text: 10 KiB, 48 rows); sites-only input has a composer of its own
+// (bvcf_compose_sites_kernel below).
+template <int MINB, uint32_t ARENA, uint32_t ROWS, bool SPEC = false>
 __global__ void __launch_bounds__(TILE_WARPS * 32, MINB) bvcf_compose_kernel(const __grid_constant__ TileParams p) {
   constexpr uint32_t TILE_ARENA = ARENA, TILE_ROWS = ROWS, TILE_SMEM_WARP = tile_smem_warp(ARENA, ROWS);
   static_assert(ROWS <= TILE_ROWS_MAX && ROWS >= TILE_THREADS, "row table size");
@@ -778,47 +778,19 @@ __global__ void __launch_bounds__(TILE_WARPS * 32, MINB) bvcf_compose_kernel(con
   sh.arena_cur = &s_cur[warp][0];
   sh.rows_cur = &s_cur[warp][1];
 
-  // Tiles are taken with a fixed stride so that a warp knows its next two tiles: the record of the tile after next is
-  // loaded (its line start, its event list) while this tile is composed, and the first bytes of the next tile's lines
-  // and events are pulled into L2.  The lines were last touched by the scan kernel gigabytes ago: without this every
-  // thread waits for DRAM two or three times in a row at the start of its record.
-  auto rec_head = [&](uint32_t t, unsigned long long &start, uint32_t &ev_start) {
-    const uint32_t i = t * TILE_THREADS + lane;
-    start = ~0ull; ev_start = 0;
-    if (t < n_tiles && i < n_rec) {
-      const uint4 a = reinterpret_cast<const uint4 *>(p.lines + i)[0], b = reinterpret_cast<const uint4 *>(p.lines + i)[1];
-      start = (unsigned long long)a.x | ((unsigned long long)a.y << 32);
-      ev_start = b.x;
-    }
-  };
-  auto pull = [&](unsigned long long start, uint32_t ev_start) {
-    if (start != ~0ull) {
-      const uint8_t *l = p.in + start;
-      asm volatile("prefetch.global.L2 [%0];\n" ::"l"(l));
-      asm volatile("prefetch.global.L2 [%0];\n" ::"l"(l + 128));
-      if (has_samples) asm volatile("prefetch.global.L2 [%0];\n" ::"l"(p.events + ev_start));
-    }
-  };
-  // Tiles are handed out by a ticket counter (rows differ a lot in cost), two tickets ahead, so that a warp knows its
-  // next two tiles: the record of the tile after next is loaded (line start, event list) while this tile is composed,
-  // and the first bytes of the next tile's lines and events are pulled into L2.  The lines were last touched by the
-  // scan kernel gigabytes ago: without this every thread waits for DRAM two or three times at the start of its record.
+  // Tiles are handed out by a ticket counter (rows differ a lot in cost), two tickets ahead: a warp holds the next two
+  // tiles it will compose.  The order was made for an L2 prefetch of those tiles' lines and events, which was measured
+  // and dropped (no gain: the waits are dependent L1/L2 hits, not DRAM); it stays because the tile schedule is part of
+  // every time measured on this kernel since, and taking one ticket per tile changes it.
   auto ticket = [&]() {
     uint32_t t = 0;
     if (lane == 0) t = atomicAdd(&p.ctr->tile_ticket, 1u);
     return __shfl_sync(FULL, t, 0);
   };
   uint32_t tile = ticket(), tile_n1 = ticket(), tile_n2;
-  unsigned long long nx_start;  // line start / event list of this lane's record in the NEXT tile
-  uint32_t nx_ev;
-  if (PREFETCH) rec_head(tile_n1, nx_start, nx_ev); else { nx_start = ~0ull; nx_ev = 0; }
   for (; tile < n_tiles; tile = tile_n1, tile_n1 = tile_n2) {
     if (lane == 0) { s_cur[warp][0] = 0; s_cur[warp][1] = TILE_THREADS; }
     tile_n2 = ticket();  // also orders the cursor reset before the lanes' allocations
-    if (PREFETCH) {
-      pull(nx_start, nx_ev);
-      rec_head(tile_n2, nx_start, nx_ev);  // consumed one iteration from now
-    }
     const uint32_t li = tile * TILE_THREADS + lane;
     const bool valid = li < n_rec;
 
@@ -909,7 +881,7 @@ __device__ __forceinline__ void sites_row_text(W &w, const DevCfg &cfg, const Li
   row_text_keep<W, false>(w, cfg, lc, oa);
 }
 
-template <int MINB, uint32_t ARENA, uint32_t ROWS, bool CACHE>
+template <int MINB, uint32_t ARENA, uint32_t ROWS>
 __global__ void __launch_bounds__(TILE_WARPS * 32, MINB) bvcf_compose_sites_kernel(const __grid_constant__ TileParams p) {
   constexpr uint32_t TILE_SMEM_WARP = tile_smem_warp(ARENA, ROWS);
   static_assert(ROWS <= TILE_ROWS_MAX && ROWS >= TILE_THREADS && ARENA < 65536u, "row table / arena size");
@@ -954,7 +926,7 @@ __global__ void __launch_bounds__(TILE_WARPS * 32, MINB) bvcf_compose_sites_kern
       DiagSink ds;
       unsigned long long line_no;
       uint32_t t[9];
-      record_open<CACHE>(p, li, rec, s_filt, s_filt_off, true, lc, g, ds, line_no, t);
+      record_open<false>(p, li, rec, s_filt, s_filt_off, true, lc, g, ds, line_no, t);  // REF / ALT in registers spill at 64
       start = rec.start; t0 = t[0]; t1 = t[1]; t2 = t[2];
       info_n = (uint32_t)lc.info_n; info_off = t[6] + 1;
       OutAllele oa;
@@ -1254,7 +1226,6 @@ __device__ __forceinline__ void warp_copy_out(uint8_t *d, const uint8_t *s, uint
   const uint32_t done = nv << 4, rest = n - done;
   if ((uint32_t)lane < rest) d[done + lane] = s[done + lane];
 }
-template <bool PREFETCH>
 __global__ void __launch_bounds__(TILE_WARPS * 32, 8) bvcf_copyout_kernel(const __grid_constant__ TileParams p) {
   const DevCfg &cfg = p.cfg;
   const int lane = threadIdx.x & 31;
@@ -1267,9 +1238,7 @@ __global__ void __launch_bounds__(TILE_WARPS * 32, 8) bvcf_copyout_kernel(const 
   const bool has_samples = cfg.n_samples > 0;
   const bool want_locus = cfg.want_dosage && has_samples;
 
-  // tiles by ticket, one ahead: the next tile's totals are loaded while this one is copied, and its whole scratch
-  // block is pulled into L2 (the dependent chain totals -> block -> row table -> staged bytes would otherwise be four
-  // DRAM round trips per tile)
+  // tiles by ticket, one ahead: the next tile's totals are loaded while this one is copied
   auto ticket = [&]() {
     uint32_t t = 0;
     if (lane == 0) t = atomicAdd(&p.ctr->tile_ticket2, 1u);
@@ -1283,10 +1252,7 @@ __global__ void __launch_bounds__(TILE_WARPS * 32, 8) bvcf_copyout_kernel(const 
   for (; tile < n_tiles; tile = tile_n1, tile_n1 = ticket()) {
     const TileAgg ag = ag_next;
     const bool more = tile_n1 < n_tiles;
-    if (more) {
-      ag_next = p.tile_agg[tile_n1];  // consumed further down, after this tile's own loads
-      if (PREFETCH) asm volatile("prefetch.global.L2 [%0];\n" ::"l"(p.tile_base + tile_n1));
-    }
+    if (more) ag_next = p.tile_agg[tile_n1];  // consumed further down, after this tile's own loads
     const TileBase tb = p.tile_base[tile];
     const uint8_t *blk = p.scratch + ag.scratch_off;
     if (ag.flags & 1u) {  // a dense block: the tile's output bytes, in order
@@ -1304,11 +1270,6 @@ __global__ void __launch_bounds__(TILE_WARPS * 32, 8) bvcf_copyout_kernel(const 
     const unsigned long long in_rl = warp_scan64((unsigned long long)lr.rows | ((unsigned long long)lr.loci << 32), tot, lane);
     const unsigned long long in_d = warp_scan64(cls == 1 ? ((unsigned long long)lr.n_desc << 32) : (cls == 0 ? (unsigned long long)lr.n_desc : 0ull), tot, lane);
     const unsigned long long in_l = warp_scan64(cls == 2 ? (unsigned long long)lr.n_desc : 0ull, tot, lane);
-    if (PREFETCH && more) {  // the next tile's block into L2
-      const uint8_t *nb = p.scratch + ag_next.scratch_off;
-      const uint32_t nbytes = TILE_BLOCK_HDR + ag_next.n_trows * (uint32_t)sizeof(TRow) + ag_next.arena_used;
-      for (uint32_t o = lane * 128u; o < nbytes; o += 32u * 128u) asm volatile("prefetch.global.L2 [%0];\n" ::"l"(nb + o));
-    }
 
     // (the tile's dosage rows were zeroed by bvcf_dosage_zero_kernel: all-reference; the small rows' samples are
     // scattered below, the queued rows' by the names kernels)

@@ -155,18 +155,17 @@ def test_sites_only_overfull_tiles():
         assert gpu_rows(vcf, **kw) == oracle_rows(vcf, **kw)
 
 
-def test_sites_only_matches_thread_per_record_composer(monkeypatch):
-    """the two sites-only composers (BVCF_SITES_OLD selects round 2's first one) give the same bytes and diagnostics"""
+def test_sites_only_heavy_mix_rows_and_diagnostics():
+    """bvcf_compose_sites_kernel with --keepInfo on 60 % multi-row and malformed records: the oracle's bytes and
+    diagnostics"""
     from oracle import oracle as O
 
     rng = random.Random(4)
     vcf = V._vcf(V.HDR8, _sites_recs(rng, 6000, heavy=0.6))
     ref = O.read_vcf(O.OracleConfig(keep_info=True), vcf)
     a = _process(vcf, _cfg(keep_info=True))
-    monkeypatch.setenv("BVCF_SITES_OLD", "1")
-    b = _process(vcf, _cfg(keep_info=True))
-    assert a.tsv == b.tsv == ref.tsv
-    assert sorted(a.diags) == sorted(b.diags) == sorted(ref.diags)
+    assert a.tsv == ref.tsv
+    assert sorted(a.diags) == sorted(ref.diags)
 
 
 def test_long_info_spans_appended_at_copy_out():
