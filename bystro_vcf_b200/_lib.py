@@ -81,7 +81,7 @@ SYMBOLS = [
     "bvcf_resident_run", "bvcf_resident_download", "bvcf_resident_peek", "bvcf_resident_line_index", "bvcf_strerror",
     "bvcf_last_error", "bvcf_abi_version", "bvcf_launch_count", "bvcf_resident_run_at", "bvcf_resident_inflate_bgzf",
     "bvcf_bgzf_text_bytes", "bvcf_resident_download_bgzf", "bvcf_resident_write_output", "bvcf_resident_results",
-    "bvcf_submit_bgzf", "bvcf_diag_fields", "bvcf_resident_download_bgzf_level",
+    "bvcf_submit_bgzf", "bvcf_diag_fields", "bvcf_resident_download_bgzf_level", "bvcf_set_regions", "bvcf_index_spans",
 ]
 
 _lib = None
@@ -148,6 +148,11 @@ def lib():
     L.bvcf_resident_line_index.restype = C.c_int
     L.bvcf_resident_line_index.argtypes = [vp, C.POINTER(u64), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), sz,
                                            C.POINTER(sz)]
+    L.bvcf_set_regions.restype = C.c_int
+    L.bvcf_set_regions.argtypes = [vp, C.POINTER(C.c_char_p), C.POINTER(C.c_int64), C.POINTER(C.c_int64), sz]
+    L.bvcf_index_spans.restype = C.c_int
+    L.bvcf_index_spans.argtypes = [vp, sz, C.POINTER(C.c_char_p), C.POINTER(C.c_int64), C.POINTER(C.c_int64), sz,
+                                   C.POINTER(u64), sz, C.POINTER(sz)]
     L.bvcf_strerror.restype = C.c_char_p
     L.bvcf_strerror.argtypes = [C.c_int]
     L.bvcf_last_error.restype = C.c_char_p

@@ -180,6 +180,65 @@ def plan_groups(buf, data_off: int, chunk_bytes: int, cap: int) -> List[Group]:
         return out
 
 
+def index_views(buf, in_path: str, regions):
+    """What a run with regions reads of the whole bgzf file buf (read from in_path) when a tabix or CSI index lies beside
+    it (in_path + ".tbi", else + ".csi"): (lo, hi, skip) per span the index gives (bvcf_index_spans) -- buf[lo:hi] holds
+    the blocks from the span's first to its last, its data lines start at text offset skip.  The C++ host's reader
+    (csrc/bvcf_host.cpp index_pieces) follows the same rule.  None when there is no index; ValueError when the index is
+    malformed or points at bytes that are not a bgzf block of buf."""
+    import ctypes as C
+    import gzip
+    import os
+
+    from . import _lib
+
+    path = next((in_path + e for e in (".tbi", ".csi") if os.path.exists(in_path + e)), None)
+    if path is None:
+        return None
+    with gzip.open(path, "rb") as f:
+        idx = f.read()
+    L, n = _lib.lib(), len(regions)
+    names = (C.c_char_p * max(n, 1))(*[c for c, _, _ in regions])
+    beg = (C.c_int64 * max(n, 1))(*[b for _, b, _ in regions])
+    end = (C.c_int64 * max(n, 1))(*[e for _, _, e in regions])
+    cap, got = 1024, C.c_size_t()
+    while True:
+        sp = (C.c_uint64 * (2 * cap))()
+        rc = L.bvcf_index_spans(idx, len(idx), names, beg, end, n, sp, cap, C.byref(got))
+        if rc != -5:  # BVCF_E_TOO_LARGE: got says how many
+            break
+        cap = got.value
+    if rc:
+        raise ValueError("%s: not a tabix or CSI index (%d)" % (path, rc))
+
+    def block_at(off: int) -> int:
+        try:
+            bs = block_size(buf, off) if off < len(buf) else 0
+        except ValueError:
+            bs = 0
+        if bs == 0 or off + bs > len(buf):
+            raise ValueError("%s: virtual offset %d << 16 is not a bgzf block of %s" % (path, off, in_path))
+        return bs
+
+    views = []
+    for k in range(got.value):
+        cb, ce, ue = sp[2 * k] >> 16, sp[2 * k + 1] >> 16, sp[2 * k + 1] & 0xFFFF
+        block_at(cb)
+        hi = ce + block_at(ce) if ue else ce
+        if hi > len(buf):
+            raise ValueError("%s: virtual offset %d << 16 is past the end of %s" % (path, ce, in_path))
+        if hi > cb:
+            views.append((cb, hi, sp[2 * k] & 0xFFFF))
+    return views
+
+
+def plan_views(buf, views, chunk_bytes: int, cap: int) -> List[Group]:
+    """plan_groups over each (lo, hi, skip) of index_views, the groups' offsets into buf"""
+    mv = memoryview(buf)
+    return [g._replace(lo=g.lo + lo, hi=g.hi + lo) for lo, hi, skip in views
+            for g in plan_groups(mv[lo:hi], skip, chunk_bytes, cap)]
+
+
 def _one_block(args) -> bytes:
     chunk, level, strategy = args
     c = zlib.compressobj(level, zlib.DEFLATED, -15, 9, strategy)

@@ -4,6 +4,7 @@
 //   bvcf_scan_genotype_kernel      index + genotype events                    (north-star kernels 1+3)
 //   bvcf_prefix_* (mode 0)         per-range record counts -> bases
 //   bvcf_compact_lines_kernel      input-ordered line table
+//   bvcf_region_{mark,compact}_    only with regions set (bvcf_set_regions): the records inside them, in input order
 //   bvcf_line_stats_{,big_}kernel  genotype summaries the scan could not finish inline
 //   bvcf_compose_kernel            FILTER + getAlleles + row text + short name lists, staged per tile of 32 records
 //   bvcf_tile_{reduce,spine,offsets}  tile totals -> output offsets, cursors            (north-star kernels 2+4)
@@ -20,11 +21,13 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <string>
 #include <vector>
 
 #include "bvcf_common.cuh"
 #include "bvcf_prefix.cuh"
+#include "bvcf_region.cuh"
 #include "bvcf_rows.cuh"
 #include "bvcf_tile.cuh"
 #include "bvcf_names.cuh"
@@ -49,6 +52,7 @@ struct Scratch {
   uint64_t row_cap = 0;       // RowDesc slots (rows one sub-chunk may emit)
   DevBuf recs, range_nrec, range_nlines, rec_base, line_base, events, dense, partial, stats1, row_desc, big_recs, tile_agg,
       tile_base, tile_partial, tile_scratch, slow;
+  DevBuf kept, keep, block_n;  // region filter (only with regions set)
   uint64_t scratch_cap = 0;   // bytes of tile blocks (grown on scratch_overflow)
   uint32_t slow_cap = 0;      // slow-path list entries (grown on slow_overflow)
 };
@@ -107,6 +111,10 @@ struct bvcf_ctx {
   std::string empty_field, field_delim;
   std::vector<std::string> allow, exclude;
   bool header_set = false;
+  // regions (bvcf_set_regions): the kernels' table and its device buffers; n_regions == 0: no region filter
+  size_t n_regions = 0;
+  RegionTable rgn{};
+  DevBuf d_rgn_names, d_rgn_name_off, d_rgn_slot, d_rgn_iv_off, d_rgn_beg, d_rgn_end;
   DevCfg dcfg{};
   DevBuf d_filt_blob, d_filt_off, d_names, d_name_off, d_name8, d_name16;
   std::vector<Slot> slots;
@@ -221,12 +229,17 @@ int scratch_reserve(bvcf_ctx *ctx, Scratch &sc, uint64_t total_bytes, uint64_t s
     if ((rc = dev_reserve(ctx, sc.row_desc, sc.row_cap * sizeof(RowDesc)))) return rc;
     if ((rc = dev_reserve(ctx, sc.big_recs, sc.max_records * 4))) return rc;
   }
+  if (ctx->n_regions) {
+    if ((rc = dev_reserve(ctx, sc.kept, sc.max_records * sizeof(LineRec)))) return rc;
+    if ((rc = dev_reserve(ctx, sc.keep, sc.max_records))) return rc;
+    if ((rc = dev_reserve(ctx, sc.block_n, (RGN_BLOCKS + 1) * 4))) return rc;
+  }
   return 0;
 }
 void scratch_free(Scratch &sc) {
   for (DevBuf *b : {&sc.recs, &sc.range_nrec, &sc.range_nlines, &sc.rec_base, &sc.line_base, &sc.events, &sc.dense,
                     &sc.partial, &sc.stats1, &sc.row_desc, &sc.big_recs, &sc.tile_agg, &sc.tile_base, &sc.tile_partial,
-                    &sc.tile_scratch, &sc.slow})
+                    &sc.tile_scratch, &sc.slow, &sc.kept, &sc.keep, &sc.block_n})
     dev_free(*b);
 }
 
@@ -330,6 +343,18 @@ int enqueue_pipeline(bvcf_ctx *ctx, Run &r, uint64_t begin, uint64_t len, uint64
     cp.dense = (LineRec *)sc.dense.p; cp.n_ranges = nr; cp.slots_per_range = sc.slots; cp.evcap_words = sc.evcap_words;
     bvcf_compact_lines_kernel<<<(nr + 7) / 8, 256, 0, st>>>(cp);
     ctx->launches += 4;
+    // 3a. regions: the records inside them, in input order, and their count in chunk_records; every later stage reads
+    // this table
+    const LineRec *lines = cp.dense;
+    if (ctx->n_regions) {
+      RegionParams rp{};
+      rp.in = d_in; rp.lines = cp.dense; rp.kept = (LineRec *)sc.kept.p; rp.keep = (uint8_t *)sc.keep.p;
+      rp.block_n = (unsigned int *)sc.block_n.p; rp.t = ctx->rgn; rp.ctr = d_ctr;
+      bvcf_region_mark_kernel<<<RGN_BLOCKS, RGN_THREADS, 0, st>>>(rp);
+      bvcf_region_compact_kernel<<<RGN_BLOCKS, RGN_THREADS, 0, st>>>(rp);
+      ctx->launches += 2;
+      lines = rp.kept;
+    }
     if (se) CK(cudaEventRecord(se->e[2], st));
     // many more CTAs than SMs: each warp gets about one block of 32 records/rows and the hardware
     // scheduler evens out the very different row sizes (1 .. 2,500 names)
@@ -337,7 +362,7 @@ int enqueue_pipeline(bvcf_ctx *ctx, Run &r, uint64_t begin, uint64_t len, uint64
     // 3b. ALT #1 genotype summary per record (warp per record)
     if (dc.n_samples > 0) {
       StatsParams tp{};
-      tp.in = d_in; tp.cfg = dc; tp.lines = cp.dense; tp.events = sp.events; tp.stats = (LineStats *)sc.stats1.p; tp.ctr = d_ctr;
+      tp.in = d_in; tp.cfg = dc; tp.lines = lines; tp.events = sp.events; tp.stats = (LineStats *)sc.stats1.p; tp.ctr = d_ctr;
       tp.big_recs = (uint32_t *)sc.big_recs.p;
       bvcf_line_stats_kernel<<<wgrid, 256, 0, st>>>(tp);
       bvcf_line_stats_big_kernel<<<(unsigned)n_sm * 4, 256, 0, st>>>(tp);
@@ -347,7 +372,7 @@ int enqueue_pipeline(bvcf_ctx *ctx, Run &r, uint64_t begin, uint64_t len, uint64
     // 4. rows: FILTER + getAlleles + row text + short name lists, one pass (tile of 128 records per CTA)
     const bool vec = (dc.name8 || dc.name16) && dc.want_tsv && dc.n_samples > 0;
     TileParams tp{};
-    tp.in = d_in; tp.cfg = dc; tp.lines = cp.dense; tp.events = sp.events; tp.stats = (const LineStats *)sc.stats1.p;
+    tp.in = d_in; tp.cfg = dc; tp.lines = lines; tp.events = sp.events; tp.stats = (const LineStats *)sc.stats1.p;
     tp.out = (uint8_t *)r.d_out.p; tp.out_cap = r.d_out.cap; tp.ctr = d_ctr;
     tp.tile_agg = (TileAgg *)sc.tile_agg.p; tp.tile_base = (TileBase *)sc.tile_base.p;
     tp.tile_partial = (unsigned long long *)sc.tile_partial.p;
@@ -405,7 +430,7 @@ int enqueue_pipeline(bvcf_ctx *ctx, Run &r, uint64_t begin, uint64_t len, uint64
     // item has one size of 5..16 bytes (bvcf_names.cuh) -- and a CTA per row beyond 4,096 quads
     if (dc.n_samples > 0) {
       NamesParams np{};
-      np.in = d_in; np.cfg = dc; np.lines = cp.dense; np.events = sp.events; np.row_desc = (const RowDesc *)sc.row_desc.p;
+      np.in = d_in; np.cfg = dc; np.lines = lines; np.events = sp.events; np.row_desc = (const RowDesc *)sc.row_desc.p;
       np.row_desc_cap = sc.row_cap; np.out = tp.out; np.ctr = d_ctr; np.dosage = d_dosage; np.dosage_cap_rows = dosage_cap_rows;
       np.long_words = tp.long_words;
       if (vec) {
@@ -739,7 +764,8 @@ void bvcf_destroy(bvcf_ctx *ctx) {
     if (s.h_loci_off) cudaFreeHost(s.h_loci_off);
   }
   for (DevBuf *b : {&ctx->d_filt_blob, &ctx->d_filt_off, &ctx->d_names, &ctx->d_name_off, &ctx->d_name8, &ctx->d_name16,
-                    &ctx->r_def_slots, &ctx->r_def_sizes, &ctx->r_def_offs, &ctx->r_def_out})
+                    &ctx->r_def_slots, &ctx->r_def_sizes, &ctx->r_def_offs, &ctx->r_def_out, &ctx->d_rgn_names,
+                    &ctx->d_rgn_name_off, &ctx->d_rgn_slot, &ctx->d_rgn_iv_off, &ctx->d_rgn_beg, &ctx->d_rgn_end})
     dev_free(*b);
   run_free(ctx->res);
   for (auto e : ctx->ev_pool) cudaEventDestroy(e);
@@ -811,6 +837,71 @@ int bvcf_set_header(bvcf_ctx *ctx, const char *chrom_line, size_t len) {
     ctx->dcfg.item_bytes = I;
   }
   ctx->header_set = true;
+  return BVCF_OK;
+}
+
+int bvcf_set_regions(bvcf_ctx *ctx, const char *const *chrom, const int64_t *beg, const int64_t *end, size_t n) {
+  if (!ctx || (n && (!chrom || !beg || !end))) return BVCF_E_ARG;
+  for (size_t i = 0; i < n; i++)
+    if (!chrom[i] || !chrom[i][0] || beg[i] < 1 || beg[i] > end[i]) return BVCF_E_ARG;
+  for (auto &s : ctx->slots)
+    if (s.busy) return BVCF_E_STATE;
+  cudaSetDevice(ctx->device);
+  ctx->n_regions = 0;
+  if (!n) return BVCF_OK;
+  // contigs in order of first appearance, each one's intervals sorted, overlapping and adjacent ones merged
+  std::vector<std::string> names;
+  std::vector<std::vector<std::pair<int64_t, int64_t>>> ivs;
+  {
+    std::map<std::string, size_t> idx;  // name -> contig
+    for (size_t i = 0; i < n; i++) {
+      auto it = idx.emplace(chrom[i], names.size()).first;
+      if (it->second == names.size()) {
+        names.push_back(it->first);
+        ivs.emplace_back();
+      }
+      ivs[it->second].push_back({beg[i], end[i]});
+    }
+  }
+  std::vector<uint8_t> blob;
+  std::vector<uint32_t> name_off{0}, iv_off{0};
+  std::vector<long long> vb, ve;
+  for (size_t c = 0; c < names.size(); c++) {
+    blob.insert(blob.end(), names[c].begin(), names[c].end());
+    name_off.push_back((uint32_t)blob.size());
+    auto &v = ivs[c];
+    std::sort(v.begin(), v.end());
+    for (auto &x : v) {
+      if (!ve.empty() && vb.size() > iv_off.back() && x.first - 1 <= ve.back()) ve.back() = std::max<long long>(ve.back(), x.second);
+      else { vb.push_back(x.first); ve.push_back(x.second); }
+    }
+    iv_off.push_back((uint32_t)vb.size());
+  }
+  uint32_t slots = 2;
+  while (slots < 2 * names.size()) slots *= 2;  // at most half full: a probe always ends at an empty slot
+  std::vector<int32_t> slot(slots, -1);
+  for (size_t c = 0; c < names.size(); c++) {
+    uint32_t h = region_hash((const uint8_t *)names[c].data(), (uint32_t)names[c].size()) & (slots - 1);
+    while (slot[h] >= 0) h = (h + 1) & (slots - 1);
+    slot[h] = (int32_t)c;
+  }
+  int rc;
+  auto put = [&](DevBuf &b, const void *src, size_t bytes) -> int {
+    int r;
+    if ((r = dev_reserve(ctx, b, bytes))) return r;
+    CK(cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice));
+    return 0;
+  };
+  if ((rc = put(ctx->d_rgn_names, blob.data(), blob.size())) || (rc = put(ctx->d_rgn_name_off, name_off.data(), name_off.size() * 4)) ||
+      (rc = put(ctx->d_rgn_slot, slot.data(), slot.size() * 4)) || (rc = put(ctx->d_rgn_iv_off, iv_off.data(), iv_off.size() * 4)) ||
+      (rc = put(ctx->d_rgn_beg, vb.data(), vb.size() * 8)) || (rc = put(ctx->d_rgn_end, ve.data(), ve.size() * 8)))
+    return rc;
+  RegionTable &t = ctx->rgn;
+  t.names = (const uint8_t *)ctx->d_rgn_names.p; t.name_off = (const uint32_t *)ctx->d_rgn_name_off.p;
+  t.slot = (const int32_t *)ctx->d_rgn_slot.p; t.hash_mask = slots - 1;
+  t.iv_off = (const uint32_t *)ctx->d_rgn_iv_off.p;
+  t.beg = (const long long *)ctx->d_rgn_beg.p; t.end = (const long long *)ctx->d_rgn_end.p;
+  ctx->n_regions = vb.size();
   return BVCF_OK;
 }
 
@@ -1289,12 +1380,13 @@ int bvcf_resident_line_index(bvcf_ctx *ctx, uint64_t *starts, uint32_t *lens, ui
                              size_t *n_records) {
   if (!ctx) return BVCF_E_ARG;
   cudaSetDevice(ctx->device);
-  // valid for single-sub-chunk runs: the dense table of the last sub-chunk
+  // valid for single-sub-chunk runs: the dense table of the last sub-chunk (with regions set, its kept records)
   const size_t n = (size_t)std::min<uint64_t>(ctx->res.h_ctr->chunk_records, cap);
   if (n_records) *n_records = ctx->res.h_ctr->chunk_records;
   if (n == 0) return BVCF_OK;
   std::vector<LineRec> tmp(n);
-  CK(cudaMemcpy(tmp.data(), ctx->res.sc.dense.p, n * sizeof(LineRec), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(tmp.data(), (ctx->n_regions ? ctx->res.sc.kept : ctx->res.sc.dense).p, n * sizeof(LineRec),
+                cudaMemcpyDeviceToHost));
   for (size_t i = 0; i < n; i++) {
     if (starts) starts[i] = tmp[i].start;
     if (lens) lens[i] = tmp[i].len;

@@ -51,6 +51,10 @@ struct Config {  // main.go:63-80
   size_t chunkBytes = 64u << 20;
   bool bgzfOut = false;  // --bgzfOut: the rows leave as bgzf blocks deflated on the GPU (the `| pigz -c` of README.md:10,71)
   int bgzfLevel = 1;     // --bgzfLevel N: 1..9 as `bgzip -l` / `pigz -N` take it (bvcf_resident_download_bgzf_level)
+  // --regions / --regionsFile: only the records inside these (contig, 1-based inclusive [beg, end]) are transformed
+  bool regionsSet = false;
+  std::vector<std::string> regionChrom;
+  std::vector<int64_t> regionBeg, regionEnd;
 };
 
 std::string trim(const std::string &s) {  // strings.TrimSpace
@@ -116,6 +120,82 @@ bool go_int(const std::string &s, long long *out) {
   return true;
 }
 
+// a decimal number of 0..2^63-1 (no sign): what --regions and --regionsFile positions are
+bool pos_int(const std::string &s, int64_t *out) {
+  if (s.empty() || s.size() > 19) return false;
+  unsigned long long v = 0;
+  for (char ch : s) {
+    if (ch < '0' || ch > '9') return false;
+    v = v * 10 + (unsigned)(ch - '0');
+  }
+  if (v > (unsigned long long)INT64_MAX) return false;
+  *out = (int64_t)v;
+  return true;
+}
+
+// --regions chr|chr:pos|chr:beg-end|chr:beg-[,...] (bcftools -r): the position part follows the last ':'
+void parse_regions(const std::string &arg, Config &c) {
+  size_t p = 0;
+  for (;;) {
+    const size_t q = arg.find(',', p);
+    const std::string item = arg.substr(p, q == std::string::npos ? std::string::npos : q - p);
+    auto bad = [&]() { fatal("--regions: malformed region \"" + item + "\""); };
+    if (item.empty()) bad();
+    const size_t colon = item.rfind(':');
+    std::string chrom = item;
+    int64_t beg = 1, end = INT64_MAX;
+    if (colon != std::string::npos) {
+      chrom = item.substr(0, colon);
+      const std::string r = item.substr(colon + 1);
+      const size_t dash = r.find('-');
+      if (dash == std::string::npos) {
+        if (!pos_int(r, &beg)) bad();
+        end = beg;
+      } else {
+        if (!pos_int(r.substr(0, dash), &beg)) bad();
+        if (dash + 1 < r.size() && !pos_int(r.substr(dash + 1), &end)) bad();
+      }
+      if (beg < 1 || beg > end) bad();
+    }
+    if (chrom.empty()) bad();
+    c.regionChrom.push_back(chrom); c.regionBeg.push_back(beg); c.regionEnd.push_back(end);
+    if (q == std::string::npos) break;
+    p = q + 1;
+  }
+}
+
+// --regionsFile: BED (0-based, half-open): "#", "track" and "browser" lines and blank lines are skipped, columns past the
+// third are ignored; an empty interval holds no position
+void parse_regions_file(const std::string &path, Config &c) {
+  FILE *f = fopen(path.c_str(), "r");
+  if (!f) fatal("--regionsFile: " + path + ": " + strerror(errno));
+  std::string line;
+  size_t line_no = 0;
+  for (int ch = 0; ch != EOF;) {
+    line.clear();
+    while ((ch = fgetc(f)) != EOF && ch != '\n') line += (char)ch;
+    line_no++;
+    if (!line.empty() && line.back() == '\r') line.pop_back();
+    std::vector<std::string> col;
+    for (size_t i = 0; i < line.size();) {
+      while (i < line.size() && (line[i] == '\t' || line[i] == ' ')) i++;
+      size_t j = i;
+      while (j < line.size() && line[j] != '\t' && line[j] != ' ') j++;
+      if (j > i) col.push_back(line.substr(i, j - i));
+      i = j;
+    }
+    if (col.empty() || col[0][0] == '#' || col[0] == "track" || col[0] == "browser") continue;
+    int64_t b, e;
+    const std::string where = "--regionsFile: " + path + " line " + std::to_string(line_no) + ": ";
+    if (col.size() < 3) { fclose(f); fatal(where + "fewer than three columns"); }
+    if (!pos_int(col[1], &b) || !pos_int(col[2], &e)) { fclose(f); fatal(where + "start and end must be non-negative integers"); }
+    if (b > e) { fclose(f); fatal(where + "start > end"); }
+    if (b == e) continue;
+    c.regionChrom.push_back(col[0]); c.regionBeg.push_back(b + 1); c.regionEnd.push_back(e);
+  }
+  fclose(f);
+}
+
 // Go `flag` syntax: -x / --x, --x=v / --x v; bool flags --x or --x=true|false; stops at the first non-flag.
 Config setup(int argc, char **argv) {  // main.go:82-126
   Config c;
@@ -130,6 +210,7 @@ Config setup(int argc, char **argv) {  // main.go:82-126
                    {"keepInfo", &c.keepInfo}, {"bgzfOut", &c.bgzfOut}};
   std::string gpus, chunk, devices, level;
   bool level_given = false;
+  std::vector<std::pair<bool, std::string>> regions;  // (is a file, value) in flag order
   for (int i = 1; i < argc; i++) {
     std::string s = argv[i];
     if (s.size() < 2 || s[0] != '-') break;
@@ -155,6 +236,10 @@ Config setup(int argc, char **argv) {  // main.go:82-126
     if (name == "chunkBytes") dst = &chunk;   // extension: host chunk size
     if (name == "devices") dst = &devices;    // extension: explicit CUDA device per worker
     if (name == "bgzfLevel") { dst = &level; level_given = true; }  // extension: --bgzfOut's compression level
+    if (name == "regions" || name == "regionsFile") {  // extension: region selection
+      regions.push_back({name == "regionsFile", ""});
+      dst = &regions.back().second;
+    }
     if (!dst) fatal("flag provided but not defined: -" + name);
     if (!has_val) {
       if (++i >= argc) fatal("flag needs an argument: -" + name);
@@ -178,6 +263,12 @@ Config setup(int argc, char **argv) {  // main.go:82-126
     if (!c.bgzfOut) fatal("--bgzfLevel needs --bgzfOut");
     c.bgzfLevel = (int)v;
   }
+  for (auto &r : regions) {
+    if (r.first) parse_regions_file(r.second, c);
+    else parse_regions(r.second, c);
+  }
+  if (!regions.empty() && c.regionChrom.empty()) fatal("--regionsFile: no intervals");
+  c.regionsSet = !regions.empty();
   return c;
 }
 
@@ -593,6 +684,77 @@ void plan_bgzf_groups(BgzfIn &in, uint64_t data_off, size_t chunk_bytes, size_t 
   }
 }
 
+// What a run reads: the input from its data lines on -- or, with regions and a tabix / CSI index beside a bgzf input, the
+// index's spans only.  A span [vbeg, vend) is a view of the mapped file from the block of vbeg to the end of the block of
+// vend, its data lines from vbeg's offset into that first block on; the records after vend in its last block and the
+// lines between two regions inside one span are dropped by the GPU's region filter.  Both drivers read these pieces
+// through BgzfIn, the streaming one cut into groups by plan_bgzf_groups.
+struct Piece {
+  Input *in;
+  BgzfIn *gz;        // null: plain text
+  uint64_t data_off;  // text offset of the first data line
+};
+struct IndexedInput {
+  std::vector<std::unique_ptr<Input>> views;
+  std::vector<std::unique_ptr<BgzfIn>> gz;
+  std::vector<Piece> pieces;
+};
+
+// the index file (`<in>.tbi`, else `<in>.csi`) inflated, or empty when there is none
+std::string read_index(const std::string &in_path, std::string *which) {
+  for (const char *ext : {".tbi", ".csi"}) {
+    *which = in_path + ext;
+    if (access(which->c_str(), F_OK) != 0) continue;
+    gzFile f = gzopen(which->c_str(), "rb");
+    if (!f) fatal(*which + ": " + strerror(errno));
+    std::string out;
+    char buf[1 << 16];
+    int n;
+    while ((n = gzread(f, buf, sizeof buf)) > 0) out.append(buf, (size_t)n);
+    if (n < 0) fatal(*which + ": not a gzip file");
+    gzclose(f);
+    return out;
+  }
+  return std::string();
+}
+
+// the pieces of a mapped bgzf input that the index of `c.inPath` gives for c's regions; false when there is no index
+bool index_pieces(const Config &c, const uint8_t *map, size_t map_len, IndexedInput &out) {
+  std::string path;
+  const std::string idx = read_index(c.inPath, &path);
+  if (idx.empty()) return false;
+  std::vector<const char *> names;
+  for (auto &s : c.regionChrom) names.push_back(s.c_str());
+  std::vector<uint64_t> sp(2 * 1024);
+  size_t n = 0;
+  int rc = bvcf_index_spans(idx.data(), idx.size(), names.data(), c.regionBeg.data(), c.regionEnd.data(), names.size(),
+                            sp.data(), sp.size() / 2, &n);
+  if (rc == BVCF_E_TOO_LARGE) {
+    sp.resize(2 * n);
+    rc = bvcf_index_spans(idx.data(), idx.size(), names.data(), c.regionBeg.data(), c.regionEnd.data(), names.size(),
+                          sp.data(), n, &n);
+  }
+  if (rc) fatal(path + ": " + bvcf_strerror(rc) + " (not a tabix or CSI index)");
+  auto block_at = [&](uint64_t off) {  // a bgzf block starts at compressed offset off: its size
+    const long long bs = off < map_len ? bgzf_header(map + off, map_len - off) : 0;
+    if (bs <= 0 || off + (uint64_t)bs > map_len)
+      fatal(path + ": virtual offset " + std::to_string(off) + " << 16 is not a bgzf block of " + c.inPath);
+    return (uint64_t)bs;
+  };
+  for (size_t k = 0; k < n; k++) {
+    const uint64_t cb = sp[2 * k] >> 16, ce = sp[2 * k + 1] >> 16, ue = sp[2 * k + 1] & 0xFFFF;
+    block_at(cb);
+    const uint64_t end = ue ? ce + block_at(ce) : ce;
+    if (end < ce || end > map_len || (ce < map_len && !ue && ce != cb && bgzf_header(map + ce, map_len - ce) <= 0))
+      fatal(path + ": virtual offset " + std::to_string(ce) + " << 16 is not a bgzf block of " + c.inPath);
+    if (end <= cb) continue;
+    out.views.emplace_back(new Input(-1, map + cb, (size_t)(end - cb), {}));
+    out.gz.emplace_back(new BgzfIn(*out.views.back()));
+    out.pieces.push_back({out.views.back().get(), out.gz.back().get(), sp[2 * k] & 0xFFFF});
+  }
+  return true;
+}
+
 // Where the results of a run go (main.go:296-343, 398-445): the rows to the output, the dosage batches to the Arrow
 // file.  Built once from the #CHROM line: it writes the sample list and opens the dosage file -- or, when the VCF has no
 // samples, writes an empty one and asks for no dosage work.
@@ -679,13 +841,19 @@ bvcf_ctx *open_ctx(const Config &c, int device, const Preamble &pre, bool want_d
   int rc = bvcf_create(&ctx, device, &bc);
   if (rc) fatal(std::string("bvcf_create(gpu ") + std::to_string(device) + "): " + bvcf_strerror(rc) + " -- a CUDA device is required, there is no CPU fallback");
   if ((rc = bvcf_set_header(ctx, pre.chrom_line.data(), pre.chrom_line.size()))) fatal(std::string("bvcf_set_header: ") + bvcf_strerror(rc));
+  if (c.regionsSet) {
+    std::vector<const char *> names;
+    for (auto &s : c.regionChrom) names.push_back(s.c_str());
+    if ((rc = bvcf_set_regions(ctx, names.data(), c.regionBeg.data(), c.regionEnd.data(), names.size())))
+      fatal(std::string("bvcf_set_regions: ") + bvcf_strerror(rc));
+  }
   return ctx;
 }
 
 // readVcf for --bgzfOut: the rows are deflated where they are made, so the input goes through one GPU's resident
 // regions a group at a time -- plain text uploaded, or whole bgzf blocks inflated there (bvcf_resident_inflate_bgzf).
-// The partial line at a group's end is carried into the next group.
-void run_resident(const Config &config, Input &in, BgzfIn *gz, const Preamble &pre, Sink &sink) {
+// The partial line at a group's end is carried into the next group; the one at a piece's end is dropped.
+void run_resident(const Config &config, const std::vector<Piece> &pieces, const Preamble &pre, Sink &sink) {
   bvcf_ctx *ctx = open_ctx(config, config.devices.empty() ? 0 : config.devices[0], pre, sink.want_dosage(), 0, 0);
   int rc;
   const size_t batch_text = std::max<size_t>(config.chunkBytes * 8, 64u << 20), max_line = 8u << 20;
@@ -695,84 +863,89 @@ void run_resident(const Config &config, Input &in, BgzfIn *gz, const Preamble &p
   uint8_t *pin = nullptr, *out_host = nullptr;   // pinned: group in, compressed rows out
   size_t pin_cap = 0, out_cap = 0;
   std::vector<uint8_t> carry, tail;
-  // the first group starts at the data lines (plain) or at the block that holds their first byte (bgzf); `begin` is
-  // where they start in it
-  size_t pos = pre.data_off, b = 0, begin = 0;
-  if (gz && gz->has(b = gz->block_at(pre.data_off))) begin = pre.data_off - (*gz)[b].start;
-  for (;;) {
-    // ---- a group: whole blocks worth about batch_text bytes of text, or batch_text bytes of plain text ----
-    size_t lo = pos, hi;
-    if (gz) {
-      size_t e = b;
-      for (uint64_t text = 0; text < batch_text && gz->has(e); e++) text += (*gz)[e].isize;
-      lo = gz->off(b); hi = gz->off(e);  // blocks without text in between go along
-      b = e;
-    } else {
-      in.fill(pos + batch_text);
-      hi = pos = std::min(in.end(), pos + batch_text);
-    }
-    if (hi == lo) break;
-    if (hi - lo > pin_cap) {
-      if (pin) bvcf_host_free(pin);
-      pin_cap = (hi - lo) + (hi - lo) / 4;
-      if (bvcf_host_alloc((void **)&pin, pin_cap)) fatal("bvcf_host_alloc failed");
-    }
-    memcpy(pin, in.at(lo), hi - lo);
-    in.release_before(hi);
-    if (!carry.empty() && (rc = bvcf_resident_upload(ctx, 0, carry.data(), carry.size()))) fatal(std::string("upload: ") + bvcf_strerror(rc));
-    size_t n_text = hi - lo;
-    if (gz) {
-      if ((rc = bvcf_resident_inflate_bgzf(ctx, pin, hi - lo, carry.size(), &n_text)))
-        fatal(std::string("bgzf: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
-    } else if ((rc = bvcf_resident_upload(ctx, carry.size(), pin, hi - lo))) {
-      fatal(std::string("upload: ") + bvcf_strerror(rc));
-    }
-    const size_t total = carry.size() + n_text;
-    // ---- the longest newline-terminated prefix; the rest is carried into the next group ----
-    const size_t tail_n = std::min(total - begin, max_line);
-    tail.resize(tail_n);
-    if (tail_n && (rc = bvcf_resident_peek(ctx, total - tail_n, tail.data(), tail_n))) fatal(std::string("peek: ") + bvcf_strerror(rc));
-    const uint8_t *last_nl = tail_n ? (const uint8_t *)memrchr(tail.data(), '\n', tail_n) : nullptr;
-    if (!last_nl) {
-      if (tail_n < total - begin) fatal("a single line exceeds 8 MiB");
-      carry.assign(tail.begin(), tail.end());  // no complete line yet: everything is carried
-      begin = 0;
-      continue;
-    }
-    const size_t end = total - tail_n + (size_t)(last_nl - tail.data()) + 1;
-    bvcf_chunk_stats st{};
-    if ((rc = bvcf_resident_run_at(ctx, begin, end, &st, nullptr))) fatal(std::string("bvcf_resident_run: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
-    if (!config.noOut && st.out_bytes) {
-      if (st.out_bytes > out_cap) {
-        if (out_host) bvcf_host_free(out_host);
-        out_cap = st.out_bytes + st.out_bytes / 4;
-        if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
+  for (const Piece &piece : pieces) {
+    Input &in = *piece.in;
+    BgzfIn *gz = piece.gz;
+    carry.clear();
+    // the first group starts at the data lines (plain) or at the block that holds their first byte (bgzf); `begin` is
+    // where they start in it
+    size_t pos = piece.data_off, b = 0, begin = 0;
+    if (gz && gz->has(b = gz->block_at(piece.data_off))) begin = piece.data_off - (*gz)[b].start;
+    for (;;) {
+      // ---- a group: whole blocks worth about batch_text bytes of text, or batch_text bytes of plain text ----
+      size_t lo = pos, hi;
+      if (gz) {
+        size_t e = b;
+        for (uint64_t text = 0; text < batch_text && gz->has(e); e++) text += (*gz)[e].isize;
+        lo = gz->off(b); hi = gz->off(e);  // blocks without text in between go along
+        b = e;
+      } else {
+        in.fill(pos + batch_text);
+        hi = pos = std::min(in.end(), pos + batch_text);
       }
-      size_t comp = 0;
-      rc = bvcf_resident_download_bgzf_level(ctx, 0, st.out_bytes, config.bgzfLevel, out_host, out_cap, &comp);
-      if (rc == BVCF_E_TOO_LARGE) {  // comp: the bytes needed
-        bvcf_host_free(out_host);
-        out_cap = comp + comp / 8;
-        if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
+      if (hi == lo) break;
+      if (hi - lo > pin_cap) {
+        if (pin) bvcf_host_free(pin);
+        pin_cap = (hi - lo) + (hi - lo) / 4;
+        if (bvcf_host_alloc((void **)&pin, pin_cap)) fatal("bvcf_host_alloc failed");
+      }
+      memcpy(pin, in.at(lo), hi - lo);
+      in.release_before(hi);
+      if (!carry.empty() && (rc = bvcf_resident_upload(ctx, 0, carry.data(), carry.size()))) fatal(std::string("upload: ") + bvcf_strerror(rc));
+      size_t n_text = hi - lo;
+      if (gz) {
+        if ((rc = bvcf_resident_inflate_bgzf(ctx, pin, hi - lo, carry.size(), &n_text)))
+          fatal(std::string("bgzf: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
+      } else if ((rc = bvcf_resident_upload(ctx, carry.size(), pin, hi - lo))) {
+        fatal(std::string("upload: ") + bvcf_strerror(rc));
+      }
+      const size_t total = carry.size() + n_text;
+      // ---- the longest newline-terminated prefix; the rest is carried into the next group ----
+      const size_t tail_n = std::min(total - begin, max_line);
+      tail.resize(tail_n);
+      if (tail_n && (rc = bvcf_resident_peek(ctx, total - tail_n, tail.data(), tail_n))) fatal(std::string("peek: ") + bvcf_strerror(rc));
+      const uint8_t *last_nl = tail_n ? (const uint8_t *)memrchr(tail.data(), '\n', tail_n) : nullptr;
+      if (!last_nl) {
+        if (tail_n < total - begin) fatal("a single line exceeds 8 MiB");
+        carry.assign(tail.begin(), tail.end());  // no complete line yet: everything is carried
+        begin = 0;
+        continue;
+      }
+      const size_t end = total - tail_n + (size_t)(last_nl - tail.data()) + 1;
+      bvcf_chunk_stats st{};
+      if ((rc = bvcf_resident_run_at(ctx, begin, end, &st, nullptr))) fatal(std::string("bvcf_resident_run: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
+      if (!config.noOut && st.out_bytes) {
+        if (st.out_bytes > out_cap) {
+          if (out_host) bvcf_host_free(out_host);
+          out_cap = st.out_bytes + st.out_bytes / 4;
+          if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
+        }
+        size_t comp = 0;
         rc = bvcf_resident_download_bgzf_level(ctx, 0, st.out_bytes, config.bgzfLevel, out_host, out_cap, &comp);
+        if (rc == BVCF_E_TOO_LARGE) {  // comp: the bytes needed
+          bvcf_host_free(out_host);
+          out_cap = comp + comp / 8;
+          if (bvcf_host_alloc((void **)&out_host, out_cap)) fatal("bvcf_host_alloc failed");
+          rc = bvcf_resident_download_bgzf_level(ctx, 0, st.out_bytes, config.bgzfLevel, out_host, out_cap, &comp);
+        }
+        if (rc) fatal(std::string("download: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
+        sink.rows(out_host, comp);
       }
-      if (rc) fatal(std::string("download: ") + bvcf_strerror(rc) + " " + bvcf_last_error(ctx));
-      sink.rows(out_host, comp);
-    }
-    {  // dosage batch and diagnostics of this group
-      bvcf_dosage_batch dos{};
-      const bvcf_diag *dg = nullptr;
-      size_t nd = 0;
-      if ((rc = bvcf_resident_results(ctx, sink.want_dosage() ? &dos : nullptr, &dg, &nd))) fatal(std::string("results: ") + bvcf_strerror(rc));
-      sink.dosage(dos);
-      char line[4096];
-      for (size_t k = 0; k < nd; k++) {
-        const size_t n = std::min<size_t>(sizeof line, end - dg[k].line_start);
-        if (dg[k].line_start < end && !bvcf_resident_peek(ctx, dg[k].line_start, line, n)) log_one_diag(line, n, dg[k]);
+      {  // dosage batch and diagnostics of this group
+        bvcf_dosage_batch dos{};
+        const bvcf_diag *dg = nullptr;
+        size_t nd = 0;
+        if ((rc = bvcf_resident_results(ctx, sink.want_dosage() ? &dos : nullptr, &dg, &nd))) fatal(std::string("results: ") + bvcf_strerror(rc));
+        sink.dosage(dos);
+        char line[4096];
+        for (size_t k = 0; k < nd; k++) {
+          const size_t n = std::min<size_t>(sizeof line, end - dg[k].line_start);
+          if (dg[k].line_start < end && !bvcf_resident_peek(ctx, dg[k].line_start, line, n)) log_one_diag(line, n, dg[k]);
+        }
       }
+      carry.assign(last_nl + 1, (const uint8_t *)tail.data() + tail_n);
+      begin = 0;
     }
-    carry.assign(last_nl + 1, (const uint8_t *)tail.data() + tail_n);
-    begin = 0;
   }
   // an unterminated last line (the carry) is dropped (main.go:354-357)
   sink.rows(BGZF_EOF, sizeof BGZF_EOF);
@@ -783,7 +956,8 @@ void run_resident(const Config &config, Input &in, BgzfIn *gz, const Preamble &p
 
 // readVcf on 1..N GPUs: a reader cuts the input into chunks (newline-aligned text, or groups of whole bgzf blocks), chunk
 // k goes to GPU k mod N, and each GPU's worker hands its results to the sink when it is the chunk's turn
-void run_streaming(const Config &config, Input &in, BgzfIn *gz, const Preamble &pre, Sink &sink) {
+void run_streaming(const Config &config, const std::vector<Piece> &pieces, const Preamble &pre, Sink &sink) {
+  Input &in = *pieces[0].in;
   // ---- one context per GPU ----
   const int n_slots = 3;
   const size_t cap = 2 * config.chunkBytes + (64u << 20);  // a chunk grows until it holds a newline
@@ -855,22 +1029,26 @@ void run_streaming(const Config &config, Input &in, BgzfIn *gz, const Preamble &
 
   // ---- reader: newline-aligned chunks, chunk k to GPU k mod N ----
   uint64_t seq = 0;
-  if (gz) {  // groups of whole bgzf blocks: a mapped input is staged by the workers, a pipe's by the reader
-    plan_bgzf_groups(*gz, pre.data_off, config.chunkBytes, cap, [&](size_t lo_b, size_t hi_b, size_t skip, const std::string &tail) {
-      const size_t lo = gz->off(lo_b), hi = gz->off(hi_b);
-      if (hi - lo > cap) fatal("a bgzf group exceeds the chunk capacity; raise --chunkBytes");
-      Chunk c;
-      c.seq = seq; c.len = hi - lo; c.gz = true; c.skip = skip; c.tail = tail;
-      if (in.mapped()) {
-        c.src = in.at(lo);
-      } else {
-        c.buf = pools[seq % n_gpu].take();
-        memcpy(c.buf, in.at(lo), c.len);
-        in.release_before(hi);
-      }
-      queues[seq % n_gpu]->push(std::move(c));
-      seq++;
-    });
+  if (pieces[0].gz) {  // groups of whole bgzf blocks: a mapped input is staged by the workers, a pipe's by the reader
+    for (const Piece &piece : pieces) {
+      Input &in = *piece.in;
+      BgzfIn *gz = piece.gz;
+      plan_bgzf_groups(*gz, piece.data_off, config.chunkBytes, cap, [&](size_t lo_b, size_t hi_b, size_t skip, const std::string &tail) {
+        const size_t lo = gz->off(lo_b), hi = gz->off(hi_b);
+        if (hi - lo > cap) fatal("a bgzf group exceeds the chunk capacity; raise --chunkBytes");
+        Chunk c;
+        c.seq = seq; c.len = hi - lo; c.gz = true; c.skip = skip; c.tail = tail;
+        if (in.mapped()) {
+          c.src = in.at(lo);
+        } else {
+          c.buf = pools[seq % n_gpu].take();
+          memcpy(c.buf, in.at(lo), c.len);
+          in.release_before(hi);
+        }
+        queues[seq % n_gpu]->push(std::move(c));
+        seq++;
+      });
+    }
   } else if (in.mapped()) {
     const uint8_t *map = in.at(0);
     size_t p = pre.data_off;
@@ -1009,8 +1187,15 @@ int main(int argc, char **argv) {
   }
 
   Sink sink(config, out_fd, pre.chrom_line);
-  if (config.bgzfOut) run_resident(config, in, gz.get(), pre, sink);
-  else run_streaming(config, in, gz.get(), pre, sink);
+  IndexedInput indexed;
+  if (!(config.regionsSet && gz && map && index_pieces(config, map, map_len, indexed)))
+    indexed.pieces.push_back({&in, gz.get(), pre.data_off});
+  if (!indexed.pieces.empty()) {
+    if (config.bgzfOut) run_resident(config, indexed.pieces, pre, sink);
+    else run_streaming(config, indexed.pieces, pre, sink);
+  } else if (config.bgzfOut) {
+    sink.rows(BGZF_EOF, sizeof BGZF_EOF);  // no span: no rows
+  }
   const int rc_exit = sink.close();
   if (map) munmap((void *)map, map_len);
   if (out_fd != 1) close(out_fd);

@@ -14,7 +14,7 @@ from __future__ import annotations
 import ctypes as C
 import re
 from dataclasses import dataclass, field
-from typing import BinaryIO, Dict, List, Optional, Sequence
+from typing import BinaryIO, Dict, List, Optional, Sequence, Tuple
 
 from . import _lib
 from ._lib import BvcfError, CChunkStats, CConfig, CDiag, CDosageBatch, CKernelTimes, check
@@ -82,14 +82,70 @@ class Config:
     # --bgzfLevel N: how hard the GPU deflates those rows, 1..9 as `bgzip -l` / `pigz -N` take it; 1 is the fast
     # single-candidate kernel with fixed codes, 2..9 search more and write dynamic Huffman codes
     bgzfLevel: int = 1
+    # --regions / --regionsFile: only the records inside these (contig, 1-based inclusive beg, end) are transformed; None:
+    # every record (bvcf_set_regions)
+    regions: Optional[List[Tuple[bytes, int, int]]] = None
 
 
 _STRING_FLAGS = {"in": "inPath", "fam": "famPath", "err": "errPath", "out": "outPath", "dosageOutput": "dosageMatrixOutPath",
                  "sample": "sampleListPath", "emptyField": "emptyField", "fieldDelimiter": "fieldDelimiter",
-                 "cpuProfile": "cpuProfile", "allowFilter": None, "excludeFilter": None}
+                 "cpuProfile": "cpuProfile", "allowFilter": None, "excludeFilter": None, "regions": None,
+                 "regionsFile": None}
 _BOOL_FLAGS = {"noOut": "noOut", "keepId": "keepID", "keepQual": "keepQual", "keepPos": "keepPos", "keepInfo": "keepInfo",
                "bgzfOut": "bgzfOut"}
 _INT_FLAGS = {"bgzfLevel": "bgzfLevel"}
+REGION_MAX = (1 << 63) - 1  # the end of an open region ("chr", "chr:beg-")
+
+
+def _pos_int(s: str) -> Optional[int]:
+    """a decimal number of 0..2^63-1 without a sign, or None"""
+    return int(s) if s and len(s) <= 19 and s.isascii() and s.isdigit() and int(s) <= REGION_MAX else None
+
+
+def parse_regions(arg: str) -> List[Tuple[bytes, int, int]]:
+    """--regions chr|chr:pos|chr:beg-end|chr:beg-[,...] (bcftools -r): 1-based inclusive (contig, beg, end); the position
+    part follows the last ':'.  ValueError on a malformed item."""
+    out = []
+    for item in arg.split(","):
+        chrom, beg, end = item, 1, REGION_MAX
+        if ":" in item:
+            chrom, r = item.rsplit(":", 1)
+            b, dash, e = r.partition("-")
+            beg = _pos_int(b)
+            end = beg if not dash else (REGION_MAX if e == "" else _pos_int(e))
+            if beg is None or end is None or beg < 1 or beg > end:
+                chrom = ""
+        if not chrom:
+            raise ValueError(f'--regions: malformed region "{item}"')
+        out.append((chrom.encode(), beg, end))
+    return out
+
+
+def read_regions_file(path: str) -> List[Tuple[bytes, int, int]]:
+    """--regionsFile: BED (0-based, half-open) -> 1-based inclusive (contig, beg, end).  "#", "track" and "browser" lines
+    and blank lines are skipped, columns past the third are ignored; an empty interval holds no position.  ValueError on
+    an unreadable file, a line with fewer than three columns or start > end."""
+    try:
+        with open(path, "rb") as f:
+            data = f.read()
+    except OSError as e:
+        raise ValueError(f"--regionsFile: {path}: {e.strerror}") from None
+    out = []
+    for no, line in enumerate(data.split(b"\n"), 1):
+        col = line.rstrip(b"\r").replace(b"\t", b" ").split()
+        if not col or col[0].startswith(b"#") or col[0] in (b"track", b"browser"):
+            continue
+        where = f"--regionsFile: {path} line {no}: "
+        if len(col) < 3:
+            raise ValueError(where + "fewer than three columns")
+        b, e = _pos_int(col[1].decode("latin-1")), _pos_int(col[2].decode("latin-1"))
+        if b is None or e is None:
+            raise ValueError(where + "start and end must be non-negative integers")
+        if b > e:
+            raise ValueError(where + "start > end")
+        if b < e:
+            out.append((col[0], b + 1, e))
+    return out
 
 
 def _go_int(val: str) -> Optional[int]:
@@ -114,6 +170,7 @@ def setup(args: Optional[Sequence[str]] = None) -> Config:
     cfg = Config()
     allow, exclude = "PASS,.", ""
     level_given = False
+    regions = None
     i = 0
     while i < len(a):
         s = a[i]
@@ -156,7 +213,9 @@ def setup(args: Optional[Sequence[str]] = None) -> Config:
                 if i >= len(a):
                     raise ValueError(f"flag needs an argument: -{name}")
                 val = a[i]
-            if name == "allowFilter":
+            if name in ("regions", "regionsFile"):
+                regions = (regions or []) + (read_regions_file(val) if name == "regionsFile" else parse_regions(val))
+            elif name == "allowFilter":
                 allow = val
             elif name == "excludeFilter":
                 exclude = val
@@ -173,6 +232,9 @@ def setup(args: Optional[Sequence[str]] = None) -> Config:
         raise ValueError(f"--bgzfLevel must be 1..9, not {cfg.bgzfLevel}")
     if level_given and not cfg.bgzfOut:
         raise ValueError("--bgzfLevel needs --bgzfOut")
+    if regions is not None and not regions:
+        raise ValueError("--regionsFile: no intervals")
+    cfg.regions = regions
     return cfg
 
 
@@ -295,6 +357,16 @@ class Transformer:
         check(self._L.bvcf_set_header(self._ctx, chrom_line, len(chrom_line)), self._ctx, "bvcf_set_header")
         n = len(chrom_line.rstrip(b"\r\n").split(b"\t"))
         self.n_samples = max(n - 9, 0)
+
+    def set_regions(self, regions: Optional[Sequence[Tuple[bytes, int, int]]]) -> None:
+        """Only the records inside these (contig, 1-based inclusive beg, end) are transformed, on both paths
+        (bvcf_set_regions); None or an empty list: every record."""
+        regions = list(regions or [])
+        n = len(regions)
+        names = (C.c_char_p * max(n, 1))(*[c.encode() if isinstance(c, str) else bytes(c) for c, _, _ in regions])
+        beg = (C.c_int64 * max(n, 1))(*[b for _, b, _ in regions])
+        end = (C.c_int64 * max(n, 1))(*[e for _, _, e in regions])
+        check(self._L.bvcf_set_regions(self._ctx, names, beg, end, n), self._ctx, "bvcf_set_regions")
 
     # -- streaming path ---------------------------------------------------------------------------
     def submit(self, seq: int, chunk) -> None:
@@ -625,66 +697,83 @@ def _read_vcf_resident(config: Config, head: bytes, reader: BinaryIO, writer: Op
 
     compressed_bytes = in_bytes = 0
     max_line = 8 << 20  # room for the carried partial line
+    # what is read: the input from its data lines on, or -- with regions and an index beside a bgzf file -- the index's
+    # spans (bgzf.index_views), each from its first block to its last; a partial line at a span's end is dropped
+    sources = [(buf, data_off)]
+    if gz and config.regions and config.inPath:
+        import mmap
+
+        with open(config.inPath, "rb") as f:
+            whole = mmap.mmap(f.fileno(), 0, access=mmap.ACCESS_READ)
+        try:
+            views = bgzf.index_views(whole, config.inPath, config.regions)
+        except ValueError as e:
+            raise BvcfError(str(e)) from None
+        if views is not None:
+            sources = [(bytearray(whole[lo:hi]), skip) for lo, hi, skip in views]
+            eof = True
     sink = Sink(config, chrom_line, writer, diag_sink)
     try:
         with Transformer(config, eol_width=width) as tr:
             tr.set_header(chrom_line)
+            if config.regions is not None:
+                tr.set_regions(config.regions)
             tr.resident_alloc(batch_text + max_line + (1 << 20), batch_text // 4 + (64 << 20))
-            carry = b""
-            begin = data_off  # the first group holds the meta lines and the header: they are skipped on the device
-            while True:
-                # ---- a group: whole blocks worth about batch_text bytes of text, or batch_text bytes of plain text ----
-                p = text = 0
-                if not gz:
-                    fill(batch_text)
-                    p = min(len(buf), batch_text)
-                while gz and text < batch_text:
-                    fill(p + (1 << 16) + 18)
-                    bs = bgzf.block_size(buf, p)
-                    if bs == 0 or p + bs > len(buf):
-                        if not eof:
-                            fill(p + max(bs, 1 << 16) + 18)
-                            continue
-                        if p < len(buf):
-                            raise BvcfError("bgzf input: truncated block at the end")
+            for buf, begin in sources:  # a source's first group holds what comes before its data lines: skipped on the device
+                carry = b""
+                while True:
+                    # ---- a group: whole blocks worth about batch_text bytes of text, or batch_text bytes of plain text ----
+                    p = text = 0
+                    if not gz:
+                        fill(batch_text)
+                        p = min(len(buf), batch_text)
+                    while gz and text < batch_text:
+                        fill(p + (1 << 16) + 18)
+                        bs = bgzf.block_size(buf, p)
+                        if bs == 0 or p + bs > len(buf):
+                            if not eof:
+                                fill(p + max(bs, 1 << 16) + 18)
+                                continue
+                            if p < len(buf):
+                                raise BvcfError("bgzf input: truncated block at the end")
+                            break
+                        text += int.from_bytes(buf[p + bs - 4:p + bs], "little")
+                        p += bs
+                    if p == 0:
                         break
-                    text += int.from_bytes(buf[p + bs - 4:p + bs], "little")
-                    p += bs
-                if p == 0:
-                    break
-                group = bytes(buf[:p])
-                del buf[:p]
-                if carry:
-                    tr.resident_upload(0, carry)
-                if gz:
-                    n_text = tr.resident_inflate_bgzf(group, len(carry))
-                else:
-                    tr.resident_upload(len(carry), group)
-                    n_text = len(group)
-                total = len(carry) + n_text
-                compressed_bytes += len(group)
-                # ---- the longest newline-terminated prefix; what follows it is carried into the next group ----
-                tail_n = min(total - begin, max_line)
-                tail = tr.resident_peek(total - tail_n, tail_n) if tail_n > 0 else b""
-                k = tail.rfind(b"\n")
-                if k < 0:
-                    if tail_n == total - begin:  # no complete line in this group at all
-                        carry = carry + tr.resident_peek(len(carry), n_text) if begin == 0 else tr.resident_peek(begin, total - begin)
-                        begin = 0
-                        continue
-                    raise BvcfError("a single line exceeds %d bytes" % max_line)
-                end = total - tail_n + k + 1
-                stats, _ = tr.resident_run(end, want_times=False, begin=begin)
-                rows = b""
-                if writer is not None and not config.noOut and stats["out_bytes"]:
-                    rows = tr.resident_download_bgzf(0, stats["out_bytes"], config.bgzfLevel)
-                loci, dosage, diags = tr.resident_results()
-                res = ChunkResult(tsv=rows, n_lines=stats["n_lines"], n_records=stats["n_records"], n_rows=stats["n_rows"],
-                                  diags=[d[:3] for d in diags], diag_starts=[d[3] for d in diags], loci=loci, dosage=dosage)
-                sink.put(res, (locus_at(tr.resident_peek(st, min(4096, end - st)), 0) for st in res.diag_starts))
-                in_bytes += end - begin
-                carry = tail[k + 1:]
-                begin = 0
+                    group = bytes(buf[:p])
+                    del buf[:p]
+                    if carry:
+                        tr.resident_upload(0, carry)
+                    if gz:
+                        n_text = tr.resident_inflate_bgzf(group, len(carry))
+                    else:
+                        tr.resident_upload(len(carry), group)
+                        n_text = len(group)
+                    total = len(carry) + n_text
+                    compressed_bytes += len(group)
+                    # ---- the longest newline-terminated prefix; what follows it is carried into the next group ----
+                    tail_n = min(total - begin, max_line)
+                    tail = tr.resident_peek(total - tail_n, tail_n) if tail_n > 0 else b""
+                    k = tail.rfind(b"\n")
+                    if k < 0:
+                        if tail_n == total - begin:  # no complete line in this group at all
+                            carry = carry + tr.resident_peek(len(carry), n_text) if begin == 0 else tr.resident_peek(begin, total - begin)
+                            begin = 0
+                            continue
+                        raise BvcfError("a single line exceeds %d bytes" % max_line)
+                    end = total - tail_n + k + 1
+                    stats, _ = tr.resident_run(end, want_times=False, begin=begin)
+                    rows = b""
+                    if writer is not None and not config.noOut and stats["out_bytes"]:
+                        rows = tr.resident_download_bgzf(0, stats["out_bytes"], config.bgzfLevel)
+                    loci, dosage, diags = tr.resident_results()
+                    res = ChunkResult(tsv=rows, n_lines=stats["n_lines"], n_records=stats["n_records"], n_rows=stats["n_rows"],
+                                      diags=[d[:3] for d in diags], diag_starts=[d[3] for d in diags], loci=loci, dosage=dosage)
+                    sink.put(res, (locus_at(tr.resident_peek(st, min(4096, end - st)), 0) for st in res.diag_starts))
+                    in_bytes += end - begin
+                    carry = tail[k + 1:]
+                    begin = 0
             # an unterminated last line (carry) is dropped (main.go:354-357)
     finally:
         sink.close()
@@ -715,6 +804,8 @@ def read_vcf(config: Config, reader: BinaryIO, writer: Optional[BinaryIO], diag_
     try:
         with Transformer(config, eol_width=width, max_chunk_bytes=cap) as tr:
             tr.set_header(chrom_line)
+            if config.regions is not None:
+                tr.set_regions(config.regions)
             ring = PinnedRing(tr.n_slots + 1, cap)
             seq_in = seq_out = 0
             pending = {}  # seq -> the chunk's text (a view of its ring buffer) while it is in flight

@@ -100,6 +100,8 @@ def _gpu_worker(cfg: Config, device: int, eol_width: int, chrom_line: bytes, dat
         ring = PinnedRing(n_slots + 1, cap)
         with Transformer(c, eol_width=eol_width, n_slots=n_slots, max_chunk_bytes=text_cap) as tr:
             tr.set_header(chrom_line)
+            if cfg.regions is not None:
+                tr.set_regions(cfg.regions)
             sub = col = 0
             while col < len(my_ids):
                 while sub < len(my_ids) and sub - col < n_slots:
@@ -145,7 +147,10 @@ def read_vcf_multi(config: Config, data, writer: Optional[BinaryIO], devices: Se
     width, chrom_line, off = read_preamble(data, gz)
     if gz:
         try:
-            chunks = bgzf.plan_groups(data, off, chunk_bytes, 2 * chunk_bytes + (64 << 20))
+            # with regions and an index beside the file, only the blocks of the index's spans are read
+            views = bgzf.index_views(data, config.inPath, config.regions) if config.regions and config.inPath else None
+            cap = 2 * chunk_bytes + (64 << 20)
+            chunks = bgzf.plan_groups(data, off, chunk_bytes, cap) if views is None else bgzf.plan_views(data, views, chunk_bytes, cap)
         except ValueError as e:
             raise BvcfError(str(e)) from None
         end = off + sum(g.text - g.skip + len(g.tail) for g in chunks)

@@ -100,7 +100,7 @@ typedef struct {
 /* per-kernel device time of the last resident run, CUDA events on the launching stream */
 typedef struct {
   float scan_ms;     /* bvcf_scan_genotype_kernel: newline/tab index + per-sample GT classify  (north-star kernels 1+3) */
-  float compact_ms;  /* line-table compaction + prefix sums */
+  float compact_ms;  /* line-table compaction + prefix sums (+ the region filter, with regions set) */
   float stats_ms;    /* bvcf_line_stats_kernel: het/hom/missing/ac/an per record (kernel 3, reduction half) */
   float rows_ms;     /* bvcf_tile_kernel: FILTER + getAlleles + row text, offsets by decoupled look-back, rows and short
                         sample-name lists written in one pass (kernels 2+4) */
@@ -124,6 +124,24 @@ int bvcf_header_line(const bvcf_config *cfg, char *buf, size_t cap);
 /* The "#CHROM\tPOS..." line, with or without its EOL (main.go:281-296,505-509): fixes the required
  * field count and uploads the (normalised) sample-name table. */
 int bvcf_set_header(bvcf_ctx *ctx, const char *chrom_line, size_t len);
+
+/* Regions (--regions / --regionsFile): only the records inside them are transformed, by both the streaming slots and the
+ * resident path.  Region i is contig chrom[i] (matched byte for byte against CHROM) and the 1-based inclusive positions
+ * [beg[i], end[i]]: a record is kept when its POS is 1 to 18 ASCII digits whose value lies in a region of its CHROM --
+ * bcftools view -t (targets) semantics: a deletion that starts before a region and reaches into it is not kept.  Other
+ * records give no row, no dosage row and no diagnostic, as if their lines were not in the input; line numbers and
+ * bvcf_chunk_stats' n_lines / n_records still count them.  The regions are copied (overlapping and adjacent ones
+ * merged); n == 0 clears them.  BVCF_E_ARG: a NULL or empty name, beg < 1 or beg > end.  BVCF_E_STATE: a chunk is in
+ * flight. */
+int bvcf_set_regions(bvcf_ctx *ctx, const char *const *chrom, const int64_t *beg, const int64_t *end, size_t n);
+
+/* Host only: the bgzf virtual-offset spans [spans[2k], spans[2k + 1]) that hold every record of the regions (given as to
+ * bvcf_set_regions) a tabix or CSI index knows of.  `index` is the index file after gzip decompression ("TBI\1" or
+ * "CSI\1"); the spans are sorted and disjoint, start and end at record boundaries, and may hold records outside the
+ * regions too (bvcf_set_regions drops those).  A contig the index does not list gives no span.  *n_spans receives the
+ * count; BVCF_E_TOO_LARGE when it is more than cap, BVCF_E_ARG on a malformed index or region. */
+int bvcf_index_spans(const void *index, size_t len, const char *const *chrom, const int64_t *beg, const int64_t *end,
+                     size_t n, uint64_t *spans, size_t cap, size_t *n_spans);
 
 /* ---- streaming path: host chunks in, host rows out (the workQueue contract, main.go:353-380) ---- */
 
