@@ -60,6 +60,10 @@ class CChunkStats(C.Structure):
     ]
 
 
+BGZF_BLOCK_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_size_t, C.c_void_p)  # (user, i, bvcf_bgzf_blk *)
+BGZF_EMIT_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_void_p, C.c_size_t)
+
+
 class CKernelTimes(C.Structure):
     _fields_ = [
         ("scan_ms", C.c_float),
@@ -82,6 +86,7 @@ SYMBOLS = [
     "bvcf_last_error", "bvcf_abi_version", "bvcf_launch_count", "bvcf_resident_run_at", "bvcf_resident_inflate_bgzf",
     "bvcf_bgzf_text_bytes", "bvcf_resident_download_bgzf", "bvcf_resident_write_output", "bvcf_resident_results",
     "bvcf_submit_bgzf", "bvcf_diag_fields", "bvcf_resident_download_bgzf_level", "bvcf_set_regions", "bvcf_index_spans",
+    "bvcf_bgzf_block", "bvcf_bgzf_blocks", "bvcf_bgzf_inflate", "bvcf_bgzf_plan",
 ]
 
 _lib = None
@@ -153,6 +158,14 @@ def lib():
     L.bvcf_index_spans.restype = C.c_int
     L.bvcf_index_spans.argtypes = [vp, sz, C.POINTER(C.c_char_p), C.POINTER(C.c_int64), C.POINTER(C.c_int64), sz,
                                    C.POINTER(u64), sz, C.POINTER(sz)]
+    L.bvcf_bgzf_block.restype = C.c_int
+    L.bvcf_bgzf_block.argtypes = [vp, sz, C.POINTER(sz), C.POINTER(C.c_uint32), C.POINTER(C.c_char_p)]
+    L.bvcf_bgzf_blocks.restype = C.c_int
+    L.bvcf_bgzf_blocks.argtypes = [vp, sz, vp, vp, sz, C.POINTER(sz), C.POINTER(C.c_char_p)]
+    L.bvcf_bgzf_inflate.restype = C.c_int
+    L.bvcf_bgzf_inflate.argtypes = [vp, sz, vp, sz, C.POINTER(C.c_char_p)]
+    L.bvcf_bgzf_plan.restype = C.c_int
+    L.bvcf_bgzf_plan.argtypes = [BGZF_BLOCK_FN, BGZF_EMIT_FN, vp, u64, sz, sz, C.POINTER(C.c_char_p)]
     L.bvcf_strerror.restype = C.c_char_p
     L.bvcf_strerror.argtypes = [C.c_int]
     L.bvcf_last_error.restype = C.c_char_p

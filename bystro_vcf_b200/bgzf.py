@@ -1,89 +1,81 @@
-"""bgzf (block gzip, SAM spec 4.1: what bgzip / htslib write and what .vcf.gz files are) on the host side:
-walking block headers, cutting a file into groups of whole blocks for the streaming path (plan_groups), and a writer
-used by the tests and the bench to make compressed workloads.  The DEFLATE payloads themselves are inflated on the
-GPU (csrc/bvcf_inflate.cuh: bvcf_submit_bgzf, bvcf_resident_inflate_bgzf)."""
+"""bgzf (block gzip, SAM spec 4.1: what bgzip / htslib write and what .vcf.gz files are) on the host side: thin wrappers
+of libbvcf's bgzf module (csrc/bvcf_bgzf.cpp, which the C++ host calls too) for the block header rule, the host inflate
+and the plan that cuts a file into groups of whole blocks for the streaming path (plan_groups); the views an index gives
+a run with regions; and a writer used by the tests and the bench to make compressed workloads.  The DEFLATE payloads
+themselves are inflated on the GPU (csrc/bvcf_inflate.cuh: bvcf_submit_bgzf, bvcf_resident_inflate_bgzf)."""
 from __future__ import annotations
 
-import bisect
+import ctypes as C
 import struct
 import zlib
 from concurrent.futures import ThreadPoolExecutor
 from typing import List, NamedTuple
 
+import numpy as np
+
+from . import _lib
+
 MAGIC = b"\x1f\x8b\x08\x04"
 EOF_BLOCK = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
 MAX_TEXT = 65280  # text bytes per block (bgzip's choice: the compressed block always fits 64 KiB)
+LINE_TOO_LONG = "a single line exceeds the chunk capacity; raise --chunkBytes"
 
 
-def _header(buf, p: int) -> int:
-    """The header of the bgzf block at buf[p]: a gzip member with FLG.FEXTRA whose extra field holds a BC subfield with
-    SLEN 2 -- anywhere in the field (SAM spec 4.1).  The subfields are walked in order, one that runs past the end of the
-    field ends the walk, and the first BC subfield gives BSIZE - 1.  The C++ host (bgzf_header) and the library
-    (bgzf_walk) follow the same rule.  Returns the block size, or 0 when the header is not complete yet; raises
-    ValueError when it is not a bgzf header."""
-    if len(buf) - p < 18:
-        return 0
-    if buf[p] != 0x1F or buf[p + 1] != 0x8B or buf[p + 2] != 8 or not buf[p + 3] & 4:
-        raise ValueError("not a bgzf block")
-    xlen = buf[p + 10] | (buf[p + 11] << 8)
-    if len(buf) - p < 12 + xlen:
-        return 0
-    q, end = p + 12, p + 12 + xlen
-    while q + 4 <= end:
-        slen = buf[q + 2] | (buf[q + 3] << 8)
-        if q + 4 + slen > end:
-            break
-        if buf[q] == 66 and buf[q + 1] == 67 and slen == 2:
-            bsize = (buf[q + 4] | (buf[q + 5] << 8)) + 1
-            if bsize < 12 + xlen + 8:
-                raise ValueError("bgzf block size %d is smaller than its header and trailer" % bsize)
-            return bsize
-        q += 4 + slen
-    raise ValueError("gzip member without the bgzf BC subfield")
+def _addr(buf) -> int:
+    """the address of a bytes-like object or mmap (read-only ones too)"""
+    return np.frombuffer(buf, dtype=np.uint8).ctypes.data
+
+
+def _reason(rc: int, why) -> str:
+    return why.value.decode() if why.value else _lib.lib().bvcf_strerror(rc).decode()
+
+
+def _block(buf, p: int, check: bool = True):
+    """(BSIZE, ISIZE) of the bgzf block at buf[p] (bvcf_bgzf_block): BSIZE 0 while its header is not complete, ISIZE 0
+    unless the whole block is there.  ValueError (with check) when it is not a bgzf block or claims ISIZE 0 but holds
+    text."""
+    size, isize, why = C.c_size_t(), C.c_uint32(), C.c_char_p()
+    rc = _lib.lib().bvcf_bgzf_block(_addr(buf) + p, len(buf) - p, C.byref(size), C.byref(isize), C.byref(why))
+    if rc and check:
+        raise ValueError("%s at byte %d" % (_reason(rc, why), p))
+    return size.value, isize.value
 
 
 def is_bgzf(head) -> bool:
-    """the first bytes of an input start with a whole bgzf header"""
-    try:
-        return _header(head, 0) > 0
-    except ValueError:
-        return False
+    """the first bytes of an input start with a whole bgzf header (a first block that is then refused as corrupt still
+    counts: reading it reports that)"""
+    return _block(head, 0, check=False)[0] > 0
 
 
 def block_size(buf, p: int) -> int:
     """total size of the bgzf block that starts at buf[p] (0 when its header is not complete yet)"""
-    return _header(buf, p)
+    return _block(buf, p)[0]
 
 
-def _payload_text(buf, p: int, bs: int) -> bytes:
-    """the text of the bgzf block at buf[p:p + bs], inflated with zlib and checked against its CRC-32 and ISIZE"""
-    xlen = buf[p + 10] | (buf[p + 11] << 8)
-    try:
-        text = zlib.decompress(bytes(buf[p + 12 + xlen:p + bs - 8]), -15)
-    except zlib.error as e:
-        raise ValueError("corrupt bgzf block at byte %d: %s" % (p, e)) from None
-    crc, isize = struct.unpack("<II", bytes(buf[p + bs - 8:p + bs]))
-    if len(text) != isize or zlib.crc32(text) != crc:
-        raise ValueError("bgzf block at byte %d fails its CRC-32 / ISIZE check" % p)
-    return text
+def _walk(buf):
+    """offset, size and ISIZE (numpy arrays) of every block of a whole bgzf buffer, walked by bvcf_bgzf_blocks"""
+    base, n, p, parts = _addr(buf), len(buf), 0, []
+    got, why = C.c_size_t(), C.c_char_p()
+    while p < n:
+        cap = min((n - p) // 26 + 1, 1 << 20)  # a bgzf block has at least 26 bytes
+        size, isize = np.empty(cap, np.uint32), np.empty(cap, np.uint32)
+        rc = _lib.lib().bvcf_bgzf_blocks(base + p, n - p, size.ctypes.data, isize.ctypes.data, cap, C.byref(got), C.byref(why))
+        if rc:
+            raise ValueError("%s at byte %d" % (_reason(rc, why), p + int(size[:got.value].sum())))
+        if got.value == 0:
+            raise ValueError("truncated bgzf block at byte %d" % p)
+        parts.append((size[:got.value], isize[:got.value]))
+        p += int(parts[-1][0].sum())
+    size = np.concatenate([s for s, _ in parts] or [np.zeros(0, np.uint32)]).astype(np.uint64)
+    isize = np.concatenate([i for _, i in parts] or [np.zeros(0, np.uint32)]).astype(np.uint64)
+    return np.cumsum(size) - size, size, isize
 
 
 def blocks(buf) -> List[tuple]:
     """(offset, size, ISIZE) of every block of a whole bgzf file.  A truncated last block or bytes that are not a bgzf
-    block raise ValueError.  A block that claims ISIZE 0 (normally only the EOF block) is inflated here, and raises
-    ValueError unless it holds no text and CRC-32 0: its text would otherwise be dropped without a word."""
-    out = []
-    p, n = 0, len(buf)
-    while p < n:
-        bs = block_size(buf, p)
-        if bs == 0 or p + bs > n:
-            raise ValueError("truncated bgzf block at byte %d" % p)
-        isize = int.from_bytes(buf[p + bs - 4:p + bs], "little")
-        if isize == 0:
-            _payload_text(buf, p, bs)
-        out.append((p, bs, isize))
-        p += bs
-    return out
+    block raise ValueError, and so does a block that claims ISIZE 0 (normally only the EOF block) unless it holds no
+    text: its text would otherwise be dropped without a word."""
+    return list(zip(*(a.tolist() for a in _walk(buf))))
 
 
 class Group(NamedTuple):
@@ -95,89 +87,62 @@ class Group(NamedTuple):
     text: int  # bytes of inflate(buf[lo:hi])
 
 
-LINE_TOO_LONG = "a single line exceeds the chunk capacity; raise --chunkBytes"
+# bvcf_bgzf_blk
+BLK = np.dtype([("bytes", np.uint64), ("size", np.uint64), ("start", np.uint64), ("isize", np.uint32)], align=True)
+
+
+def plan_blocks(block, data_off: int, chunk_bytes: int, cap: int) -> List[tuple]:
+    """bvcf_bgzf_plan over block(i) -> the address of block i's bvcf_bgzf_blk (BLK), or None past the last: the groups as
+    (lo_block, hi_block, skip, tail).  An exception raised by block() ends the plan and is raised here (ctypes would
+    swallow it); a refusal raises ValueError with the library's reason."""
+    out, err = [], []
+
+    def block_fn(_, i, b):
+        try:
+            a = block(i)
+        except BaseException as e:
+            err.append(e)
+            return -1
+        if a is None:
+            return 0
+        C.memmove(b, a, BLK.itemsize)
+        return 1
+
+    def emit_fn(_, lo, hi, skip, tail, n):
+        out.append((lo, hi, skip, C.string_at(tail, n) if n else b""))
+        return 0
+
+    why = C.c_char_p()
+    rc = _lib.lib().bvcf_bgzf_plan(_lib.BGZF_BLOCK_FN(block_fn), _lib.BGZF_EMIT_FN(emit_fn), None, data_off, chunk_bytes,
+                                   cap, C.byref(why))
+    if err:
+        raise err[0]
+    if rc:
+        raise ValueError(_reason(rc, why))
+    return out
+
+
+def block_table(buf):
+    """the blocks with text of a whole bgzf buffer as bvcf_bgzf_blk (BLK) records, and their offsets with len(buf) after
+    the last"""
+    off, size, isize = _walk(buf)
+    keep = isize > 0
+    table = np.zeros(int(keep.sum()), BLK)
+    table["bytes"], table["size"], table["isize"] = off[keep] + _addr(buf), size[keep], isize[keep]
+    table["start"] = np.cumsum(table["isize"]) - table["isize"]
+    return table, np.append(off[keep], np.uint64(len(buf)))
 
 
 def plan_groups(buf, data_off: int, chunk_bytes: int, cap: int) -> List[Group]:
     """Cut a whole bgzf file into groups of whole blocks of about chunk_bytes of text, data lines from text offset
-    data_off (the end of the #CHROM line) on.  The same rule as the C++ host's reader (csrc/bvcf_host.cpp):
-
-    * a group's blocks are taken while its text is below chunk_bytes (empty blocks, the EOF block among them, add none);
-      the first group starts at the block that holds text byte data_off, its skip is where data_off falls in it;
-    * the line that crosses into the next group belongs to this one: its continuation -- the next group's text up to and
-      including its first newline, inflated here -- is this group's tail, and the next group's skip jumps past it.  A next
-      group with no newline at all is merged into this one;
-    * the last group ends at the file's last newline (an unterminated last line is dropped, main.go:354-357): the blocks
-      from the one holding that newline on are inflated here and left out, their text up to the newline is the tail;
-    * a group whose text plus tail exceeds cap raises ValueError(LINE_TOO_LONG)."""
-    bl = [b for b in blocks(buf) if b[2]]
-    n = len(bl)
-    starts = [0] * (n + 1)
-    for i, b in enumerate(bl):
-        starts[i + 1] = starts[i] + b[2]
-    if data_off >= starts[n]:
-        return []
-    text_of = lambda i: _payload_text(buf, bl[i][0], bl[i][1])  # noqa: E731
-    lo_of = lambda i: bl[i][0] if i < n else len(buf)  # noqa: E731
-    b = bisect.bisect_right(starts, data_off) - 1
-    skip = data_off - starts[b]
-    out: List[Group] = []
-
-    def take(i: int) -> int:  # end block of the group candidate that starts at block i
-        e = i
-        while e < n and starts[e] - starts[i] < chunk_bytes:
-            e += 1
-        return e
-
-    def emit(lo_b: int, hi_b: int, skip_: int, tail: bytes) -> None:
-        text = starts[hi_b] - starts[lo_b]
-        if text + len(tail) > cap:
-            raise ValueError(LINE_TOO_LONG)
-        if text - skip_ + len(tail) > 0:
-            out.append(Group(lo_of(lo_b), lo_of(hi_b), skip_, tail, text))
-
-    while True:
-        e = take(b)
-        tail = None
-        while e < n and tail is None:
-            e2 = take(e)
-            parts = []
-            for j in range(e, e2):  # the continuation: inflated until its newline
-                t = text_of(j)
-                k = t.find(b"\n")
-                if k >= 0:
-                    parts.append(t[:k + 1])
-                    tail = b"".join(parts)
-                    break
-                parts.append(t)
-            if tail is None:
-                e = e2  # no newline in the next group: it joins this one
-        if tail is not None:
-            emit(b, e, skip, tail)
-            b, skip = e, len(tail)
-            continue
-        # the last group [b, n): it ends at the file's last newline
-        f, tail = n, None
-        while f > b and tail is None:
-            f -= 1
-            t = text_of(f)
-            k = t.rfind(b"\n")
-            if k >= 0:
-                tail = t[:k + 1]
-        if tail is None:
-            return out  # nothing but an unterminated last line
-        data_start = starts[b] + skip
-        if data_start < starts[f]:
-            emit(b, f, skip, tail)
-        elif data_start - starts[f] < len(tail):  # the rest is inside the block of the last newline
-            rest = tail[data_start - starts[f]:]
-            if out:  # the previous group's tail takes it
-                g = out.pop()
-                lo_b = bisect.bisect_left(starts, starts[b] - g.text)
-                emit(lo_b, b, g.skip, g.tail + rest)
-            else:
-                emit(f, f, 0, rest)
-        return out
+    data_off (the end of the #CHROM line) on, by bvcf_bgzf_plan (include/bvcf.h states the rule).  A group whose text
+    plus tail exceeds cap raises ValueError(LINE_TOO_LONG)."""
+    table, lo_of = block_table(buf)
+    a0, n = table.ctypes.data, len(table)
+    starts = np.append(table["start"], table["start"][-1] + table["isize"][-1] if n else np.uint64(0)).tolist()
+    lo_of = lo_of.tolist()
+    return [Group(lo_of[lo], lo_of[hi], skip, tail, starts[hi] - starts[lo]) for lo, hi, skip, tail in
+            plan_blocks(lambda i: a0 + i * BLK.itemsize if i < n else None, data_off, chunk_bytes, cap)]
 
 
 def index_views(buf, in_path: str, regions):
@@ -186,11 +151,8 @@ def index_views(buf, in_path: str, regions):
     the blocks from the span's first to its last, its data lines start at text offset skip.  The C++ host's reader
     (csrc/bvcf_host.cpp index_pieces) follows the same rule.  None when there is no index; ValueError when the index is
     malformed or points at bytes that are not a bgzf block of buf."""
-    import ctypes as C
     import gzip
     import os
-
-    from . import _lib
 
     path = next((in_path + e for e in (".tbi", ".csi") if os.path.exists(in_path + e)), None)
     if path is None:
@@ -267,14 +229,16 @@ def compress(data, level: int = 6, block_text: int = MAX_TEXT, threads: int = 0,
 def inflate_host(buf, max_text: int) -> bytes:
     """the text of the whole blocks at the start of a bgzf buffer, until there are at least max_text bytes of it, inflated
     on the host and checked against each block's CRC-32 and ISIZE: only used to read the VCF preamble"""
-    out = []
-    n = 0
-    p = 0
+    out, n, p = [], 0, 0
     while p < len(buf) and n < max_text:
-        bs = block_size(buf, p)
+        bs, isize = _block(buf, p)
         if bs == 0 or p + bs > len(buf):
             break
-        out.append(_payload_text(buf, p, bs))
-        n += len(out[-1])
+        text, why = C.create_string_buffer(isize), C.c_char_p()
+        rc = _lib.lib().bvcf_bgzf_inflate(_addr(buf) + p, bs, text, isize, C.byref(why))
+        if rc:
+            raise ValueError("%s at byte %d" % (_reason(rc, why), p))
+        out.append(text.raw)
+        n += isize
         p += bs
     return b"".join(out)

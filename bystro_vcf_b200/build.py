@@ -20,7 +20,7 @@ NVCC_FLAGS = [
 ]
 
 TARGETS = {
-    "libbvcf.so": (["bvcf_api.cu", "bvcf_index.cpp"], []),
+    "libbvcf.so": (["bvcf_api.cu", "bvcf_index.cpp", "bvcf_bgzf.cpp"], ["-lz"]),
     # host and device must produce the same bytes: no FMA contraction in the generator
     "libbvcfsynth.so": (["bvcf_synth.cu"], ["-fmad=false"]),
 }

@@ -25,6 +25,7 @@
 #include <string>
 #include <vector>
 
+#include "bvcf_bgzf.h"
 #include "bvcf_common.cuh"
 #include "bvcf_prefix.cuh"
 #include "bvcf_region.cuh"
@@ -1122,26 +1123,16 @@ int bvcf_resident_run_at(bvcf_ctx *ctx, size_t begin, size_t len, bvcf_chunk_sta
 }
 
 // ---- bgzf input (SURVEY 8f-3) ------------------------------------------------------------------------------
-// walk the gzip members of a bgzf buffer (RFC 1952 header with the "BC" extra subfield of the SAM spec 4.1).  The header
-// rule is the one of bgzf.py block_size and bvcf_host.cpp bgzf_header: FLG has FEXTRA; the subfields of the extra field
-// are walked in order, a subfield that runs past the end of the field ends the walk, and the first BC subfield with
-// SLEN 2 gives BSIZE - 1.  Members with ISIZE 0 stay in the block table: the kernel checks that they inflate to nothing
-// with CRC-32 0, so text hidden behind a zero ISIZE is refused instead of dropped.
+// walk the gzip members of a bgzf buffer of whole blocks, each header by the rule of bvcf_bgzf.cpp.  Members with
+// ISIZE 0 stay in the block table: the kernel checks that they inflate to nothing with CRC-32 0, so text hidden behind a
+// zero ISIZE is refused instead of dropped.
 static int bgzf_walk(const uint8_t *c, size_t n, std::vector<InflateBlock> *blocks, uint64_t *text_bytes) {
   size_t p = 0;
   uint64_t out = 0;
   while (p < n) {
-    if (n - p < 18 || c[p] != 0x1f || c[p + 1] != 0x8b || c[p + 2] != 8 || !(c[p + 3] & 4)) return BVCF_E_ARG;
-    const size_t xlen = (size_t)c[p + 10] | ((size_t)c[p + 11] << 8);
-    if (n - p < 12 + xlen) return BVCF_E_ARG;
-    size_t bsize = 0;
-    for (size_t q = p + 12; q + 4 <= p + 12 + xlen;) {
-      const size_t slen = (size_t)c[q + 2] | ((size_t)c[q + 3] << 8);
-      if (q + 4 + slen > p + 12 + xlen) break;
-      if (c[q] == 'B' && c[q + 1] == 'C' && slen == 2) { bsize = ((size_t)c[q + 4] | ((size_t)c[q + 5] << 8)) + 1; break; }
-      q += 4 + slen;
-    }
-    if (bsize < 12 + xlen + 8 || n - p < bsize) return BVCF_E_ARG;  // not bgzf, or a truncated last block
+    const long long bs = bgzf_header(c + p, n - p, nullptr);
+    if (bs <= 0 || n - p < (size_t)bs) return BVCF_E_ARG;  // not bgzf, or a truncated last block
+    const size_t bsize = (size_t)bs, xlen = (size_t)c[p + 10] | ((size_t)c[p + 11] << 8);
     const uint32_t isize = (uint32_t)c[p + bsize - 4] | ((uint32_t)c[p + bsize - 3] << 8) | ((uint32_t)c[p + bsize - 2] << 16) |
                            ((uint32_t)c[p + bsize - 1] << 24);
     if (blocks) {

@@ -5,7 +5,7 @@
 // (main.go:345-380) with GPUs as the workers:
 //   reader     finds newline-aligned chunk boundaries; stdin is read straight into pinned buffers, a regular
 //              --in file is memory-mapped and only the boundaries are computed here.  A .vcf.gz (bgzf) input is cut
-//              into groups of whole blocks instead (BgzfIn / plan rule below): the compressed bytes go to the GPUs;
+//              into groups of whole blocks instead (BgzfIn, bvcf_bgzf_plan): the compressed bytes go to the GPUs;
 //   GPU worker one per GPU (chunk k goes to GPU k mod N): stages its chunks into its own pinned ring (parallel
 //              memcpy out of the mapping), keeps n_slots chunks in flight on its context, and -- when it is chunk
 //              k's turn -- writes the rows, appends the dosage batch to the Arrow file and logs the diagnostics,
@@ -417,34 +417,13 @@ struct Turnstile {
 // Replaces the `pigz -d -c in.vcf.gz |` in front of the reference (README.md:10,46).  Groups of whole blocks are
 // uploaded and inflated on the GPU: into a slot's input buffer (bvcf_submit_bgzf), or with --bgzfOut into the resident
 // input region (bvcf_resident_inflate_bgzf).
-// The header of the bgzf block at p (the rule of bgzf.py block_size and of bgzf_walk in bvcf_api.cu): a gzip member with
-// FLG.FEXTRA whose extra field holds a BC subfield with SLEN 2 -- anywhere in the field (SAM spec 4.1).  The subfields
-// are walked in order, one that runs past the end of the field ends the walk, and the first BC subfield gives BSIZE - 1.
-// Returns the block size, 0 when the header is not complete in n bytes, BGZF_NOT_GZIP / BGZF_NO_BC / BGZF_TOO_SMALL.
-enum : long long { BGZF_NOT_GZIP = -1, BGZF_NO_BC = -2, BGZF_TOO_SMALL = -3 };
-long long bgzf_header(const uint8_t *p, size_t n) {
-  if (n < 18) return 0;
-  if (p[0] != 0x1f || p[1] != 0x8b || p[2] != 8 || !(p[3] & 4)) return BGZF_NOT_GZIP;
-  const size_t xlen = (size_t)p[10] | ((size_t)p[11] << 8);
-  if (n < 12 + xlen) return 0;
-  for (size_t q = 12; q + 4 <= 12 + xlen;) {
-    const size_t slen = (size_t)p[q + 2] | ((size_t)p[q + 3] << 8);
-    if (q + 4 + slen > 12 + xlen) break;
-    if (p[q] == 'B' && p[q + 1] == 'C' && slen == 2) {
-      const size_t bsize = ((size_t)p[q + 4] | ((size_t)p[q + 5] << 8)) + 1;
-      return bsize < 12 + xlen + 8 ? BGZF_TOO_SMALL : (long long)bsize;
-    }
-    q += 4 + slen;
-  }
-  return BGZF_NO_BC;
-}
-bool looks_bgzf(const uint8_t *p, size_t n) { return bgzf_header(p, n) > 0; }
-size_t bgzf_block_size(const uint8_t *p, size_t n) {  // 0: header incomplete
-  const long long r = bgzf_header(p, n);
-  if (r == BGZF_NOT_GZIP) fatal("bgzf input: bytes that are not a bgzf block");
-  if (r == BGZF_NO_BC) fatal("gzip input without the bgzf BC subfield: decompress it first (gzip -dc | ...)");
-  if (r == BGZF_TOO_SMALL) fatal("bgzf input: a block smaller than its header and trailer");
-  return (size_t)r;
+// the input starts with a whole bgzf block header (a first block refused as corrupt is reported by BgzfIn)
+bool looks_bgzf(const uint8_t *p, size_t n) {
+  size_t bs = 0;
+  uint32_t isize;
+  const char *why;
+  bvcf_bgzf_block(p, n, &bs, &isize, &why);
+  return bs > 0;
 }
 
 // one bgzf block (SAM spec 4.1) around `text` (< 64 KiB), deflated on the host: the TSV header line
@@ -537,27 +516,24 @@ class Input {
   bool eof_;
 };
 
-// The blocks of a bgzf input, walked as they are needed.  Blocks without text (the EOF block among them) are left out
-// of the list; offsets are absolute in the compressed stream.
+// The blocks of a bgzf input, walked as they are needed (pipe input stays bounded in memory).  Blocks without text (the
+// EOF block among them) are checked by bvcf_bgzf_block and left out of the list; offsets are absolute in the compressed
+// stream.  It is also the block source of bvcf_bgzf_plan.
 class BgzfIn {
  public:
   struct Blk { size_t off, size; uint64_t start; uint32_t isize; };
   explicit BgzfIn(Input &in) : in_(in) {}
-  // block i exists (reads and walks headers until it does or the input ends; a truncated block is fatal)
+  // block i exists (reads and walks headers until it does or the input ends; a truncated or corrupt block is fatal)
   bool has(size_t i) {
     while (blk_.size() <= i && !walked_) {
-      in_.fill(walk_ + (1u << 16) + 18);
+      in_.fill(walk_ + (1u << 16) + 18);  // a whole block, unless the input ends first
       if (walk_ == in_.end()) { walked_ = true; break; }
-      size_t bs = bgzf_block_size(in_.at(walk_), in_.end() - walk_);
-      if (bs && walk_ + bs > in_.end()) { in_.fill(walk_ + bs); }
-      bs = bgzf_block_size(in_.at(walk_), in_.end() - walk_);
+      size_t bs = 0;
+      uint32_t isize = 0;
+      const char *why = nullptr;
+      if (bvcf_bgzf_block(in_.at(walk_), in_.end() - walk_, &bs, &isize, &why)) fatal(std::string("bgzf input: ") + why);
       if (!bs || walk_ + bs > in_.end()) fatal("bgzf input: truncated block at the end");
-      const uint8_t *e = in_.at(walk_ + bs - 4);
-      const uint32_t isize = (uint32_t)e[0] | ((uint32_t)e[1] << 8) | ((uint32_t)e[2] << 16) | ((uint32_t)e[3] << 24);
-      // a block that claims no text is checked here (normally only the 28-byte EOF block): one that inflates to text
-      // would otherwise have that text dropped without a word
       if (isize) blk_.push_back({walk_, bs, text_, isize});
-      else inflate_checked({walk_, bs, text_, 0});
       text_ += isize;
       walk_ += bs;
     }
@@ -571,35 +547,28 @@ class BgzfIn {
     while (has(b) && blk_[b].start + blk_[b].isize <= text_off) b++;
     return b;
   }
-  // block i inflated on the host, its CRC-32 and ISIZE checked
-  std::string inflate_block(size_t i) { return inflate_checked(blk_[i]); }
-  // the first `want` text bytes (fewer at the end of the input): the preamble
+  // the first `want` text bytes (fewer at the end of the input), inflated on the host: the preamble
   std::string prefix(size_t want) {
     std::string out;
-    for (size_t i = 0; out.size() < want && has(i); i++) out += inflate_block(i);
+    for (size_t i = 0; out.size() < want && has(i); i++) {
+      const size_t n = out.size();
+      const char *why = nullptr;
+      out.resize(n + blk_[i].isize);
+      if (bvcf_bgzf_inflate(in_.at(blk_[i].off), blk_[i].size, &out[n], blk_[i].isize, &why))
+        fatal(std::string("bgzf input: ") + why);
+    }
     return out;
+  }
+  // bvcf_bgzf_block_fn over this input
+  static int block(void *self, size_t i, bvcf_bgzf_blk *b) {
+    BgzfIn &g = *(BgzfIn *)self;
+    if (!g.has(i)) return 0;
+    const Blk &k = g.blk_[i];
+    *b = {g.in_.at(k.off), k.size, k.start, k.isize};
+    return 1;
   }
 
  private:
-  // the text of block b, inflated with zlib; a block that fails its CRC-32 or ISIZE is fatal
-  std::string inflate_checked(const Blk &b) {
-    const uint8_t *p = in_.at(b.off);
-    const size_t xlen = (size_t)p[10] | ((size_t)p[11] << 8);
-    std::string text(b.isize, '\0');
-    z_stream z{};
-    if (inflateInit2(&z, -15) != Z_OK) fatal("zlib: inflateInit2 failed");
-    z.next_in = const_cast<Bytef *>(p + 12 + xlen); z.avail_in = (uInt)(b.size - 12 - xlen - 8);
-    z.next_out = (Bytef *)text.data(); z.avail_out = b.isize;
-    const int zr = inflate(&z, Z_FINISH);
-    const size_t got = z.total_out;
-    inflateEnd(&z);
-    const uint8_t *t = p + b.size - 8;
-    const uint32_t crc = (uint32_t)t[0] | ((uint32_t)t[1] << 8) | ((uint32_t)t[2] << 16) | ((uint32_t)t[3] << 24);
-    if (zr != Z_STREAM_END || got != b.isize || crc32(crc32(0L, Z_NULL, 0), (const Bytef *)text.data(), (uInt)got) != crc)
-      fatal("bgzf input: a corrupt block (inflate, CRC-32 or ISIZE check failed)");
-    return text;
-  }
-
   Input &in_;
   size_t walk_ = 0;
   uint64_t text_ = 0;
@@ -607,88 +576,11 @@ class BgzfIn {
   std::vector<Blk> blk_;
 };
 
-// The groups of a bgzf input (the rule of bystro_vcf_b200/bgzf.py plan_groups): blocks are taken while a group's text
-// is below chunk_bytes; the first group starts at the block holding text byte data_off.  The line that crosses into the
-// next group belongs to this one: the next group's text up to and including its first newline, inflated here, is this
-// group's tail and the next group's skip; a next group with no newline is merged into this one.  The last group ends at
-// the last newline of the input (an unterminated last line is dropped, main.go:354-357): the blocks from the one
-// holding it on are inflated here and left out, their text up to it is the tail.  emit(lo_block, hi_block, skip, tail)
-// receives each group in order (hi_block: one past its last block).
-template <class Emit>
-void plan_bgzf_groups(BgzfIn &in, uint64_t data_off, size_t chunk_bytes, size_t cap, Emit emit_out) {
-  size_t b = in.block_at(data_off);
-  if (!in.has(b)) return;
-  size_t skip = (size_t)(data_off - in[b].start);
-  auto take = [&](size_t i) {
-    size_t e = i;
-    while (in.has(e) && in[e].start - in[i].start < chunk_bytes) e++;
-    return e;
-  };
-  auto text_of = [&](size_t lo, size_t hi) { return (uint64_t)((in.has(hi) ? in[hi].start : in[hi - 1].start + in[hi - 1].isize) - in[lo].start); };
-  // one group is held back: the last group may still hand its text to it
-  struct G { size_t lo, hi, skip; std::string tail; bool set = false; } prev;
-  auto emit = [&](size_t lo, size_t hi, size_t skip_, std::string tail) {
-    const uint64_t text = hi > lo ? text_of(lo, hi) : 0;
-    if (text + tail.size() > cap) fatal("a single line exceeds the chunk capacity; raise --chunkBytes");
-    if (text - skip_ + tail.size() == 0) return;
-    if (prev.set) emit_out(prev.lo, prev.hi, prev.skip, prev.tail);
-    prev.lo = lo; prev.hi = hi; prev.skip = skip_; prev.tail = std::move(tail); prev.set = true;
-  };
-  for (;;) {
-    size_t e = take(b);
-    bool found = false;
-    std::string tail;
-    while (in.has(e) && !found) {
-      const size_t e2 = take(e);
-      tail.clear();
-      for (size_t j = e; j < e2 && !found; j++) {  // the continuation: inflated until its newline
-        const std::string t = in.inflate_block(j);
-        const size_t k = t.find('\n');
-        if (k != std::string::npos) { tail.append(t, 0, k + 1); found = true; }
-        else tail += t;
-      }
-      if (!found) e = e2;  // no newline in the next group: it joins this one
-    }
-    if (found) {
-      const size_t n = tail.size();
-      emit(b, e, skip, std::move(tail));
-      b = e; skip = n;
-      continue;
-    }
-    // the last group [b, n): it ends at the input's last newline
-    size_t f = e;
-    std::string last;
-    bool nl = false;
-    while (f > b && !nl) {
-      f--;
-      const std::string t = in.inflate_block(f);
-      const size_t k = t.rfind('\n');
-      if (k != std::string::npos) { last.assign(t, 0, k + 1); nl = true; }
-    }
-    if (nl) {
-      const uint64_t data_start = in[b].start + skip;
-      if (data_start < in[f].start) {
-        emit(b, f, skip, std::move(last));
-      } else if (data_start - in[f].start < last.size()) {  // the rest is inside the block of the last newline
-        std::string rest = last.substr((size_t)(data_start - in[f].start));
-        if (prev.set) {
-          prev.tail += rest;  // the previous group's tail takes it
-          if (text_of(prev.lo, prev.hi) + prev.tail.size() > cap) fatal("a single line exceeds the chunk capacity; raise --chunkBytes");
-        } else {
-          emit(f, f, 0, std::move(rest));
-        }
-      }
-    }
-    if (prev.set) emit_out(prev.lo, prev.hi, prev.skip, prev.tail);
-    return;
-  }
-}
-
 // What a run reads: the input from its data lines on -- or, with regions and a tabix / CSI index beside a bgzf input, the
 // index's spans only.  A span [vbeg, vend) is a view of the mapped file from the block of vbeg to the end of the block of
 // vend, its data lines from vbeg's offset into that first block on; the records after vend in its last block and the
 // lines between two regions inside one span are dropped by the GPU's region filter.  Both drivers read these pieces
-// through BgzfIn, the streaming one cut into groups by plan_bgzf_groups.
+// through BgzfIn, the streaming one cut into groups by bvcf_bgzf_plan.
 struct Piece {
   Input *in;
   BgzfIn *gz;        // null: plain text
@@ -735,17 +627,23 @@ bool index_pieces(const Config &c, const uint8_t *map, size_t map_len, IndexedIn
                           sp.data(), n, &n);
   }
   if (rc) fatal(path + ": " + bvcf_strerror(rc) + " (not a tabix or CSI index)");
-  auto block_at = [&](uint64_t off) {  // a bgzf block starts at compressed offset off: its size
-    const long long bs = off < map_len ? bgzf_header(map + off, map_len - off) : 0;
-    if (bs <= 0 || off + (uint64_t)bs > map_len)
+  auto size_at = [&](uint64_t off) {  // the size of the bgzf block at compressed offset off; 0 when there is none
+    size_t bs = 0;
+    uint32_t isize;
+    const char *why;
+    return off < map_len && !bvcf_bgzf_block(map + off, map_len - off, &bs, &isize, &why) ? (uint64_t)bs : 0;
+  };
+  auto block_at = [&](uint64_t off) {  // a whole bgzf block starts at compressed offset off: its size
+    const uint64_t bs = size_at(off);
+    if (!bs || off + bs > map_len)
       fatal(path + ": virtual offset " + std::to_string(off) + " << 16 is not a bgzf block of " + c.inPath);
-    return (uint64_t)bs;
+    return bs;
   };
   for (size_t k = 0; k < n; k++) {
     const uint64_t cb = sp[2 * k] >> 16, ce = sp[2 * k + 1] >> 16, ue = sp[2 * k + 1] & 0xFFFF;
     block_at(cb);
     const uint64_t end = ue ? ce + block_at(ce) : ce;
-    if (end < ce || end > map_len || (ce < map_len && !ue && ce != cb && bgzf_header(map + ce, map_len - ce) <= 0))
+    if (end < ce || end > map_len || (ce < map_len && !ue && ce != cb && !size_at(ce)))
       fatal(path + ": virtual offset " + std::to_string(ce) + " << 16 is not a bgzf block of " + c.inPath);
     if (end <= cb) continue;
     out.views.emplace_back(new Input(-1, map + cb, (size_t)(end - cb), {}));
@@ -1033,11 +931,11 @@ void run_streaming(const Config &config, const std::vector<Piece> &pieces, const
     for (const Piece &piece : pieces) {
       Input &in = *piece.in;
       BgzfIn *gz = piece.gz;
-      plan_bgzf_groups(*gz, piece.data_off, config.chunkBytes, cap, [&](size_t lo_b, size_t hi_b, size_t skip, const std::string &tail) {
+      auto emit = [&](size_t lo_b, size_t hi_b, size_t skip, const uint8_t *tail, size_t tail_len) {
         const size_t lo = gz->off(lo_b), hi = gz->off(hi_b);
         if (hi - lo > cap) fatal("a bgzf group exceeds the chunk capacity; raise --chunkBytes");
         Chunk c;
-        c.seq = seq; c.len = hi - lo; c.gz = true; c.skip = skip; c.tail = tail;
+        c.seq = seq; c.len = hi - lo; c.gz = true; c.skip = skip; c.tail.assign((const char *)tail, tail_len);
         if (in.mapped()) {
           c.src = in.at(lo);
         } else {
@@ -1047,7 +945,14 @@ void run_streaming(const Config &config, const std::vector<Piece> &pieces, const
         }
         queues[seq % n_gpu]->push(std::move(c));
         seq++;
-      });
+      };
+      struct Plan { BgzfIn *gz; decltype(emit) *out; } plan{gz, &emit};
+      const char *why = nullptr;
+      const int rc = bvcf_bgzf_plan(
+          [](void *u, size_t i, bvcf_bgzf_blk *b) { return BgzfIn::block(((Plan *)u)->gz, i, b); },
+          [](void *u, size_t lo, size_t hi, size_t skip, const uint8_t *t, size_t n) { (*((Plan *)u)->out)(lo, hi, skip, t, n); return 0; },
+          &plan, piece.data_off, config.chunkBytes, cap, &why);
+      if (rc) fatal(rc == BVCF_E_ARG && why ? std::string("bgzf input: ") + why : why ? why : bvcf_strerror(rc));
     }
   } else if (in.mapped()) {
     const uint8_t *map = in.at(0);

@@ -729,7 +729,10 @@ def _read_vcf_resident(config: Config, head: bytes, reader: BinaryIO, writer: Op
                         p = min(len(buf), batch_text)
                     while gz and text < batch_text:
                         fill(p + (1 << 16) + 18)
-                        bs = bgzf.block_size(buf, p)
+                        try:
+                            bs = bgzf.block_size(buf, p)
+                        except ValueError as e:  # not bgzf, or a block that claims ISIZE 0 but holds text
+                            raise BvcfError("bgzf input: %s" % e) from None
                         if bs == 0 or p + bs > len(buf):
                             if not eof:
                                 fill(p + max(bs, 1 << 16) + 18)

@@ -13,7 +13,7 @@ Two partitions are provided:
                      k mod N, results are written in chunk order.  Output streams while the GPUs work and host
                      memory stays bounded (a few chunks per GPU), which N contiguous shards cannot offer: shard 1's
                      whole output would have to wait for shard 0's.  A bgzf (.vcf.gz) input is cut into groups of
-                     whole blocks (bgzf.plan_groups): the compressed bytes go to the GPUs, which inflate them.
+                     whole blocks (bgzf.plan_groups, libbvcf's bvcf_bgzf_plan): the compressed bytes go to the GPUs, which inflate them.
 Both are pure host logic around bvcf_submit / bvcf_collect.
 """
 from __future__ import annotations

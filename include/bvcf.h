@@ -195,6 +195,55 @@ int bvcf_resident_inflate_bgzf(bvcf_ctx *ctx, const void *comp, size_t comp_len,
  * counted, those with ISIZE 0 (the EOF block among them) too: the GPU inflates and checks them like any other. */
 int bvcf_bgzf_text_bytes(const void *comp, size_t comp_len, uint64_t *text_bytes, uint64_t *n_blocks);
 
+/* ---- bgzf input on the host: what a host needs to read a .vcf.gz before its groups go to the GPU ---- */
+
+/* Host only: the bgzf block at p[0, n) -- a gzip member with FLG.FEXTRA whose extra field holds a BC subfield with
+ * SLEN 2 anywhere in it (SAM spec 4.1; the first such subfield gives BSIZE - 1).  *size receives 0 while the header is
+ * not complete in n bytes, else BSIZE -- also when the block is then refused as corrupt, so *size > 0 tells a bgzf
+ * header.  When the whole block is in p[0, n), *isize receives its ISIZE, and a block with ISIZE 0 is inflated and
+ * refused unless it holds no text.  BVCF_E_ARG with a static reason in *why: not a bgzf block, no BC subfield, smaller
+ * than its header and trailer, or corrupt. */
+int bvcf_bgzf_block(const void *p, size_t n, size_t *size, uint32_t *isize, const char **why);
+/* Host only: bvcf_bgzf_block over the blocks that follow each other from p on: the first cap of them, or those before
+ * the first that is not whole in p[0, n), give size[k] and isize[k]; *n_blocks receives their count (on a refusal, the
+ * count of those before the refused one). */
+int bvcf_bgzf_blocks(const void *p, size_t n, uint32_t *size, uint32_t *isize, size_t cap, size_t *n_blocks,
+                     const char **why);
+/* Host only: inflate the whole bgzf block at block[0, n) into text[0, ISIZE) with zlib and check its CRC-32 and ISIZE.
+ * BVCF_E_ARG with a static reason in *why: not bgzf, truncated or corrupt; BVCF_E_TOO_LARGE: cap < ISIZE. */
+int bvcf_bgzf_inflate(const void *block, size_t n, void *text, size_t cap, const char **why);
+
+/* Block i of the input for bvcf_bgzf_plan: a block with text (those with ISIZE 0 already checked and left out). */
+typedef struct {
+  const uint8_t *bytes; /* its first byte: read only before the next call of the block function */
+  size_t size;          /* BSIZE */
+  uint64_t start;       /* text offset of its first byte: the sum of the ISIZEs before it */
+  uint32_t isize;
+} bvcf_bgzf_blk;
+/* 1 with *b filled, 0 past the last block, < 0 an error that ends the plan */
+typedef int (*bvcf_bgzf_block_fn)(void *user, size_t i, bvcf_bgzf_blk *b);
+/* one group, blocks [lo_block, hi_block): its text is inflate(blocks)[skip:] + tail; non-zero ends the plan */
+typedef int (*bvcf_bgzf_emit_fn)(void *user, size_t lo_block, size_t hi_block, size_t skip, const uint8_t *tail,
+                                 size_t tail_len);
+/* Host only: cut an input into the groups of whole blocks that bvcf_submit_bgzf takes, data lines from text offset
+ * data_off (the end of the #CHROM line) on, and hand each group to emit in input order.
+ *  - A group's blocks are taken while its text is below chunk_bytes; the first group starts at the block holding text
+ *    byte data_off, its skip is where data_off falls in it.
+ *  - The line that crosses into the next group belongs to this one: its continuation -- the next group's text up to and
+ *    including its first newline, inflated here -- is this group's tail and the next group's skip.  A next group with
+ *    no newline joins this one.
+ *  - The last group ends at the input's last newline (an unterminated last line is dropped): the blocks from the one
+ *    holding it on are inflated here and left out, their text up to it is the tail.  What is left of the data inside the
+ *    block of that newline goes to the tail of the group before.
+ *  - A group whose text plus tail exceeds cap is refused: BVCF_E_TOO_LARGE, *why "a single line exceeds the chunk
+ *    capacity; raise --chunkBytes".
+ * Blocks are asked for in order, i = 0, 1, 2, ... until block returns 0, and block i once more right before its bytes are
+ * read.  Once emit returns for a group, the planner reads no block bytes before that group's hi_block, so a reader may
+ * drop them.  A non-zero return of a callback ends the plan and is returned; a corrupt block inflated here gives
+ * BVCF_E_ARG and its reason in *why. */
+int bvcf_bgzf_plan(bvcf_bgzf_block_fn block, bvcf_bgzf_emit_fn emit, void *user, uint64_t data_off, size_t chunk_bytes,
+                   size_t cap, const char **why);
+
 /* bgzf-compressed output (downstream of the reference stands `| pigz -c`, README.md:10,71): the rows in
  * [offset, offset + len) of the resident output region are deflated on the GPU (48 KiB slices, LZ77 + fixed Huffman
  * codes, CRC-32) and only the compressed blocks cross PCIe.  The bytes are whole bgzf blocks: concatenate the

@@ -1,5 +1,5 @@
 """bgzf input on the host, without a GPU: the DEFLATE corpus of deflate_writer.py checked against zlib (before any GPU
-decodes it), one header rule for the five bgzf header parsers, and members that claim ISIZE 0 checked instead of
+decodes it), the one bgzf header rule (libbvcf's bvcf_bgzf.cpp) as both CLIs apply it, and members that claim ISIZE 0 checked instead of
 skipped."""
 import ctypes
 import os
@@ -97,9 +97,9 @@ def _header_table():
 
 @pytest.mark.parametrize("case", [c[0] for c in _header_table()])
 def test_bgzf_header_parsers_agree(case, tmp_path):
-    """bgzf.is_bgzf, bgzf.block_size, bvcf_bgzf_text_bytes (the library's walk) and the C++ host's looks_bgzf /
-    bgzf_block_size accept the same headers -- BC anywhere in the extra field, the first BC subfield with SLEN 2 inside
-    the field -- and agree on the block size"""
+    """the one header rule -- BC anywhere in the extra field, the first BC subfield with SLEN 2 inside the field -- as
+    bgzf.is_bgzf / block_size / blocks, bvcf_bgzf_text_bytes (the library's walk) and the C++ CLI's refusals see it:
+    they accept the same headers and agree on the block size"""
     from bystro_vcf_b200 import _lib, bgzf
 
     name, first, ok = next(c for c in _header_table() if c[0] == case)
@@ -175,15 +175,19 @@ def test_plan_groups_refuses_hidden_text(where):
 
 
 def test_hidden_text_in_the_preamble_is_refused_by_both_clis(tmp_path):
-    """a member inside the ## lines whose trailer claims ISIZE 0 but which inflates to text: exit 1 before any device
-    work, piped or from --in"""
+    """a member inside the ## lines -- or the first member -- whose trailer claims ISIZE 0 but which inflates to text, or
+    an empty first member with a wrong CRC-32: exit 1 before any device work, piped or from --in, with the bgzf refusal
+    (the input is still told to be bgzf by its header, not taken for plain text)"""
     from bystro_vcf_b200 import bgzf
 
     head = VCF[:VCF.index(b"#CHROM")]
-    data = bgzf.compress(head[:20], eof=False) + _hidden() + bgzf.compress(VCF[20:])
-    inp = tmp_path / "in.vcf.gz"
-    inp.write_bytes(data)
-    for cmd in [PY] + ([[BIN]] if os.path.exists(BIN) else []):
-        for r in (_cli(cmd + ["--in", str(inp)], b""), _cli(cmd, data)):
-            assert r.returncode == 1, (cmd, r.stderr[-400:])
-            assert b"bgzf" in r.stderr, (cmd, r.stderr[-400:])
+    for data in (bgzf.compress(head[:20], eof=False) + _hidden() + bgzf.compress(VCF[20:]),
+                 _hidden() + bgzf.compress(VCF), D.member(b"\x03\x00", b"", crc=1) + bgzf.compress(VCF)):
+        assert bgzf.is_bgzf(data)
+        inp = tmp_path / "in.vcf.gz"
+        inp.write_bytes(data)
+        for cmd in [PY] + ([[BIN]] if os.path.exists(BIN) else []):
+            for r in (_cli(cmd + ["--in", str(inp)], b""), _cli(cmd, data)):
+                assert r.returncode == 1, (cmd, r.stderr[-400:])
+                assert b"bgzf" in r.stderr and b"CRC-32" in r.stderr, (cmd, r.stderr[-400:])
+                assert b"Not a VCF file" not in r.stderr and b"Traceback" not in r.stderr, (cmd, r.stderr[-400:])

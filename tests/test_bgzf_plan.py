@@ -96,3 +96,28 @@ def test_truncated_or_garbage_input_is_an_error():
     flipped[len(comp) - 28 - 8] ^= 1
     with pytest.raises(ValueError, match="CRC-32"):
         bgzf.plan_groups(bytes(flipped), len(PRE), 1 << 16, 1 << 30)
+
+
+def test_an_exception_in_the_block_source_ends_the_plan():
+    """bvcf_bgzf_plan driven through ctypes (bgzf.plan_blocks) with a block source that raises partway through: the
+    exception reaches the caller, not a partial plan"""
+    data = PRE + b"1\t1\tx\n" * 100000
+    comp = bgzf.compress(data, block_text=4000)
+    table, _ = bgzf.block_table(comp)
+    addr = [table.ctypes.data + i * bgzf.BLK.itemsize for i in range(len(table))]
+    whole = bgzf.plan_blocks(lambda i: addr[i] if i < len(addr) else None, len(PRE), 1 << 16, 1 << 30)
+    assert [g[2:4] for g in whole] == [g[2:4] for g in bgzf.plan_groups(comp, len(PRE), 1 << 16, 1 << 30)]
+    assert len(whole) > 4
+
+    class Stop(Exception):
+        pass
+
+    def block(i):
+        if i >= len(addr) // 2:
+            raise Stop(i)
+        return addr[i]
+
+    got = None
+    with pytest.raises(Stop):
+        got = bgzf.plan_blocks(block, len(PRE), 1 << 16, 1 << 30)
+    assert got is None

@@ -154,7 +154,7 @@ def _cli(cmd, data):
 def test_end_to_end_with_long_codes(chr1_sample, tmp_path):
     """chr1 lines re-encoded as bgzf with random codes of up to 15 bits: read_vcf (auto-detected, small chunks: groups
     and host-inflated tails), the C++ CLI from --in and from a pipe, and --bgzfOut in both CLIs give the plain run's
-    rows; with one middle member's ISIZE set to 0 both CLIs exit 1"""
+    rows; with one middle member's ISIZE set to 0 both CLIs exit 1 with a bgzf message, not a traceback"""
     from bystro_vcf_b200 import Config, bgzf, read_vcf
 
     vcf = chr1_sample
@@ -188,3 +188,4 @@ def test_end_to_end_with_long_codes(chr1_sample, tmp_path):
         for flags in ([], ["--bgzfOut"]):
             for r in (_cli(cmd + flags + ["--in", str(inp)], b""), _cli(cmd + flags, bytes(bad))):
                 assert r.returncode == 1, (cmd, flags, r.stderr.decode()[-2000:])
+                assert b"bgzf" in r.stderr and b"Traceback" not in r.stderr, (cmd, flags, r.stderr.decode()[-2000:])
